@@ -234,6 +234,42 @@ def frame_hash(torch, dist, r, world, frames=2):
             "recipe": "FNV-1a-64 over per-row (RGBA8, accumulation) wrap-around weighted word sums, rows in yi order"}
 
 
+DUMP_PIXELS = 1 << 20  # pixels sampled by --dump-outputs: 2 x 16 MB of float32 + 8 MB of indices
+
+
+def dump_outputs(torch, dist, r, rank, out_dir):
+    """--dump-outputs DIR: what the last timed frame left for a caller of the frame loop — the RGBA8 image and the float4
+    accumulation — at a fixed, seeded sample of DUMP_PIXELS pixel indices (every pixel if the image is smaller), so that two
+    builds can be compared output for output.  Written by rank 0 as DIR/pixels.npy (n x 4, float32 of the 0-255 channel
+    values), DIR/accumulation.npy (n x 4, float32) and DIR/pixel_index.npy (n, float64: index into the image buffer, whose
+    rows are stored bottom-up)."""
+    import numpy as np
+
+    torch.cuda.synchronize()
+    first = r.slabs[0]
+    W, H = first.W, first.H
+    acc = torch.zeros(H * W * 4, dtype=torch.int32, device="cuda")  # raw float bits: the sum below only moves them
+    pix = torch.zeros(H * W, dtype=torch.int32, device="cuda")
+    for sl in r.slabs:  # every row comes from the slab that rendered it
+        if sl.y1 <= sl.y0:
+            continue
+        a, b = (H - sl.y1) * W, (H - sl.y0) * W
+        acc[4 * a:4 * b] = sl._rows(sl.t_acc, 16, sl.y0, sl.y1).view(torch.int32)
+        pix[a:b] = sl._rows(sl.t_pix, 4, sl.y0, sl.y1).view(torch.int32)
+    if dist is not None:
+        dist.all_reduce(acc)
+        dist.all_reduce(pix)
+    if rank != 0:
+        return
+    n = W * H
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    sel = torch.from_numpy(idx).to("cuda")
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "accumulation.npy"), acc.view(torch.float32).reshape(n, 4)[sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "pixels.npy"), pix.view(torch.uint8).reshape(n, 4)[sel].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+
+
 # ============================================================================================== reference GPU comparator
 def run_ref_gpu(W, H, steps, warmup, tiles=(3, 2), timeout=900):
     """the reference's own Orochi/HIPRT CUDA build of examples/10_restir_di on this GPU (baseline/_ref/bin/ref_gpu, built
@@ -420,6 +456,8 @@ def run_cuda(args):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        dump_outputs(torch, dist if world > 1 else None, r, rank, args.dump_outputs)
     launches = r.launch_count() - launches0
     rays1 = r.shadow_rays_traced()
     shadow_rays = [(b - a) / args.steps for a, b in zip(rays0, rays1)]  # per frame: (visibility reuse, resolve)
@@ -1006,7 +1044,14 @@ def main():
                          "synchronise after every frame like the reference's loop")
     ap.add_argument("--mode", default="fused", choices=["fused", "dropin"],
                     help="fused: one crt_restir_* frame call sequence (default); dropin: the reference's launch list")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed frames, write the last one's RGBA8 image and accumulation (a seeded sample of "
+                         "pixels) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "cuda" or args.config != "10"):
+        ap.error("--dump-outputs is available for the default workload (--impl cuda --config 10)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -11,7 +11,7 @@
 //     double, adds each fraction digit as d * 10^-k (a table of the literals 0.1 ... 0.0000001 for k <= 7, pow(10,-k)
 //     beyond), applies an exponent as ldexp(m * pow(5, e), e), and only then narrows to float.  parse_real() below
 //     performs the same operations in the same order, so the floats match bit for bit
-//     (tests/test_host_obj.py checks all four reference scenes against the reference loader's output).
+//     (tests/test_host_obj.py checks them against the reference loader's output).
 #pragma once
 #include <cmath>
 #include <cstdio>

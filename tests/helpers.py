@@ -16,6 +16,22 @@ def small_scene(name):
     return np.ascontiguousarray(golden("scenes_small.npz")[name])
 
 
+# blocks_pt (852 070 triangles, 4 lights) and blocks_restir (1 598 368 triangles, 145 982 lights) are tens of MB: the
+# repository does not hold them, so a seeded procedural city of the same size and character stands in for each
+STAND_INS = {"blocks_pt": dict(n_blocks=71006, seed=8, extent=200.0, emissive_fraction=5e-5),
+             "blocks_restir": dict(n_blocks=133197, seed=10, extent=400.0, emissive_fraction=0.0913)}
+
+
+def scene(name):
+    """a scene the examples load, from the repository alone: cornellbox1 and blocks_ao as the reference loader produced
+    them (golden/scenes_small.npz), blocks_pt and blocks_restir as their procedural stand-ins (STAND_INS)"""
+    if name in STAND_INS:
+        import scenes
+
+        return scenes.procedural_blocks(**STAND_INS[name])
+    return small_scene(name)
+
+
 def same(a, b):
     """bit-level equality that treats NaN == NaN (compares raw bytes of float arrays)."""
     a, b = np.ascontiguousarray(a), np.ascontiguousarray(b)

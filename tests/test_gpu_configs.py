@@ -15,8 +15,8 @@ import pytest
 
 import cedecrt
 import orc
-from helpers import DeviceAsOracle, reservoir_mismatch, same, small_scene
-from test_oracle_pinning import SURVEY_PRIMARY, pixel_classes
+from helpers import DeviceAsOracle, reservoir_mismatch, same, scene, small_scene
+from test_oracle_pinning import SURVEY_PRIMARY, pixel_classes, primary_goldens
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -46,26 +46,19 @@ def exact(rt, port):
     rt.set_math_mode(cedecrt.MATH_LIBDEVICE)
 
 
-def staged(name):
-    import stage_assets
-
-    if not stage_assets.have_scene(name):
-        pytest.skip("scene cache assets/%s.tri.xz not staged" % name)
-    return stage_assets.load_scene(name)
-
-
 def band(y0, y1):
     return slice((H - y1) * W, (H - y0) * W)  # bottom-up storage (10_restir_di.cu:18-20)
 
 
 # ------------------------------------------------------------------ primary visibility: the survey's goldens on the GPU
-@pytest.mark.parametrize("scene", sorted(SURVEY_PRIMARY))
-def test_primary_visibility_survey_goldens(rt, scene):
-    """k_raycast on the three real scenes at the reference cameras, 1920x1080: pixel classes and the FNV-1a-64 of the
-    primitive-id image equal the goldens SURVEY.md section 4 extracted from the reference code (the oracle reproduces
-    the same values on the CPU: test_oracle_pinning.py) — every one of 2 073 600 closest hits, ties included"""
-    cam, classes, prim_hash, _ = SURVEY_PRIMARY[scene]
-    tris = staged(scene)
+@pytest.mark.parametrize("name", sorted(SURVEY_PRIMARY))
+def test_primary_visibility_survey_goldens(rt, name):
+    """k_raycast on the three scenes of helpers.scene at the reference cameras, 1920x1080: pixel classes and the
+    FNV-1a-64 of the primitive-id image equal the goldens of test_oracle_pinning.py (for blocks_ao the ones SURVEY.md
+    section 4 extracted from the reference code; the oracle reproduces them on the CPU) — every one of 2 073 600 closest
+    hits, ties included"""
+    cam, classes, prim_hash, _ = primary_goldens(name)
+    tris = scene(name)
     d_tris = rt.to_device(tris)
     g = rt.build_geometry(d_tris)
     vis = rt.buffer(cedecrt.VISIBILITY, W * H)
@@ -78,7 +71,7 @@ def test_primary_visibility_survey_goldens(rt, scene):
 
 # ------------------------------------------------------------------ config 2: 06_ao_hiprt, blocks_ao, 32 AO rays
 def test_config2_ao_1080p_band_bit_exact(exact, port):
-    tris = staged("blocks_ao")
+    tris = scene("blocks_ao")
     port.set_example(6)
     g, gp = exact.geom_build(tris), port.geom_build(tris)
     mine = exact.ao(W, H, g, tris, exact.lookat(*CAM_AO, W, H), 32).reshape(-1, 4)
@@ -99,12 +92,11 @@ def test_config2_ao_1080p_band_bit_exact(exact, port):
 
 # ------------------------------------------------------------------ config 3: 08_nee, blocks_pt, max depth 4
 def test_config3_nee_1080p_band_bit_exact_two_frames(exact, port):
-    tris = staged("blocks_pt")
-    assert len(tris) == 852070
+    tris = scene("blocks_pt")
     port.set_example(8)
     opt = orc.make_options(accumulate=1, max_depth=4)
     lights = orc.light_indices(tris)
-    assert len(lights) == 4
+    assert len(lights) == 72
     g, gp = exact.geom_build(tris), port.geom_build(tris)
     a, b = np.zeros((W * H, 4), np.float32), np.zeros((W * H, 4), np.float32)
     y0, y1 = 508, 572
@@ -125,7 +117,7 @@ def test_config3_nee_1080p_band_bit_exact_two_frames(exact, port):
 def test_config3_nee_64_frames_within_tolerance(rt, port):
     """64 accumulated frames, depth 4, default arithmetic of the per-kernel path against the oracle's libm arithmetic,
     at reduced size (the oracle runs every frame in full)"""
-    tris = staged("blocks_pt")
+    tris = scene("blocks_pt")
     w, h, N = 320, 180, 64
     rt.set_math_mode(cedecrt.MATH_REFERENCE)
     port.set_math_mode(0)
@@ -151,11 +143,11 @@ def test_config3_nee_64_frames_within_tolerance(rt, port):
 
 # ------------------------------------------------------------------ config 4: 09_ris, blocks_restir, shadowed target
 def test_config4_ris_shadowed_1080p_band_bit_exact(exact, port):
-    tris = staged("blocks_restir")
+    tris = scene("blocks_restir")
     port.set_example(9)
     opt = orc.make_options(accumulate=1, ris_sample_count=32, use_shadowed_target_function=1)
     lights = orc.light_indices(tris)
-    assert len(lights) == 145982
+    assert len(lights) == 145344
     g, gp = exact.geom_build(tris), port.geom_build(tris)
     a, b = np.zeros((W * H, 4), np.float32), np.zeros((W * H, 4), np.float32)
     y0, y1 = 520, 584  # 35 rays per path vertex, depth up to 6: 64 rows keep the oracle at a few seconds
@@ -246,18 +238,17 @@ def test_headless_cpp_host_matches_the_ctypes_path(rt, tmp_path):
     crt_launch for the nine kernel names of the frame, Stopwatch; host/crt_host.hpp) — renders the same frames as the
     Python host does through ctypes: accumulation bit for bit, in launch-list mode and with --fused"""
     exe = os.path.join(ROOT, "cedec-2024-rt_b200", "restir_di_headless")
-    scene = os.path.join(ROOT, "assets", "blocks_restir.tri.xz")
-    if not (os.path.exists(exe) and os.path.exists(scene)):
-        pytest.skip("C++ host or scene cache not built/staged")
-    tris = staged("blocks_restir")
+    tris = scene("blocks_restir")
+    tri_file = str(tmp_path / "blocks_restir.tri")
+    tris.tofile(tri_file)
     w, h, frames = 480, 270, 3
     kw = dict(accumulate=1, use_temporal_resampling=1, use_spatial_resampling=1)
     for fused in (False, True):
         out = str(tmp_path / ("acc_%d.f32" % fused))
-        cmd = [exe, "--scene", scene, "--size", str(w), str(h), "--frames", str(frames), "--dump-accum", out]
+        cmd = [exe, "--scene", tri_file, "--size", str(w), str(h), "--frames", str(frames), "--dump-accum", out]
         r = subprocess.run(cmd + (["--fused"] if fused else []), capture_output=True, text=True, timeout=600)
         assert r.returncode == 0, (r.stdout[-1000:], r.stderr[-2000:])
-        assert "lights: 145982" in r.stdout and "mean kernel time" in r.stdout
+        assert "lights: 145344" in r.stdout and "mean kernel time" in r.stdout
         theirs = np.fromfile(out, np.float32).reshape(-1, 4)
         # the C++ host leaves the library's default arithmetic (CRT_MATH_REFERENCE): so does this context
         rt.set_math_mode(cedecrt.MATH_REFERENCE)
@@ -400,7 +391,7 @@ def test_temporal_reprojection_bit_exact_with_a_moving_camera(rt, exact, port):
 def test_frame_overlap_changes_no_bit():
     """crt_set_frame_overlap: the tail of every frame (resolve rays + tone mapping) on a second stream, beside the next
     frame's raycast / candidate kernels — accumulation, RGBA8 and final reservoirs stay what the serial frames give"""
-    tris = staged("blocks_restir")
+    tris = scene("blocks_restir")
     w, h, frames = 960, 540, 5
     kw = dict(accumulate=1, use_temporal_resampling=1, use_spatial_resampling=1)
     serial, lapped = cedecrt.Runtime(0), cedecrt.Runtime(0)
@@ -447,8 +438,6 @@ def test_bench_frame_hash(rt):
     if not torch.cuda.is_available():
         pytest.skip("needs CUDA")
     tris, cam, _ = bench.load_workload()
-    if len(tris) != 9590208:
-        pytest.skip("blocks_restir cache not staged")
     torch.cuda.set_device(0)
     with torch.cuda.stream(torch.cuda.Stream()):
         one = slabs.SlabRenderer(torch, None, 0, 1, tris, cam, 3840, 2160, fused=True)
@@ -461,9 +450,9 @@ def test_bench_frame_hash(rt):
         group.close()
     assert h1["value"] == h3["value"]
     golden = json.load(open(os.path.join(ROOT, "tests", "golden", "frame_hash.json")))
-    print("frame_hash", h1["value"], "golden", golden.get("config5_4k"))
-    if golden.get("config5_4k"):
-        assert h1["value"] == golden["config5_4k"]
+    key = "config5_4k" if len(tris) == 9590208 else "procedural_4k"  # the staged scene or bench.py's stand-in
+    print("frame_hash", h1["value"], "golden", golden[key])
+    assert h1["value"] == golden[key]
 
 
 # ------------------------------------------------------------------ pipelined read-back (bench.py's e2e loop)

@@ -3,8 +3,10 @@
 The committed fixture's golden was produced by oracle/_ref/libref_loader.so (the reference loader itself):
     python -c "import sys; sys.path.insert(0,'oracle'); import orc, numpy as np; \
       np.save('tests/golden/obj/tricky_reference_loader.npy', orc.load_obj_reference('tests/golden/obj/tricky.obj','tests/golden/obj/'))"
+cornellbox1.obj and blocks_ao.obj (+ .mtl) hold two of the scenes the examples load, written back from the reference loader's
+Triangle[] in golden/scenes_small.npz (the original asset files are not part of the repository): one `v` per distinct
+position and one material per distinct (Kd, Ke), every value as printf("%.9g") of its float, faces in triangle order.
 """
-import lzma
 import os
 import subprocess
 
@@ -36,13 +38,9 @@ def test_missing_file_is_an_error(tmp_path):
     assert r.returncode == 1 and "cannot open" in r.stderr
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/assets/blocks_ao.obj"), reason="needs /root/reference")
-@pytest.mark.parametrize("scene", ["cornellbox1", "blocks_ao", "blocks_pt", "blocks_restir"])
+@pytest.mark.parametrize("scene", ["cornellbox1", "blocks_ao"])
 def test_reference_scenes_match_staged_caches(scene, tmp_path):
-    """the four scenes the examples load: identical to the bytes staged from the reference loader"""
-    cache = os.path.join(ROOT, "assets", scene + ".tri.xz")
-    if not os.path.exists(cache):
-        pytest.skip("scene cache not staged (python oracle/stage_assets.py)")
-    want = lzma.open(cache, "rb").read()
-    got = _convert("/root/reference/assets/%s.obj" % scene, tmp_path)
+    """two of the scenes the examples load: identical to the bytes of the reference loader (golden/scenes_small.npz)"""
+    want = np.load(os.path.join(ROOT, "tests", "golden", "scenes_small.npz"))[scene].tobytes()
+    got = _convert(os.path.join(OBJ, scene + ".obj"), tmp_path)
     assert got == want
