@@ -81,25 +81,65 @@ CRT_HD bool ray_triangle(f3 ro, f3 rd, float tmin, float tmax, f3 v0, f3 v1, f3 
     return true;
 }
 
-// The accept / reject decision of ray_triangle() alone, with every operation spelled as a single-rounding intrinsic, so
-// that the answer is the walk's own — bit for bit — in whatever translation unit it is compiled (the per-pixel kernels
-// of the REFERENCE and FAST builds contract a * b + c into FMAs; the walk's triangle test is never contracted).
+// The accept / reject decision of ray_triangle() alone, with every operation and comparison spelled as one PTX instruction
+// without .ftz, so that the answer is the walk's own — bit for bit — in whatever translation unit it is compiled.  The
+// per-pixel kernels of the REFERENCE and FAST builds contract a * b + c into FMAs, and the FAST build's -use_fast_math
+// implies -ftz=true, under which even __fmul_rn and a < 0.0f flush denormal operands and results to zero (a sub-area of
+// -1e-40 would compare as -0 and accept a triangle the walk rejects); the walk's triangle test is neither contracted nor
+// flushed (tests/test_gpu_math_modes.py: rays that leave a floor's edge and cross its plane a denormal distance outside).
 // Used for OWN-TRIANGLE PRE-TESTS: a per-pixel kernel that emits a shadow ray knows the triangle the ray starts on, and
 // in these scenes a third of the rays towards freshly sampled lights point below that triangle's plane (the reference's
 // target function takes |cos|, reservoir.hpp:42-59 / core.hpp:287-295, so such lights are legitimate candidates) and are
 // stopped by it at t ~ 1e-3.  An any-hit answer is "some triangle accepts": if this one does, the ray is occluded and
 // need not be traced.  Measured (profiles/bvh_lab/lab2.cpp, config 5): 30.6 % of the visibility-reuse rays, 34.5 % of
 // their node steps; 0.7 % of the resolve rays (not used there).
-#if defined(__CUDA_ARCH__)
+#if defined(__CUDA_ARCH__) && defined(CRT_FASTMATH_TU)
+// -ftz=true (kernels_fast.cu's FAST build): explicit PTX without .ftz.  Only here: in the builds without flushing the
+// intrinsics and plain comparisons below compile to the same operations, and the compiler folds the three sign tests
+// into one three-way minimum, which it cannot see through inline assembly.
+#define CRT_RN_OP(name, ptx)                                    \
+    __device__ __forceinline__ float name(float a, float b)    \
+    {                                                           \
+        float r;                                                \
+        asm(ptx " %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));     \
+        return r;                                               \
+    }
+CRT_RN_OP(rn_mul_f, "mul.rn.f32")
+CRT_RN_OP(rn_add_f, "add.rn.f32")
+CRT_RN_OP(rn_sub_f, "sub.rn.f32")
+CRT_RN_OP(rn_div_f, "div.rn.f32")
+#undef CRT_RN_OP
+// a < b and a <= b, IEEE (false for NaN), denormals compared as they are
+#define CRT_RN_CMP(name, ptx)                                                                          \
+    __device__ __forceinline__ bool name(float a, float b)                                             \
+    {                                                                                                  \
+        uint32_t r;                                                                                    \
+        asm("{ .reg .pred p; " ptx " p, %1, %2; selp.u32 %0, 1, 0, p; }" : "=r"(r) : "f"(a), "f"(b)); \
+        return r != 0u;                                                                                \
+    }
+CRT_RN_CMP(rn_lt_f, "setp.lt.f32")
+CRT_RN_CMP(rn_le_f, "setp.le.f32")
+#undef CRT_RN_CMP
+#define CRT_RN_MUL(a, b) rn_mul_f(a, b)
+#define CRT_RN_ADD(a, b) rn_add_f(a, b)
+#define CRT_RN_SUB(a, b) rn_sub_f(a, b)
+#define CRT_RN_DIV(a, b) rn_div_f(a, b)
+#define CRT_RN_LT(a, b) rn_lt_f(a, b)
+#define CRT_RN_LE(a, b) rn_le_f(a, b)
+#elif defined(__CUDA_ARCH__)
 #define CRT_RN_MUL(a, b) __fmul_rn(a, b)
 #define CRT_RN_ADD(a, b) __fadd_rn(a, b)
 #define CRT_RN_SUB(a, b) __fsub_rn(a, b)
 #define CRT_RN_DIV(a, b) __fdiv_rn(a, b)
+#define CRT_RN_LT(a, b) ((a) < (b))
+#define CRT_RN_LE(a, b) ((a) <= (b))
 #else
 #define CRT_RN_MUL(a, b) ((a) * (b))
 #define CRT_RN_ADD(a, b) ((a) + (b))
 #define CRT_RN_SUB(a, b) ((a) - (b))
 #define CRT_RN_DIV(a, b) ((a) / (b))
+#define CRT_RN_LT(a, b) ((a) < (b))
+#define CRT_RN_LE(a, b) ((a) <= (b))
 #endif
 CRT_HD f3 rn_sub(f3 a, f3 b) { return {CRT_RN_SUB(a.x, b.x), CRT_RN_SUB(a.y, b.y), CRT_RN_SUB(a.z, b.z)}; }
 CRT_HD f3 rn_cross(f3 a, f3 b)
@@ -113,12 +153,12 @@ CRT_HD bool segment_hits_triangle(f3 ro, f3 rd, float tmin, float tmax, f3 v0, f
     const f3 e0 = rn_sub(v1, v0), e1 = rn_sub(v2, v1), e2 = rn_sub(v0, v2);
     const f3 n = rn_cross(e0, e1);
     const float t = CRT_RN_DIV(rn_dot(rn_sub(v0, ro), n), rn_dot(n, rd));
-    if (!(tmin <= t && t <= tmax)) return false;
+    if (!(CRT_RN_LE(tmin, t) && CRT_RN_LE(t, tmax))) return false;
     const f3 p{CRT_RN_ADD(ro.x, CRT_RN_MUL(rd.x, t)), CRT_RN_ADD(ro.y, CRT_RN_MUL(rd.y, t)), CRT_RN_ADD(ro.z, CRT_RN_MUL(rd.z, t))};
     const float a0 = rn_dot(n, rn_cross(e0, rn_sub(p, v0)));
     const float a1 = rn_dot(n, rn_cross(e1, rn_sub(p, v1)));
     const float a2 = rn_dot(n, rn_cross(e2, rn_sub(p, v2)));
-    return !(a0 < 0.0f || a1 < 0.0f || a2 < 0.0f);
+    return !(CRT_RN_LT(a0, 0.0f) || CRT_RN_LT(a1, 0.0f) || CRT_RN_LT(a2, 0.0f));
 }
 
 struct u4 { uint32_t x, y, z, w; };
