@@ -106,6 +106,17 @@ extern "C" int crt_set_math_mode(crt_ctx* ctx, int mode)
     return CRT_OK;
 }
 
+extern "C" int crt_set_light_sampling(crt_ctx* ctx, int mode, int log2_slots)
+{
+    CRT_REQUIRE(ctx, "null context");
+    CRT_REQUIRE(mode == CRT_LIGHTS_UNIFORM || mode == CRT_LIGHTS_POWER, "unknown light sampling mode");
+    CRT_REQUIRE(log2_slots >= 0, "log2_slots must be 0 (the default) or the log2 of the slot count");
+    // whether 2^log2_slots fits the light count is checked by the first call that samples lights
+    ctx->light_mode = mode;
+    ctx->light_log2 = log2_slots;
+    return CRT_OK;
+}
+
 extern "C" int crt_set_row_range(crt_ctx* ctx, int y_begin, int y_end)
 {
     CRT_REQUIRE(ctx, "null context");

@@ -50,7 +50,9 @@ struct crt_ctx
     unsigned* queue2_counters = nullptr;
     size_t queue2_capacity = 0;
     int wavefront = 1;  // 0: trace shadow rays inside the per-pixel kernels (CRT_WAVEFRONT=0)
-    int light_table = 1;  // 0: sample lights through lights[] -> triangles[] like the reference (CRT_LIGHT_TABLE=0)
+    int light_table = 1;  // 0: sample lights through lights[] -> triangles[] like the reference (CRT_LIGHT_TABLE=0; uniform mode only)
+    int light_mode = CRT_LIGHTS_UNIFORM;  // crt_set_light_sampling
+    int light_log2 = 0;                   // requested log2 of the slot count of CRT_LIGHTS_POWER; 0: the default
     // fused frame (kernels_fast.cu): G-buffer + pixel-class plane, 25 bytes per pixel, grown on demand
     void* gbuf = nullptr;
     size_t gbuf_pixels = 0;
@@ -89,10 +91,15 @@ struct crt_geometry_t
     float build_ms = 0.0f;
     float pad = 0.0f;
     int device = 0;
-    // 64-byte light records (restir_core.cuh: LightRec) for the light list last seen by generate_candidate
+    // 64-byte light records (restir_core.cuh: LightRec) for the light list last seen by a light-sampling kernel: one per
+    // light, or one per slot of power-proportional selection (light_table_log2 = log2 K; -1: uniform)
     void* light_table = nullptr;
     const void* light_table_key = nullptr;
     size_t light_table_n = 0;
+    size_t light_table_cap = 0;  // records the allocation holds
+    int light_table_log2 = -1;
+    void* light_scratch = nullptr;  // the slot table's build scratch (geometry.cu: build_light_slots), grown on demand
+    size_t light_scratch_bytes = 0;
     float postpone_ratio = crt::kPostponeRatio;
     // refit (crt_refit_geometry): first node of every level of the wide tree, exact node boxes (allocated on demand)
     std::vector<uint32_t> level_begin;

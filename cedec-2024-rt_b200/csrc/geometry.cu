@@ -10,6 +10,7 @@
 
 #include "bvh_build.cuh"
 #include "ctx.cuh"
+#include "restir_core.cuh"
 
 namespace crt
 {
@@ -443,6 +444,84 @@ __global__ void __launch_bounds__(256) k_trace_brute(const float* tris60, uint32
         out_tuv[3 * ray + 2] = bv;
     }
 }
+
+// ---- the slot table of power-proportional light selection (restir_core.cuh: light_power .. slot_owner).  Rebuilt per
+// (geometry, light list, K) and after every refit or crt_lights_changed, so a host that animates emitters pays it per frame.
+__global__ void __launch_bounds__(kBuildBlock)
+    k_light_power(uint32_t n, const float* tris60, const uint32_t* lights, float* power, uint32_t* pmax_bits)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const float p = i < n ? light_power(tris60, CRT_LDG(lights + i)) : 0.0f;
+    if (i < n) power[i] = p;
+    // non-negative finite floats order like their bit patterns: the maximum is independent of the order of the atomics
+    const uint32_t m = __reduce_max_sync(0xffffffffu, __float_as_uint(p));
+    if ((threadIdx.x & 31) == 0 && m) atomicMax(pmax_bits, m);
+}
+__global__ void __launch_bounds__(kBuildBlock)
+    k_light_quantise(uint32_t n, const float* power, const uint32_t* pmax_bits, unsigned long long* q)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) q[i] = light_quantum(power[i], __uint_as_float(*pmax_bits));
+    else if (i == n) q[n] = 0ull;  // the exclusive scan's last element is then S = S_n
+}
+__global__ void __launch_bounds__(kBuildBlock)
+    k_light_starts(uint32_t n, uint32_t K, const unsigned long long* prefix, uint32_t* start)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) start[i] = light_start(i, n, K, prefix[i], prefix[n]);
+    else if (i == n) start[n] = K;
+}
+// one thread per slot: a binary search over the starts keeps the work even when one light owns most of the slots
+__global__ void __launch_bounds__(kBuildBlock)
+    k_light_slots(uint32_t K, uint32_t n, const uint32_t* start, const float* tris60, const uint32_t* lights, LightRec* table)
+{
+    for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s < K; s += gridDim.x * blockDim.x)
+    {
+        const uint32_t i = slot_owner(start, n, s);
+        table[s] = light_rec(tris60, CRT_LDG(lights + i), slot_sel(CRT_LDG(start + i + 1) - CRT_LDG(start + i), K));
+    }
+}
+int build_light_slots(crt_ctx* ctx, crt_geometry geom, const float* tris60, const uint32_t* lights, uint32_t n, int log2_slots,
+                      LightRec* table)
+{
+    const uint32_t K = 1u << log2_slots;
+    cudaStream_t st = ctx->stream;
+    size_t scan_bytes = 0;
+    CRT_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                           (int)n + 1, st));
+    // scratch: q and its prefix (n + 1 each), power (n), starts (n + 1), the maximum, CUB's temporary storage
+    const size_t q_bytes = ((size_t)n + 1) * 8, off_prefix = q_bytes, off_power = 2 * q_bytes,
+                 off_start = off_power + (((size_t)n * 4 + 255) & ~(size_t)255), off_max = off_start + ((((size_t)n + 1) * 4 + 255) & ~(size_t)255),
+                 off_tmp = off_max + 256, bytes = off_tmp + scan_bytes;
+    if (geom->light_scratch_bytes < bytes)
+    {
+        if (geom->light_scratch) CRT_CUDA(cudaFree(geom->light_scratch));
+        geom->light_scratch = nullptr;
+        geom->light_scratch_bytes = 0;
+        CRT_CUDA(cudaMalloc(&geom->light_scratch, bytes));
+        geom->light_scratch_bytes = bytes;
+    }
+    char* base = (char*)geom->light_scratch;
+    unsigned long long *q = (unsigned long long*)base, *prefix = (unsigned long long*)(base + off_prefix);
+    float* power = (float*)(base + off_power);
+    uint32_t *start = (uint32_t*)(base + off_start), *pmax = (uint32_t*)(base + off_max);
+    CRT_CUDA(cudaMemsetAsync(pmax, 0, 4, st));
+    k_light_power<<<div_up(n, kBuildBlock), kBuildBlock, 0, st>>>(n, tris60, lights, power, pmax);
+    int rc = check_launch(ctx, "light_power");
+    if (rc != CRT_OK) return rc;
+    k_light_quantise<<<div_up((size_t)n + 1, kBuildBlock), kBuildBlock, 0, st>>>(n, power, pmax, q);
+    rc = check_launch(ctx, "light_quantise");
+    if (rc != CRT_OK) return rc;
+    CRT_CUDA(cub::DeviceScan::ExclusiveSum(base + off_tmp, scan_bytes, q, prefix, (int)n + 1, st));
+    rc = check_launch(ctx, "light_scan");
+    if (rc != CRT_OK) return rc;
+    k_light_starts<<<div_up((size_t)n + 1, kBuildBlock), kBuildBlock, 0, st>>>(n, K, prefix, start);
+    rc = check_launch(ctx, "light_starts");
+    if (rc != CRT_OK) return rc;
+    const size_t want = div_up(K, kBuildBlock), cap = (size_t)ctx->sm_count * 16;
+    k_light_slots<<<(unsigned)(want < cap ? want : cap), kBuildBlock, 0, st>>>(K, n, start, tris60, lights, table);
+    return check_launch(ctx, "light_slots");
+}
 }  // namespace crt
 
 using namespace crt;
@@ -478,6 +557,13 @@ extern "C" int crt_refit_geometry(crt_ctx* ctx, crt_geometry g)
     return refit(ctx, g);
 }
 
+extern "C" int crt_lights_changed(crt_ctx* ctx, crt_geometry g)
+{
+    CRT_REQUIRE(ctx && g, "null context or geometry");
+    g->light_table_key = nullptr;  // the records (and in power mode the slot counts) are rebuilt at the next use
+    return CRT_OK;
+}
+
 extern "C" int crt_destroy_geometry(crt_ctx* ctx, crt_geometry g)
 {
     CRT_REQUIRE(ctx, "null context");
@@ -487,6 +573,7 @@ extern "C" int crt_destroy_geometry(crt_ctx* ctx, crt_geometry g)
     CRT_CUDA(cudaFree(g->tris));
     if (g->node_box) CRT_CUDA(cudaFree(g->node_box));
     if (g->light_table) CRT_CUDA(cudaFree(g->light_table));
+    if (g->light_scratch) CRT_CUDA(cudaFree(g->light_scratch));
     delete g;
     return CRT_OK;
 }

@@ -131,15 +131,15 @@ __device__ __forceinline__ void count_rays(unsigned long long* counters, uint32_
         if (s) atomicAdd(counters + 1, (unsigned long long)s);
     }
 }
-template <int EX, int MODE>
+template <int EX, int MODE, class LS>
 __global__ void __launch_bounds__(256)
-    k_path_trace(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const uint32_t* lights, uint32_t n_lights,
+    k_path_trace(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const typename LS::Elem* lights, uint32_t n_lights,
                  crt_raygen raygen, crt_options options, crt_float4* accum, unsigned long long* ray_counters)
 {
     const TilePix t = this_pixel(W, H, rows);
     uint32_t n = 0;
     if (t.in)
-        n = px_path_trace<EX, Math<MODE>>(t.px, W, H, frame, bvh, tris60, lights, n_lights, raygen, make_opt(options), accum);
+        n = px_path_trace<EX, Math<MODE>, LS>(t.px, W, H, frame, bvh, tris60, lights, n_lights, raygen, make_opt(options), accum);
     count_rays(ray_counters, n & 0xffffu, n >> 16);
 }
 template <int MODE>
@@ -359,12 +359,13 @@ extern "C" int crt_generate_candidate(crt_ctx* ctx, int W, int H, int frame, crt
     }
     const dim3 grid = tile_grid(W, rows);
     const bool sh = options.use_shadowed_target_function != 0;
-    if (ctx->light_table)
+    if (use_light_table(ctx))
     {
         const LightRec* table = nullptr;
-        const int rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table);
+        uint32_t n_slots = 0;
+        const int rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table, &n_slots);
         if (rc != CRT_OK) return rc;
-        const LightsTable L{table, n_lights};
+        const LightsTable L{table, n_slots};
         if (wf) { if (sh) k_generate_candidate<LightsTable, true, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LightsTable, true, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
         else { if (sh) k_generate_candidate<LightsTable, false, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LightsTable, false, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
     }
@@ -377,6 +378,20 @@ extern "C" int crt_generate_candidate(crt_ctx* ctx, int W, int H, int frame, crt
     int rc = check_launch(ctx, "generate_candidate");
     if (rc != CRT_OK || !wf) return rc;
     return queue_trace<kEpiReservoirVisibility>(ctx, geom, q, ShadowSink{res, nullptr, 0, nullptr});
+}
+
+extern "C" int crt_light_sampling_table(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, const void** d_records, uint32_t* n_slots)
+{
+    CRT_REQUIRE(ctx && geom && d_records && n_slots, "null argument");
+    CRT_REQUIRE(bsize(lights) == 0 || lights.data != nullptr, "null light buffer");
+    CRT_REQUIRE(bsize(lights) < 0xffffffffull, "too many lights");
+    CRT_REQUIRE(geom->src != nullptr, "geometry has no triangle array");
+    CRT_JOIN_TAIL(ctx);
+    const LightRec* table = nullptr;
+    const int rc = light_table_for(ctx, geom, (const float*)geom->src, (const uint32_t*)lights.data, bsize(lights), &table, n_slots);
+    if (rc != CRT_OK) return rc;
+    *d_records = table;
+    return CRT_OK;
 }
 
 extern "C" int crt_temporal_resampling(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,
@@ -566,14 +581,29 @@ static int path_trace(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, 
     CRT_REQUIRE(EX == 7 || bsize(lights) == 0 || lights.data != nullptr, "null light buffer");
     CRT_JOIN_TAIL(ctx);
     unsigned long long* counters = nullptr;
-    const int rc = inline_ray_counters(ctx, &counters);
+    int rc = inline_ray_counters(ctx, &counters);
     if (rc != CRT_OK) return rc;
+    const LightRec* slots = nullptr;  // power-proportional selection: the slot table (uniform: lights[] as the reference)
+    uint32_t n_slots = 0;
+    if (EX != 7 && ctx->light_mode == CRT_LIGHTS_POWER && bsize(lights))
+    {
+        CRT_REQUIRE(bsize(lights) < 0xffffffffull, "too many lights");
+        rc = light_table_for(ctx, geom, (const float*)triangles.data, (const uint32_t*)lights.data, bsize(lights), &slots, &n_slots);
+        if (rc != CRT_OK) return rc;
+    }
     // the wavefront form (kernels_paths.cu) packs path | ray << 27 into a record word and keeps a 32-bit visibility mask per vertex
     const bool wave_ok = (size_t)W * H < ((size_t)1 << 27) && (!options.use_shadowed_target_function || options.ris_sample_count <= 32);
     if (ctx->wavefront && wave_ok)
         return path_trace_wavefront(ctx, EX, W, H, frame, geom, (const float*)triangles.data, (const uint32_t*)lights.data,
-                                    (uint32_t)bsize(lights), raygen, options, (crt_float4*)accumulation.data, counters);
-    auto k = ctx->math_mode == CRT_MATH_EXACT ? k_path_trace<EX, 1> : k_path_trace<EX, 0>;
+                                    (uint32_t)bsize(lights), slots, n_slots, raygen, options, (crt_float4*)accumulation.data, counters);
+    if (slots)
+    {
+        auto k = ctx->math_mode == CRT_MATH_EXACT ? k_path_trace<EX, 1, LightsTable> : k_path_trace<EX, 0, LightsTable>;
+        k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
+                                                   slots, n_slots, raygen, options, (crt_float4*)accumulation.data, counters);
+        return check_launch(ctx, "path_trace");
+    }
+    auto k = ctx->math_mode == CRT_MATH_EXACT ? k_path_trace<EX, 1, LightsIndexed> : k_path_trace<EX, 0, LightsIndexed>;
     k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
                                                (const uint32_t*)lights.data, (uint32_t)bsize(lights), raygen, options,
                                                (crt_float4*)accumulation.data, counters);

@@ -400,9 +400,10 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     const bool exact = ctx->math_mode == CRT_MATH_EXACT;
     const HaloPeers peers = halo_peers(ctx, 0, rows, true, n);
     const LightRec* table = nullptr;
-    if (ctx->light_table)
+    uint32_t n_slots = n_lights;
+    if (use_light_table(ctx))
     {
-        rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table);
+        rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table, &n_slots);
         if (rc != CRT_OK) return rc;
     }
     Reprojection rp;
@@ -426,7 +427,7 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     }
     CRT_MODE_NS(ctx, launch_candidate_temporal)(
         ctx->stream, exact, grid, W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), table,
-        (const uint32_t*)lights.data, n_lights, options, T, g, q, peers, reproject ? &rp : nullptr);
+        (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr);
     rc = check_launch(ctx, "candidate_temporal");
     if (rc != CRT_OK || !options.use_visibility_reuse) return rc;
     ShadowSink sink{nullptr, nullptr, 0, (uint32_t*)T.plane(0, 0)};

@@ -167,9 +167,11 @@ __device__ __forceinline__ uint32_t reserve_rays(const ShadowQueue& q, bool emit
 }
 
 // EX 7 / 8 / 9: the vertex of every live path after its closest-hit walk (07_pt.cu:36-70, 08_nee.cu:40-80, 09_ris.cu:40-100)
-template <int EX, int MODE>
+// LS: the light source — LightsIndexed over the reference's light list (uniform selection) or LightsTable over the slot
+// table of power-proportional selection (n_lights = K, restir_core.cuh)
+template <int EX, int MODE, class LS>
 __global__ void __launch_bounds__(256)
-    k_pt_vertex(int W, int H, Rows rows, int depth, Bvh bvh, const float* tris60, const uint32_t* lights, uint32_t n_lights,
+    k_pt_vertex(int W, int H, Rows rows, int depth, Bvh bvh, const float* tris60, const typename LS::Elem* lights, uint32_t n_lights,
                 crt_options options, PathState st, ShadowQueue q, unsigned long long* ray_counters)
 {
     const TilePix t = this_pixel(W, H, rows);
@@ -232,7 +234,7 @@ __global__ void __launch_bounds__(256)
     }
     if (EX == 7) return;
     const bool shadowed = EX == 9 && opt.shadowed;
-    const LightsIndexed L{tris60, lights, n_lights};
+    const LS L = LS::at(tris60, lights, n_lights);
     const f3 org = surf.p + 0.001f * surf.n;  // check_visibility's segment (raytrace.hpp:45-52): direction p1 - p0, t in [0, 0.99]
     Pcg rng(0, 0);
     if (lit)
@@ -338,9 +340,9 @@ __global__ void __launch_bounds__(256)
 }
 
 // shadowed 09_ris: Reservoir::update over the candidates with their visibilities, then the ray towards the selected sample
-template <int MODE>
+template <int MODE, class LS>
 __global__ void __launch_bounds__(256)
-    k_pt_replay(int W, int H, Rows rows, Bvh bvh, const float* tris60, const uint32_t* lights, uint32_t n_lights, crt_options options,
+    k_pt_replay(int W, int H, Rows rows, Bvh bvh, const float* tris60, const typename LS::Elem* lights, uint32_t n_lights, crt_options options,
                 PathState st, ShadowQueue q, unsigned long long* ray_counters)
 {
     const TilePix t = this_pixel(W, H, rows);
@@ -357,7 +359,7 @@ __global__ void __launch_bounds__(256)
     const float4 rot = st.ro_t[idx], rdp = st.rd_prim[idx];
     const TriRef tri = tri_at(tris60, prim);
     const Surf surf = surface_from_hit(tri, xyz(rot), xyz(rdp), rot.w);
-    const LightsIndexed L{tris60, lights, n_lights};
+    const LS L = LS::at(tris60, lights, n_lights);
     Pcg rng = pcg_from_state(st.rng_snap[idx]);
     const uint32_t vmask = st.vmask[idx];
     Res r = empty_res();
@@ -372,7 +374,8 @@ __global__ void __launch_bounds__(256)
         // target function with visibility, in the reference's order: ((1/pi * G) * V) * luminance (reservoir.hpp:42-59)
         const float V = ((vmask >> c) & 1u) ? 1.0f : 0.0f;
         const float p_hat = kInvPi * geometry_term(surf.p, surf.n, ls.p, ls.n) * V * luminance(ls.emissive);
-        ris_apply(surf, ls, inv_n, u, p_hat, r);
+        if (LS::kHasPdf) ris_apply_pdf(surf, ls, ls.pdf, u, p_hat, r);
+        else ris_apply(surf, ls, inv_n, u, p_hat, r);
     }
     st.sel0[idx] = make_float4(r.s.hp.x, r.s.hp.y, r.s.hp.z, r.w_sum);
     st.sel1[idx] = make_float4(r.s.hn.x, r.s.hn.y, r.s.hn.z, __int_as_float(r.M));
@@ -382,9 +385,9 @@ __global__ void __launch_bounds__(256)
 }
 
 // 08_nee.cu:66-106 / 09_ris.cu:102-150: the vertex's radiance with the traced visibility, then the bounce
-template <int EX, int MODE>
+template <int EX, int MODE, class LS>
 __global__ void __launch_bounds__(256)
-    k_pt_shade_bounce(int W, int H, Rows rows, Bvh bvh, const float* tris60, const uint32_t* lights, uint32_t n_lights,
+    k_pt_shade_bounce(int W, int H, Rows rows, Bvh bvh, const float* tris60, const typename LS::Elem* lights, uint32_t n_lights,
                       crt_options options, PathState st)
 {
     const TilePix t = this_pixel(W, H, rows);
@@ -407,11 +410,11 @@ __global__ void __launch_bounds__(256)
         const float r0 = rs.next_f();
         const float r1 = rs.next_f();
         const float r2 = rs.next_f();
-        const LightSample ls = LightsIndexed{tris60, lights, n_lights}.sample(r0, r1, r2);
+        const LightSample ls = LS::at(tris60, lights, n_lights).sample(r0, r1, r2);
         const float V = (st.vmask[idx] & 1u) ? 1.0f : 0.0f;
         const f3 brdf = kInvPi * color;
         const float G = geometry_term(surf.p, surf.n, ls.p, ls.n);
-        const float light_pdf = 1.0f / (float)n_lights * 1.0f / ls.area;
+        const float light_pdf = light_pdf_of<LS>(ls, n_lights);
         radiance = radiance + thr * brdf * G * V * ls.emissive / light_pdf;
     }
     else
@@ -473,9 +476,9 @@ static int path_state(crt_ctx* ctx, size_t n, PathState* st)
     return CRT_OK;
 }
 
-template <int EX, int MODE>
+template <int EX, int MODE, class LS>
 static int path_trace_wavefront_impl(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, const float* tris60,
-                                     const uint32_t* lights, uint32_t n_lights, crt_raygen raygen, crt_options options,
+                                     const typename LS::Elem* lights, uint32_t n_lights, crt_raygen raygen, crt_options options,
                                      crt_float4* accum, unsigned long long* counters)
 {
     const Rows all = rows_of(ctx, H);
@@ -533,7 +536,7 @@ static int path_trace_wavefront_impl(crt_ctx* ctx, int W, int H, int frame, crt_
                 if (rc != CRT_OK) break;
                 q.stride4 = 2;
             }
-            k_pt_vertex<EX, MODE><<<grid, 256, 0, ctx->stream>>>(W, H, rows, depth, bvh, tris60, lights, n_lights, options, st, q, counters);
+            k_pt_vertex<EX, MODE, LS><<<grid, 256, 0, ctx->stream>>>(W, H, rows, depth, bvh, tris60, lights, n_lights, options, st, q, counters);
             rc = check_launch(ctx, "pt_vertex");
             if (rc != CRT_OK || EX == 7) continue;
             ShadowSink sink{nullptr, nullptr, 0, nullptr};
@@ -545,14 +548,14 @@ static int path_trace_wavefront_impl(crt_ctx* ctx, int W, int H, int frame, crt_
                 rc = queue_prepare(ctx, (n_px + 1) / 2, &q);
                 if (rc != CRT_OK) break;
                 q.stride4 = 2;
-                k_pt_replay<MODE><<<grid, 256, 0, ctx->stream>>>(W, H, rows, bvh, tris60, lights, n_lights, options, st, q, counters);
+                k_pt_replay<MODE, LS><<<grid, 256, 0, ctx->stream>>>(W, H, rows, bvh, tris60, lights, n_lights, options, st, q, counters);
                 rc = check_launch(ctx, "pt_replay");
                 if (rc != CRT_OK) break;
                 sink.visible_count = st.vfinal;
                 rc = queue_trace<kEpiBitmask>(ctx, geom, q, sink);
                 if (rc != CRT_OK) break;
             }
-            k_pt_shade_bounce<EX, MODE><<<grid, 256, 0, ctx->stream>>>(W, H, rows, bvh, tris60, lights, n_lights, options, st);
+            k_pt_shade_bounce<EX, MODE, LS><<<grid, 256, 0, ctx->stream>>>(W, H, rows, bvh, tris60, lights, n_lights, options, st);
             rc = check_launch(ctx, "pt_shade_bounce");
         }
         if (rc != CRT_OK) return rc;
@@ -564,15 +567,17 @@ static int path_trace_wavefront_impl(crt_ctx* ctx, int W, int H, int frame, crt_
 }
 
 int path_trace_wavefront(crt_ctx* ctx, int example, int W, int H, int frame, crt_geometry geom, const float* tris60,
-                         const uint32_t* lights, uint32_t n_lights, crt_raygen raygen, crt_options options, crt_float4* accum,
-                         unsigned long long* counters)
+                         const uint32_t* lights, uint32_t n_lights, const LightRec* slots, uint32_t n_slots, crt_raygen raygen,
+                         crt_options options, crt_float4* accum, unsigned long long* counters)
 {
     const bool ex = ctx->math_mode == CRT_MATH_EXACT;
-#define CRT_PT(EX) (ex ? path_trace_wavefront_impl<EX, 1>(ctx, W, H, frame, geom, tris60, lights, n_lights, raygen, options, accum, counters) \
-                       : path_trace_wavefront_impl<EX, 0>(ctx, W, H, frame, geom, tris60, lights, n_lights, raygen, options, accum, counters))
-    if (example == 7) return CRT_PT(7);
+#define CRT_PT_LS(EX, LS, P, N) (ex ? path_trace_wavefront_impl<EX, 1, LS>(ctx, W, H, frame, geom, tris60, P, N, raygen, options, accum, counters) \
+                                    : path_trace_wavefront_impl<EX, 0, LS>(ctx, W, H, frame, geom, tris60, P, N, raygen, options, accum, counters))
+#define CRT_PT(EX) (slots ? CRT_PT_LS(EX, LightsTable, slots, n_slots) : CRT_PT_LS(EX, LightsIndexed, lights, n_lights))
+    if (example == 7) return CRT_PT_LS(7, LightsIndexed, lights, n_lights);
     if (example == 8) return CRT_PT(8);
     return CRT_PT(9);
 #undef CRT_PT
+#undef CRT_PT_LS
 }
 }  // namespace crt

@@ -116,16 +116,36 @@ static int queue_trace(crt_ctx* ctx, crt_geometry geom, const ShadowQueue& q, co
     k_trace_shadow_queue<EPI><<<blocks_per_sm * ctx->sm_count, kShadowWarps * 32, 0, st>>>(geom->view(), q, sink);
     return check_launch(ctx, EPI == kEpiCountVisible ? "trace_ao" : EPI == kEpiBitmask ? "trace_shadow" : (EPI == kEpiReservoirVisibility || EPI == kEpiSoaVisibility) ? "trace_visibility_reuse" : "trace_resolve", st);
 }
-// light records for (geometry, light list); rebuilt when another list is passed
+// power-proportional slot table of 2^log2_slots records (geometry.cu)
+int build_light_slots(crt_ctx* ctx, crt_geometry geom, const float* tris60, const uint32_t* lights, uint32_t n, int log2_slots,
+                      LightRec* table);
+// light records for (geometry, light list, selection mode, K): one per light (uniform selection) or one per slot
+// (CRT_LIGHTS_POWER); *n_out is the count LightsTable draws over, n or K.  Rebuilt when any of the four changes.
 static int light_table_for(crt_ctx* ctx, crt_geometry geom, const float* tris60, const uint32_t* lights, size_t n,
-                           const LightRec** out)
+                           const LightRec** out, uint32_t* n_out)
 {
-    if (geom->light_table_key != lights || geom->light_table_n != n)
+    const bool power = ctx->light_mode == CRT_LIGHTS_POWER && n > 0;
+    const int k = power ? light_slots_log2(n, ctx->light_log2) : -1;
+    CRT_REQUIRE(!power || k >= 0, n > ((size_t)1 << kMaxLightSlotsLog2) ? "power light selection takes at most 2^23 lights"
+                                                                          : "log2_slots: 2^k must be at least the light count, k at most 23");
+    const size_t count = power ? (size_t)1 << k : n;
+    if (geom->light_table_key != lights || geom->light_table_n != n || geom->light_table_log2 != k)
     {
-        if (geom->light_table) CRT_CUDA(cudaFree(geom->light_table));
-        geom->light_table = nullptr;
-        CRT_CUDA(cudaMalloc(&geom->light_table, (n ? n : 1) * sizeof(LightRec)));
-        if (n)
+        geom->light_table_key = nullptr;
+        if (geom->light_table_cap < (count ? count : 1))  // a rebuild of the same size (refit, new emission) reuses the memory
+        {
+            if (geom->light_table) CRT_CUDA(cudaFree(geom->light_table));
+            geom->light_table = nullptr;
+            geom->light_table_cap = 0;
+            CRT_CUDA(cudaMalloc(&geom->light_table, (count ? count : 1) * sizeof(LightRec)));
+            geom->light_table_cap = count ? count : 1;
+        }
+        if (power)
+        {
+            const int rc = build_light_slots(ctx, geom, tris60, lights, (uint32_t)n, k, (LightRec*)geom->light_table);
+            if (rc != CRT_OK) return rc;
+        }
+        else if (n)
         {
             k_build_light_table<<<div_up(n, 256), 256, 0, ctx->stream>>>((uint32_t)n, tris60, lights, (LightRec*)geom->light_table);
             const int rc = check_launch(ctx, "build_light_table");
@@ -133,18 +153,23 @@ static int light_table_for(crt_ctx* ctx, crt_geometry geom, const float* tris60,
         }
         geom->light_table_key = lights;
         geom->light_table_n = n;
+        geom->light_table_log2 = k;
     }
     *out = (const LightRec*)geom->light_table;
+    *n_out = (uint32_t)count;
     return CRT_OK;
 }
+// every kernel that samples lights reads the table in power mode; in uniform mode CRT_LIGHT_TABLE=0 reads lights[] instead
+inline bool use_light_table(const crt_ctx* ctx) { return ctx->light_table || ctx->light_mode == CRT_LIGHTS_POWER; }
 }  // namespace crt
 
 namespace crt
 {
 // force the (lazily loaded) kernels of a translation unit into the context; see crt_slab_set_links
+// slots != nullptr: examples 08 / 09 select lights from the power-proportional slot table (n_slots records)
 int path_trace_wavefront(crt_ctx* ctx, int example, int W, int H, int frame, crt_geometry geom, const float* tris60,
-                         const uint32_t* lights, uint32_t n_lights, crt_raygen raygen, crt_options options, crt_float4* accum,
-                         unsigned long long* counters);
+                         const uint32_t* lights, uint32_t n_lights, const LightRec* slots, uint32_t n_slots, crt_raygen raygen,
+                         crt_options options, crt_float4* accum, unsigned long long* counters);
 int raycast_or_prefetched(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_buffer triangles, crt_raygen raygen, crt_buffer visibility);
 int tone_mapping_on(crt_ctx* ctx, cudaStream_t st, crt_buffer pixels, crt_buffer accumulation, int W, int H);
 int preload_fused_kernels();

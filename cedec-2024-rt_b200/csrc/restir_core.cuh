@@ -148,6 +148,8 @@ struct LightsIndexed
         return ls;
     }
     CRT_HD LightSample sample(float rv0, float rv1, float rv2) const { return finish(fetch(rv0), rv1, rv2); }
+    using Elem = uint32_t;
+    static CRT_HD LightsIndexed at(const float* tris60, const uint32_t* lights, uint32_t n) { return LightsIndexed{tris60, lights, n}; }
 };
 struct alignas(16) LightRec  // 64 bytes
 {
@@ -156,6 +158,18 @@ struct alignas(16) LightRec  // 64 bytes
     float v2x, v2y, v2z, ny;
     float ex, ey, ez, nz;
 };
+// the record of a light selected with probability `sel`
+CRT_HD LightRec light_rec(const float* tris60, uint32_t tri_index, float sel)
+{
+    const TriRef t = tri_at(tris60, (int)tri_index);
+    const f3 v0 = t.v(0), v1 = t.v(1), v2 = t.v(2), e = t.emissive();
+    const f3 c = cross(v1 - v0, v2 - v0);
+    const float len = length(c);
+    const f3 n = c / len;
+    return LightRec{v0.x, v0.y, v0.z, sel * 1.0f / (0.5f * len), v1.x, v1.y, v1.z, n.x, v2.x, v2.y, v2.z, n.y, e.x, e.y, e.z, n.z};
+}
+// the uniform record, sel = 1/n (kept as its own function: written through light_rec, nvcc schedules the division
+// differently and k_build_light_table's SASS changes)
 CRT_HD LightRec make_light_rec(const float* tris60, uint32_t tri_index, uint32_t n_lights)
 {
     const TriRef t = tri_at(tris60, (int)tri_index);
@@ -166,6 +180,56 @@ CRT_HD LightRec make_light_rec(const float* tris60, uint32_t tri_index, uint32_t
     const float inv_n = 1.0f / (float)n_lights;  // as ris_candidates computes it
     return LightRec{v0.x, v0.y, v0.z, inv_n * 1.0f / (0.5f * len), v1.x, v1.y, v1.z, n.x, v2.x, v2.y, v2.z, n.y, e.x, e.y, e.z, n.z};
 }
+
+// ---- power-proportional light selection (crt_set_light_sampling, CRT_LIGHTS_POWER; DESIGN.md section 14).  Light i
+// owns the slots [start_i, start_{i+1}) of a table of K = 2^k slots, n <= K <= 2^23, and slot s holds light_rec(...,
+// slot_sel(c_i, K)), c_i = start_{i+1} - start_i >= 1.  LightsTable{slots, K} draws nth = (uint32)(rv0 * (float)K): rv0
+// is a multiple of 2^-23, so every slot has probability exactly 1/K and light i exactly c_i / K, the record's `sel`.
+// The slot counts are computed in integers from quantised powers, so that they do not depend on summation order: the
+// host's restatement (the CPU specification) and this device build produce the same table bit for bit.
+constexpr int kMaxLightSlotsLog2 = 23;
+// log2 K for n lights: requested (1..23, 2^k >= n) or, for 0, min(23, ceil(log2 n) + 2); -1 when none fits
+CRT_HD int light_slots_log2(uint64_t n, int requested)
+{
+    if (requested == 0)
+    {
+        int c = 0;
+        while (((uint64_t)1 << c) < n) c++;
+        if (c > kMaxLightSlotsLog2) return -1;  // more than 2^23 lights
+        return c + 2 < kMaxLightSlotsLog2 ? c + 2 : kMaxLightSlotsLog2;
+    }
+    if (requested < 0 || requested > kMaxLightSlotsLog2 || ((uint64_t)1 << requested) < n) return -1;
+    return requested;
+}
+// P_i = max(0, luminance(Le_i)) * area_i; non-finite -> 0 (so every value compares as an unsigned integer)
+CRT_HD float light_power(const float* tris60, uint32_t tri_index)
+{
+    const TriRef t = tri_at(tris60, (int)tri_index);
+    const float l = luminance(t.emissive());
+    const float p = (l > 0.0f ? l : 0.0f) * tri_area(t.v(0), t.v(1), t.v(2));
+    return p <= kFltMax ? p : 0.0f;
+}
+// q_i = trunc((P_i / Pmax) * 2^32)
+CRT_HD uint64_t light_quantum(float p, float pmax) { return pmax > 0.0f ? (uint64_t)((p / pmax) * 4294967296.0f) : 0u; }
+// start_i = i + floor(R * S_i / S), R = K - n, S_i = sum_{j<i} q_j (R S_i < 2^78: 128-bit); S = 0: i + floor(R i / n)
+CRT_HD uint32_t light_start(uint32_t i, uint32_t n, uint32_t K, uint64_t s_i, uint64_t s)
+{
+    const uint64_t R = (uint64_t)K - n;
+    return i + (uint32_t)(s ? (uint64_t)((unsigned __int128)R * s_i / s) : R * i / n);
+}
+// the light that owns slot s: the last i with start[i] <= s (start[0] = 0, strictly increasing)
+CRT_HD uint32_t slot_owner(const uint32_t* start, uint32_t n, uint32_t s)
+{
+    uint32_t lo = 0, hi = n - 1;
+    while (lo < hi)
+    {
+        const uint32_t mid = lo + (hi - lo + 1) / 2;
+        if (CRT_LDG(start + mid) <= s) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+CRT_HD float slot_sel(uint32_t c, uint32_t K) { return (float)c * (1.0f / (float)K); }
 struct LightsTable
 {
     const LightRec* table;
@@ -237,7 +301,16 @@ struct LightsTable
         return ls;
     }
     CRT_HD LightSample sample(float rv0, float rv1, float rv2) const { return finish(fetch(rv0), rv1, rv2); }
+    using Elem = LightRec;
+    static CRT_HD LightsTable at(const float*, const LightRec* table, uint32_t n) { return LightsTable{table, n}; }
 };
+// the pdf the reference divides a light sample by: 1.0f / size * 1.0f / area (08_nee.cu, 10_restir_di.cu:98-99), or the
+// record's own (LightsTable)
+template <class L>
+CRT_HD float light_pdf_of(const LightSample& ls, uint32_t n)
+{
+    return L::kHasPdf ? ls.pdf : 1.0f / (float)n * 1.0f / ls.area;
+}
 CRT_HD float geometry_term(f3 p0, f3 n0, f3 p1, f3 n1)  // core.hpp:287-295
 {
     f3 v = p1 - p0;
@@ -407,7 +480,8 @@ CRT_HD Res ris_candidates_shadowed(const Bvh& bvh, const L& lights, const Surf& 
             if (state != kWalkContinue)
             {
                 const float V = state == kWalkHitAny ? 0.0f : 1.0f;
-                ris_apply(surf, ls, inv_n, u, inv_pi_g * V * luminance(ls.emissive), r);
+                if (L::kHasPdf) ris_apply_pdf(surf, ls, ls.pdf, u, inv_pi_g * V * luminance(ls.emissive), r);
+                else ris_apply(surf, ls, inv_n, u, inv_pi_g * V * luminance(ls.emissive), r);
                 ++c;
                 walking = false;
             }

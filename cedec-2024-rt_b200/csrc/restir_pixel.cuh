@@ -295,9 +295,10 @@ CRT_HD DeferredRay px_resolve(const Pix& px, crt_float4* accum, const Bvh& bvh, 
 // ---- 07_pt.cu:11-90 (EX = 7), 08_nee.cu:11-129 (EX = 8), 09_ris.cu:11-166 (EX = 9)
 // Returns the rays this pixel traced: closest-hit (camera + bounce rays) in the low 16 bits, shadow rays in the high 16
 // (SURVEY.md section 8d: 08_nee 1 + 1 per path vertex; 09_ris 1 + 1, or 1 + 32 + 1 + 1 with the shadowed target function).
-template <int EX, class M>
+// LS: the light source, see k_pt_vertex (kernels_paths.cu)
+template <int EX, class M, class LS = LightsIndexed>
 CRT_HD uint32_t px_path_trace(const Pix& px, int W, int H, int frame, const Bvh& bvh, const float* tris60,
-                              const uint32_t* lights, uint32_t n_lights, const crt_raygen& raygen, const Opt& opt,
+                              const typename LS::Elem* lights, uint32_t n_lights, const crt_raygen& raygen, const Opt& opt,
                               crt_float4* accum)
 {
     uint32_t n_closest = 0, n_shadow = 0;
@@ -328,17 +329,17 @@ CRT_HD uint32_t px_path_trace(const Pix& px, int W, int H, int frame, const Bvh&
             const float r0 = rng.next_f();
             const float r1 = rng.next_f();
             const float r2 = rng.next_f();
-            const LightSample ls = LightsIndexed{tris60, lights, n_lights}.sample(r0, r1, r2);
+            const LightSample ls = LS::at(tris60, lights, n_lights).sample(r0, r1, r2);
             ++n_shadow;
             const float V = check_visibility(bvh, surf.p, surf.n, ls.p);
             const f3 brdf = kInvPi * color;
             const float G = geometry_term(surf.p, surf.n, ls.p, ls.n);
-            const float light_pdf = 1.0f / (float)n_lights * 1.0f / ls.area;
+            const float light_pdf = light_pdf_of<LS>(ls, n_lights);
             radiance = radiance + throughput * brdf * G * V * ls.emissive / light_pdf;
         }
         else if (EX == 9)
         {
-            const Res r = ris_candidates(bvh, LightsIndexed{tris60, lights, n_lights}, surf, opt.ris_count, opt.shadowed, rng);
+            const Res r = ris_candidates(bvh, LS::at(tris60, lights, n_lights), surf, opt.ris_count, opt.shadowed, rng);
             n_shadow += 1u + (opt.shadowed ? (uint32_t)(opt.ris_count > 0 ? opt.ris_count : 0) + 1u : 0u);
             const f3 brdf = kInvPi * color;
             const float G = geometry_term(surf.p, surf.n, r.s.hp, r.s.hn);

@@ -48,6 +48,8 @@ class Device
     const char* name() const { return crt_device_name(m_ctx); }
     void synchronize() const { CRT_CHECKED(crt_sync(m_ctx)); }
     void setRowRange(int y0, int y1) const { CRT_CHECKED(crt_set_row_range(m_ctx, y0, y1)); }
+    // CRT_LIGHTS_UNIFORM (the reference) or CRT_LIGHTS_POWER; log2_slots = 0: the default slot count
+    void setLightSampling(int mode, int log2_slots = 0) const { CRT_CHECKED(crt_set_light_sampling(m_ctx, mode, log2_slots)); }
 
    private:
     crt_ctx* m_ctx = nullptr;

@@ -29,6 +29,7 @@ FLOAT4 = np.dtype((np.float32, (4,)))
 assert TRIANGLE.itemsize == 60 and VISIBILITY.itemsize == 16 and RESERVOIR.itemsize == 76
 
 MATH_LIBDEVICE, MATH_EXACT, MATH_FAST, MATH_REFERENCE = 0, 1, 2, 3  # include/cedecrt.h: CRT_MATH_*
+LIGHTS_UNIFORM, LIGHTS_POWER = 0, 1  # include/cedecrt.h: CRT_LIGHTS_*
 
 
 class Float3(C.Structure):
@@ -120,6 +121,9 @@ def _load():
         "crt_init": [I, C.POINTER(C.c_void_p)],
         "crt_shutdown": [P],
         "crt_set_math_mode": [P, I],
+        "crt_set_light_sampling": [P, I, I],
+        "crt_light_sampling_table": [P, G, B, C.POINTER(C.c_void_p), C.POINTER(C.c_uint32)],
+        "crt_lights_changed": [P, G],
         "crt_set_stream": [P, C.c_void_p],
         "crt_set_frame_overlap": [P, I],
         "crt_frame_join": [P],
@@ -322,6 +326,26 @@ class Runtime:
     def set_math_mode(self, mode):
         self._check(self.lib.crt_set_math_mode(self.ctx, mode))
         self.math_mode = mode
+
+    def set_light_sampling(self, mode, log2_slots=0):
+        """LIGHTS_UNIFORM (the reference, default) or LIGHTS_POWER: select lights in proportion to their emitted power from
+        a table of 2^log2_slots slots (0: the default size; include/cedecrt.h: crt_set_light_sampling)"""
+        self._check(self.lib.crt_set_light_sampling(self.ctx, mode, log2_slots))
+        self.light_mode, self.light_log2 = mode, log2_slots
+
+    def light_sampling_table(self, geom, lights):
+        """the light records the kernels read for `lights` (a TypedBuffer of uint32 triangle indices), copied to the host as
+        a float32 array of shape (n_slots, 16)"""
+        ptr, n = C.c_void_p(), C.c_uint32()
+        self._check(self.lib.crt_light_sampling_table(self.ctx, geom.handle, lights.arg(), C.byref(ptr), C.byref(n)))
+        out = np.zeros((n.value, 16), np.float32)
+        if n.value:
+            self._check(self.lib.crt_memcpy_d2h(self.ctx, out.ctypes.data, ptr, out.nbytes))
+        return out
+
+    def lights_changed(self, geom):
+        """the host changed emission of triangles in place: rebuild the light records at their next use"""
+        self._check(self.lib.crt_lights_changed(self.ctx, geom.handle))
 
     def set_row_range(self, y_begin=0, y_end=-1):
         """multi-GPU row slabs: kernels compute rows yi in [y_begin, y_end) only; indices stay global"""

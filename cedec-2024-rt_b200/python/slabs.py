@@ -348,6 +348,9 @@ class SlabRenderer:
     def set_math_mode(self, mode):
         self.rt.set_math_mode(mode)
 
+    def set_light_sampling(self, mode, log2_slots=0):
+        self.rt.set_light_sampling(mode, log2_slots)
+
     def last_copy_events(self, slot):
         return [self._copy_events[slot]]
 
@@ -686,6 +689,10 @@ class SlabGroup:
     def set_math_mode(self, mode):
         for s in self.slabs:
             s.rt.set_math_mode(mode)
+
+    def set_light_sampling(self, mode, log2_slots=0):
+        for s in self.slabs:
+            s.rt.set_light_sampling(mode, log2_slots)
 
     def download_pixels(self):
         for s in self.slabs:

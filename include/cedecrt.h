@@ -99,6 +99,31 @@ int crt_shutdown(crt_ctx* ctx);
 const char* crt_device_name(crt_ctx* ctx);  /* oroGetDeviceProperties().name (10_restir_di.cpp:47-52) */
 const char* crt_last_error(void);
 int crt_set_math_mode(crt_ctx* ctx, int mode);
+/* Light selection (extension; the reference always selects uniformly).  Applies to every kernel that samples a light:
+ * the candidates of 10_restir_di (crt_generate_candidate, the fused frame), the NEE sample of crt_path_trace_08 and the
+ * candidates of crt_path_trace_09.
+ *   CRT_LIGHTS_UNIFORM  one emissive triangle in n, pdf 1/n * 1/area: the reference's behaviour.  Default.
+ *   CRT_LIGHTS_POWER    in proportion to emitted power P_i = max(0, luminance(Le_i)) * area_i, with every light keeping a
+ *                       nonzero probability (so RIS stays unbiased against the reference's target function): light i owns
+ *                       c_i >= 1 of K = 2^log2_slots slots, K >= n, and is selected with probability c_i / K.  The K - n
+ *                       slots beyond one per light go by power, so the mix is about (n / K) uniform.  log2_slots = 0
+ *                       picks min(23, ceil(log2 n) + 2) (about 1/4 uniform, 3/4 by power).  The table holds one
+ *                       64-byte record per slot (K * 64 bytes per geometry).  A log2_slots with 2^k < n or k > 23, or
+ *                       more than 2^23 lights, makes the first call that samples lights return CRT_EINVAL.
+ * Temporal and spatial resampling, resolve and the shadow rays do not read the source pdf and are unchanged.  The table
+ * is a pure function of the triangles and the light list (built in integers from quantised powers), so every row slab
+ * and every GPU builds the same one.  It is cached per (geometry, light list pointer, count, mode, K) and rebuilt after
+ * crt_refit_geometry; a host that changes emission in place calls crt_lights_changed (power mode reads Ke for its slot
+ * counts, and the records of both modes hold a copy of Ke). */
+enum { CRT_LIGHTS_UNIFORM = 0, CRT_LIGHTS_POWER = 1 };
+int crt_set_light_sampling(crt_ctx* ctx, int mode, int log2_slots);
+/* the light records the context's kernels would read for this light list (built now if needed), for inspection: K
+ * LightRec records of 16 floats {v0.xyz, pdf, v1.xyz, n.x, v2.xyz, n.y, Le.xyz, n.z} with pdf = sel * 1 / area
+ * (sel = c_i / K in power mode, 1 / n in uniform mode, where *n_slots = n); device memory owned by the geometry,
+ * valid until the next rebuild */
+int crt_light_sampling_table(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, const void** d_records, uint32_t* n_slots);
+/* the host has changed emission (Ke) of triangles in place: the light records are rebuilt at their next use */
+int crt_lights_changed(crt_ctx* ctx, crt_geometry geom);
 /* Multi-GPU row slabs: the kernels of this context compute only image rows yi in [y_begin, y_end) (y_end < 0:
  * to the image height).  Pixel coordinates, RNG keys and buffer indices stay global, so N slabs give exactly
  * the single-GPU frame; buffers are full-size and the host exchanges the halo rows the spatial pass reads. */
