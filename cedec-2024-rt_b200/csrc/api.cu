@@ -117,6 +117,16 @@ extern "C" int crt_set_light_sampling(crt_ctx* ctx, int mode, int log2_slots)
     return CRT_OK;
 }
 
+extern "C" int crt_set_reuse_weights(crt_ctx* ctx, int mode)
+{
+    CRT_REQUIRE(ctx, "null context");
+    CRT_REQUIRE(mode == CRT_REUSE_REFERENCE || mode == CRT_REUSE_UNBIASED, "unknown reuse weight mode");
+    // the combinations CRT_REUSE_UNBIASED does not cover (a previous camera, the fused frame on a row range) are refused by
+    // the calls that would run them
+    ctx->reuse_mode = mode;
+    return CRT_OK;
+}
+
 extern "C" int crt_set_row_range(crt_ctx* ctx, int y_begin, int y_end)
 {
     CRT_REQUIRE(ctx, "null context");

@@ -53,6 +53,7 @@ struct crt_ctx
     int light_table = 1;  // 0: sample lights through lights[] -> triangles[] like the reference (CRT_LIGHT_TABLE=0; uniform mode only)
     int light_mode = CRT_LIGHTS_UNIFORM;  // crt_set_light_sampling
     int light_log2 = 0;                   // requested log2 of the slot count of CRT_LIGHTS_POWER; 0: the default
+    int reuse_mode = CRT_REUSE_REFERENCE;  // crt_set_reuse_weights
     // fused frame (kernels_fast.cu): G-buffer + pixel-class plane, 25 bytes per pixel, grown on demand
     void* gbuf = nullptr;
     size_t gbuf_pixels = 0;

@@ -47,15 +47,16 @@ __global__ void __launch_bounds__(256)
     if (t.in) d = px_generate_candidate(t.px, frame, bvh, tris60, vis, eye, lights, kernel_opt<SH>(options), AosStore{out}, WF);
     if (WF) queue_push(q, d.want, to_shadow_ray(d, t.px.idx), d.decided);
 }
-template <int MODE, bool SH>
+// RW: the reuse weights (crt_set_reuse_weights), CRT_REUSE_REFERENCE or CRT_REUSE_UNBIASED
+template <int MODE, bool SH, int RW>
 __global__ void __launch_bounds__(256)
     k_temporal(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
                crt_options options, const crt_reservoir* prev, crt_reservoir* cur)
 {
     const TilePix t = this_pixel(W, H, rows);
     if (t.in)
-        px_temporal<Math<MODE>>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
-                                AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur});
+        px_temporal<Math<MODE>, RW>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
+                                    AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur});
 }
 // the same with reprojection into the previous frame's camera (extension; reads `prev` anywhere in the image)
 template <int MODE, bool SH>
@@ -75,15 +76,15 @@ __global__ void __launch_bounds__(256) k_save_temporal(size_t n_words, const uin
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_words; i += (size_t)gridDim.x * blockDim.x)
         dst[i] = src[i];
 }
-template <int MODE, bool SH>
+template <int MODE, bool SH, int RW>
 __global__ void __launch_bounds__(256)
     k_spatial(int W, int H, Rows rows, int frame, int pass, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
               crt_options options, const crt_reservoir* in, crt_reservoir* out)
 {
     const TilePix t = this_pixel(W, H, rows);
     if (t.in)
-        px_spatial<Math<MODE>>(t.px, W, H, frame, pass, bvh, tris60, vis, eye, kernel_opt<SH>(options),
-                               AosStore{const_cast<crt_reservoir*>(in)}, AosStore{out});
+        px_spatial<Math<MODE>, RW>(t.px, W, H, frame, pass, bvh, tris60, vis, eye, kernel_opt<SH>(options),
+                                   AosStore{const_cast<crt_reservoir*>(in)}, AosStore{out});
 }
 template <bool WF>
 __global__ void __launch_bounds__(256)
@@ -405,7 +406,11 @@ extern "C" int crt_temporal_resampling(crt_ctx* ctx, int W, int H, int frame, cr
     CRT_CHECK_BUF(reservoirs, (size_t)W * H, "reservoir");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
     const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_temporal<1, true> : k_temporal<1, false>) : (sh ? k_temporal<0, true> : k_temporal<0, false>);
+    auto k = ex ? (sh ? k_temporal<1, true, CRT_REUSE_REFERENCE> : k_temporal<1, false, CRT_REUSE_REFERENCE>)
+                : (sh ? k_temporal<0, true, CRT_REUSE_REFERENCE> : k_temporal<0, false, CRT_REUSE_REFERENCE>);
+    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
+        k = ex ? (sh ? k_temporal<1, true, CRT_REUSE_UNBIASED> : k_temporal<1, false, CRT_REUSE_UNBIASED>)
+               : (sh ? k_temporal<0, true, CRT_REUSE_UNBIASED> : k_temporal<0, false, CRT_REUSE_UNBIASED>);
     k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
                                                (const crt_visibility*)visibility_buffer.data, to_f3(eye), options,
                                                (const crt_reservoir*)previous_reservoirs.data,
@@ -425,6 +430,8 @@ extern "C" int crt_temporal_resampling_reprojected(crt_ctx* ctx, int W, int H, i
     CRT_CHECK_BUF(reservoirs, (size_t)W * H, "reservoir");
     CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "reprojection reads other pixels of the previous buffer: it cannot run in place");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
+    CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED, "unbiased reuse weights do not take a previous camera: the history "
+                                                       "pixel's surface in the previous frame is not kept");
     const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
     auto k = ex ? (sh ? k_temporal_reprojected<1, true> : k_temporal_reprojected<1, false>)
                 : (sh ? k_temporal_reprojected<0, true> : k_temporal_reprojected<0, false>);
@@ -462,7 +469,11 @@ extern "C" int crt_spatial_resampling(crt_ctx* ctx, int W, int H, int frame, int
     CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "spatial_resampling cannot run in place");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
     const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_spatial<1, true> : k_spatial<1, false>) : (sh ? k_spatial<0, true> : k_spatial<0, false>);
+    auto k = ex ? (sh ? k_spatial<1, true, CRT_REUSE_REFERENCE> : k_spatial<1, false, CRT_REUSE_REFERENCE>)
+                : (sh ? k_spatial<0, true, CRT_REUSE_REFERENCE> : k_spatial<0, false, CRT_REUSE_REFERENCE>);
+    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
+        k = ex ? (sh ? k_spatial<1, true, CRT_REUSE_UNBIASED> : k_spatial<1, false, CRT_REUSE_UNBIASED>)
+               : (sh ? k_spatial<0, true, CRT_REUSE_UNBIASED> : k_spatial<0, false, CRT_REUSE_UNBIASED>);
     k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, pass, geom->view(), (const float*)triangles.data,
                                                (const crt_visibility*)visibility_buffer.data, to_f3(eye), options,
                                                (const crt_reservoir*)previous_reservoirs.data,

@@ -47,7 +47,8 @@ namespace CRT_KNS
 #ifndef CRT_CT_MINBLOCKS
 #define CRT_CT_MINBLOCKS 3  // 80 registers; measured best with kRisBatch = 2 (profiles/r1/tuning_j.txt)
 #endif
-template <class L, int MODE>
+// RW: the reuse weights of the temporal merge (crt_set_reuse_weights), CRT_REUSE_REFERENCE or CRT_REUSE_UNBIASED
+template <class L, int MODE, int RW>
 __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
     k_candidate_temporal(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
                          L lights, crt_options options, SoaStore temporal, GBuf g, ShadowQueue q, HaloPeers peers)
@@ -58,7 +59,7 @@ __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
     if (t.in) cp = classify_pixel(t.px, tris60, vis);
     // lanes 2k, 2k+1 are horizontal neighbours of the warp's 8x4 tile: they share their light-record gathers
     const unsigned pairs = complete_pairs(__ballot_sync(0xffffffffu, t.in && !cp.skip));
-    if (t.in) d = px_candidate_temporal<Math<MODE>>(t.px, cp, frame, bvh, tris60, eye, lights, make_opt(options), temporal, g, peers, pairs);
+    if (t.in) d = px_candidate_temporal<Math<MODE>, L, false, RW>(t.px, cp, frame, bvh, tris60, eye, lights, make_opt(options), temporal, g, peers, pairs);
     queue_push(q, d.want, to_shadow_ray(d, t.px.idx), d.decided);
 }
 // the same with temporal reprojection (px_candidate_temporal<..., REPROJ = true>); a kernel of its own so that the
@@ -78,13 +79,13 @@ __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
 #ifndef CRT_SP_MINBLOCKS
 #define CRT_SP_MINBLOCKS 4  // 64 registers: 0.83 -> 0.75 ms per pass against 3 (profiles/r1/tuning_q.txt)
 #endif
-template <int MODE>
+template <int MODE, int RW>
 __global__ void __launch_bounds__(256, CRT_SP_MINBLOCKS)
     k_spatial_fast(int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye, crt_options options, SoaStore in,
                    SoaStore out, GBuf g, HaloPeers peers)
 {
     const TilePix t = this_pixel(W, H, rows);
-    if (t.in) px_spatial_fast<Math<MODE>>(t.px, W, H, frame, pass, bvh, eye, make_opt(options), in, out, g, peers);
+    if (t.in) px_spatial_fast<Math<MODE>, RW>(t.px, W, H, frame, pass, bvh, eye, make_opt(options), in, out, g, peers);
 }
 __global__ void __launch_bounds__(256)
     k_resolve_fast(crt_float4* accum, int W, int H, Rows rows, const float* tris60,
@@ -107,7 +108,7 @@ __global__ void __launch_bounds__(256)
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp)
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse)
 {
     if (rp)
     {
@@ -125,23 +126,27 @@ void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, in
         }
         return;
     }
+    const bool unb = reuse == CRT_REUSE_UNBIASED;
     if (table)
     {
         const LightsTable L{table, n_lights};
-        auto k = exact ? k_candidate_temporal<LightsTable, 1> : k_candidate_temporal<LightsTable, 0>;
+        auto k = exact ? k_candidate_temporal<LightsTable, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal<LightsTable, 0, CRT_REUSE_REFERENCE>;
+        if (unb) k = exact ? k_candidate_temporal<LightsTable, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal<LightsTable, 0, CRT_REUSE_UNBIASED>;
         k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
     }
     else
     {
         const LightsIndexed L{tris60, light_ids, n_lights};
-        auto k = exact ? k_candidate_temporal<LightsIndexed, 1> : k_candidate_temporal<LightsIndexed, 0>;
+        auto k = exact ? k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_REFERENCE>;
+        if (unb) k = exact ? k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_UNBIASED>;
         k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
     }
 }
 void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
-                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers)
+                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse)
 {
-    auto k = exact ? k_spatial_fast<1> : k_spatial_fast<0>;
+    auto k = exact ? k_spatial_fast<1, CRT_REUSE_REFERENCE> : k_spatial_fast<0, CRT_REUSE_REFERENCE>;
+    if (reuse == CRT_REUSE_UNBIASED) k = exact ? k_spatial_fast<1, CRT_REUSE_UNBIASED> : k_spatial_fast<0, CRT_REUSE_UNBIASED>;
     k<<<grid, 256, 0, st>>>(W, H, rows, frame, pass, bvh, eye, options, in, out, g, peers);
 }
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
@@ -152,12 +157,12 @@ void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H,
 int preload()
 {
     cudaFuncAttributes a;
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 0>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 1>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 0>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 0, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 1, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1, CRT_REUSE_REFERENCE>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_resolve_fast));
     return CRT_OK;
 }
@@ -170,9 +175,9 @@ int preload();
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp);
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse);
 void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
-                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers);
+                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
                     const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
 }  // namespace fm
@@ -182,9 +187,9 @@ int preload();
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp);
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse);
 void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
-                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers);
+                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
                     const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
 }  // namespace rf
@@ -295,6 +300,15 @@ HaloPeers halo_peers(const crt_ctx* ctx, int which, Rows rows, bool with_class, 
     (void)n;
     return p;
 }
+// the fused spatial pass of CRT_REUSE_UNBIASED reads its neighbours' G-buffer records, which exist for this context's own
+// rows only (halo rows are neither computed nor mirrored): it runs on the whole image and without slab links
+bool unbiased_rows_ok(const crt_ctx* ctx, int H, const crt_options& o)
+{
+    const Rows rows = rows_of(ctx, H);
+    return !fused(o) || (rows.y0 == 0 && rows.y1 == H && !ctx->links_set);
+}
+const char* const kUnbiasedRowsMsg = "unbiased reuse weights in the fused frame need the whole image on one context (no row "
+                                     "range, no slab links): the G-buffer of halo rows is not kept; the per-kernel path takes row ranges";
 int which_of(const crt_restir_buffers* b, const crt_buffer& x) { return x.data == b->temporal.data ? 0 : x.data == b->reservoir0.data ? 1 : 2; }
 // input and output of spatial pass k in fused mode
 void pass_buffers(const crt_restir_buffers* b, int pass, crt_buffer* in, crt_buffer* out)
@@ -319,6 +333,8 @@ extern "C" int crt_restir_is_fused(crt_options options) { return fused(options) 
 extern "C" int crt_restir_set_previous_camera(crt_ctx* ctx, const crt_raygen* previous_raygen)
 {
     CRT_REQUIRE(ctx, "null context");
+    CRT_REQUIRE(!previous_raygen || ctx->reuse_mode != CRT_REUSE_UNBIASED,
+                "unbiased reuse weights do not take a previous camera: the history pixel's surface in the previous frame is not kept");
     ctx->prev_cam_set = previous_raygen != nullptr;
     if (previous_raygen) ctx->prev_cam = *previous_raygen;
     return CRT_OK;
@@ -342,6 +358,12 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     rc = raycast_or_prefetched(ctx, W, H, geom, triangles, raygen, b->visibility);
     if (rc != CRT_OK) return rc;
     ctx->frame_fused = fused(options);
+    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
+    {
+        CRT_REQUIRE(!ctx->prev_cam_set, "unbiased reuse weights do not take a previous camera: the history pixel's surface in "
+                                        "the previous frame is not kept");
+        CRT_REQUIRE(unbiased_rows_ok(ctx, H, options), kUnbiasedRowsMsg);
+    }
     if (ctx->links_set)
     {
         // what the direct-store halo protocol (slab_p2p.cu) covers; anything else must use a host-side exchange
@@ -427,7 +449,7 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     }
     CRT_MODE_NS(ctx, launch_candidate_temporal)(
         ctx->stream, exact, grid, W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), table,
-        (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr);
+        (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr, ctx->reuse_mode);
     rc = check_launch(ctx, "candidate_temporal");
     if (rc != CRT_OK || !options.use_visibility_reuse) return rc;
     ShadowSink sink{nullptr, nullptr, 0, (uint32_t*)T.plane(0, 0)};
@@ -453,6 +475,7 @@ extern "C" int crt_restir_spatial_pass(crt_ctx* ctx, int W, int H, int frame, in
                                       odd ? b->reservoir1 : b->reservoir0, odd ? b->reservoir0 : b->reservoir1);
     }
     if (!options.use_spatial_resampling) return CRT_OK;  // the reference's disabled pass is a copy
+    CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED || unbiased_rows_ok(ctx, H, options), kUnbiasedRowsMsg);
     CRT_REQUIRE(ctx->gbuf && ctx->gbuf_pixels >= (size_t)W * H, "crt_restir_frame_begin has not run for this image size");
     const size_t n = (size_t)W * H;
     const Rows rows = rows_of(ctx, H);
@@ -465,7 +488,7 @@ extern "C" int crt_restir_spatial_pass(crt_ctx* ctx, int W, int H, int frame, in
     const HaloPeers peers = pass + 1 < options.spatial_resampling_passes ? halo_peers(ctx, which_of(b, out), rows, false, n) : HaloPeers();
     CRT_MODE_NS(ctx, launch_spatial)(
         ctx->stream, ctx->math_mode == CRT_MATH_EXACT, tile_grid(W, rows), W, H, rows, frame, pass, geom->view(), to_f3(eye),
-        options, soa(in, n), soa(out, n), g, peers);
+        options, soa(in, n), soa(out, n), g, peers, ctx->reuse_mode);
     return check_launch(ctx, "spatial_fast");
 }
 

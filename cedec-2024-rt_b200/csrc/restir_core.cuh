@@ -642,6 +642,80 @@ CRT_HD void spatial_merge(const Bvh& bvh, const Surf& surf, f3 eye, const Opt& o
     if (u < weight / r.w_sum) r.s = nb.s;
 }
 
+// ---- unbiased reuse weights (extension: crt_set_reuse_weights, CRT_REUSE_UNBIASED; DESIGN.md section 15).  A merge
+// combines domains: the pixel's own reservoir and each accepted neighbour (spatial), or the current reservoir and the
+// history (temporal).  A domain's surface is its *pixel's* primary-hit surface, never the sample's stored origin, so its
+// confidence c_j = trunc(M_j * heuristics(S_q, S_j)) depends on the neighbour draws and skips alone.  The merge weight
+// is p_hat_q(y_j) * ucw_j * c_j (the stored visibility bit multiplies nothing), r.M accumulates sum c_j as before, and
+// after the last domain, with y the selected sample,
+//   Z = sum_j c_j [p_hat_j(y) > 0],   ucw = p_hat_q(y) > 0 && Z > 0 ? w_sum / (Z p_hat_q(y)) : 0.
+// The rejection heuristics of reservoir.hpp:61-87 (rejection_heuristics above), on two pixel surfaces
+template <class M>
+CRT_HD float surface_heuristics(const Surf& s0, const Surf& s1, f3 eye)
+{
+    const float d0 = length(s0.p - eye);
+    const float d1 = length(s1.p - eye);
+    const float diff = (d1 - d0) * (d1 - d0) / d0;
+    float w = 1.0f;
+    w *= M::exp(-32.0f * diff);
+    const float c = dot(s0.n, s1.n);
+    w *= M::pow(c > 0.0f ? c : 0.0f, 8.0f);
+    return w;
+}
+// c_j of a domain with M = m whose pixel surface is `theirs` (int *= float, 10_restir_di.cu:211-212)
+template <class M>
+CRT_HD int confidence(int m, const Surf& mine, const Surf& theirs, f3 eye)
+{
+    return f2i_trunc((float)m * surface_heuristics<M>(mine, theirs, eye));
+}
+// [p_hat_j(y) > 0] at surface s; with the shadowed target function its ray is traced only when the unshadowed value is
+// positive (((1/pi G) V) lum > 0 exactly when (1/pi G) lum > 0 and V = 1)
+CRT_HD bool target_positive(const Bvh& bvh, const Surf& s, const Sample& y, bool shadowed)
+{
+    if (!(target_function(bvh, s.p, s.n, y.hp, y.hn, y.rad, false) > 0.0f)) return false;
+    return !shadowed || check_visibility(bvh, s.p, s.n, y.hp) != 0.0f;
+}
+// Z after one more domain of confidence c and surface s
+CRT_HD int z_of(int z, int c, const Bvh& bvh, const Surf& s, const Sample& y, bool shadowed)
+{
+    return target_positive(bvh, s, y, shadowed) ? z + c : z;
+}
+CRT_HD float ucw_unbiased(float w_sum, int z, float p_hat) { return p_hat > 0.0f && z > 0 ? w_sum / ((float)z * p_hat) : 0.0f; }
+
+// temporal_merge with unbiased weights.  Without reprojection the history's pixel is this pixel and its primary-hit
+// surface this frame's (deterministic primary rays, static geometry): c_h = trunc(M_h * heuristics(S_q, S_q)), and
+// p_hat_h(y) = p_hat_q(y), so Z = c_own + c_h whenever p_hat_q(y) > 0.
+template <class M>
+CRT_HD bool temporal_merge_unbiased(const Bvh& bvh, const Surf& surf, f3 eye, const Opt& opt, Res prev, Res& r, Pcg& rng)
+{
+    const int cap = 20 * opt.ris_count;  // M-cap, :186-188
+    prev.M = prev.M < cap ? prev.M : cap;
+    const float p_hat_y = target_function(bvh, surf.p, surf.n, prev.s.hp, prev.s.hn, prev.s.rad, opt.shadowed);
+    const int c_own = r.M;
+    prev.M = confidence<M>(prev.M, surf, surf, eye);
+    const float weight = p_hat_y * prev.ucw * (float)prev.M;
+    const float u = rng.next_f();
+    r.w_sum += weight;
+    r.M += prev.M;
+    const bool accepted = u < weight / r.w_sum;
+    if (accepted) r.s = prev.s;
+    r.ucw = ucw_unbiased(r.w_sum, c_own + prev.M, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, opt.shadowed));
+    return accepted;
+}
+// spatial_merge with unbiased weights: `nsurf` is the neighbour pixel's surface, `nb` its input reservoir
+template <class M>
+CRT_HD void spatial_merge_unbiased(const Bvh& bvh, const Surf& surf, const Surf& nsurf, f3 eye, const Opt& opt, const Res& nb,
+                                   Res& r, Pcg& rng)
+{
+    const float p_hat_y = target_function(bvh, surf.p, surf.n, nb.s.hp, nb.s.hn, nb.s.rad, opt.shadowed);
+    const int c = confidence<M>(nb.M, surf, nsurf, eye);
+    const float weight = p_hat_y * nb.ucw * (float)c;
+    const float u = rng.next_f();
+    r.w_sum += weight;
+    r.M += c;
+    if (u < weight / r.w_sum) r.s = nb.s;
+}
+
 // neighbour pixel of spatial_resampling (10_restir_di.cu:309-313): two randoms, Box-Muller, truncation
 template <class M>
 CRT_HD void spatial_neighbour(int xi, int yi, float radius, Pcg& rng, int& x, int& y)

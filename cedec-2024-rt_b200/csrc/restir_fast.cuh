@@ -237,7 +237,8 @@ struct Reprojection
     crt_raygen prev_cam{};
     int W = 0, H = 0;
 };
-template <class M, class L, bool REPROJ = false>
+// RW: CRT_REUSE_REFERENCE, or CRT_REUSE_UNBIASED (temporal_merge_unbiased; not combined with REPROJ)
+template <class M, class L, bool REPROJ = false, int RW = CRT_REUSE_REFERENCE>
 CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int frame, const Bvh& bvh, const float* tris60,
                                          f3 eye, const L& lights, const Opt& opt_in, const SoaStore& temporal,
                                          const GBuf& g, const HaloPeers& peers = HaloPeers(), unsigned pair_mask = 0u,
@@ -275,7 +276,8 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
                                                                                           : empty_res();
         }
         else history = temporal.load(px.idx);
-        candidate_survives = !temporal_merge<M>(bvh, surf, eye, opt, history, r, rng_t);
+        if (RW == CRT_REUSE_UNBIASED) candidate_survives = !temporal_merge_unbiased<M>(bvh, surf, eye, opt, history, r, rng_t);
+        else candidate_survives = !temporal_merge<M>(bvh, surf, eye, opt, history, r, rng_t);
     }
     if (opt.reuse && candidate_survives)
     {
@@ -288,6 +290,55 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
     return ray;
 }
 
+// px_spatial's unbiased form (CRT_REUSE_UNBIASED) on this data flow, from the pixel's input reservoir `r` and its random
+// stream: a neighbour's surface is its G-buffer record (24 bytes) instead of plane 0's sample origin, planes 1-2 are read
+// for every visited neighbour (the visibility bit weighs nothing, so there is no weightless shortcut), and the replayed
+// second pass sums Z.  The G-buffer must hold every neighbour's row: the whole image on one context.
+template <class M>
+CRT_HD void spatial_fast_unbiased(const Pix& px, int W, int H, const Bvh& bvh, f3 eye, const Opt& opt, const SoaStore& in,
+                                  const GBuf& g, const Surf& surf, Pcg rng, Res& r)
+{
+    const Pcg rng_z = rng;
+    const int c_own = r.M;
+    for (int k = 0; k < opt.spatial_count; ++k)
+    {
+        int x, y;
+        spatial_neighbour<M>(px.xi, px.yi, opt.radius, rng, x, y);
+        if (x < 0 || x >= W || y < 0 || y >= H) continue;
+        if (x == px.xi && y == px.yi) continue;
+        const int pid = x + (H - y - 1) * W;
+        const ResHead nh = in.load_head(pid);
+        if (nh.skip()) continue;
+        const int c = confidence<M>(nh.M(), surf, g.load(pid), eye);
+        const float u = rng.next_f();
+        const Res nb = in.finish_load(pid, nh);
+        const float weight = target_function(bvh, surf.p, surf.n, nb.s.hp, nb.s.hn, nb.s.rad, false) * nb.ucw * (float)c;
+        r.w_sum += weight;  // spatial_merge_unbiased
+        r.M += c;
+        if (u < weight / r.w_sum) r.s = nb.s;
+    }
+    const float p_hat = target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, false);
+    int z = c_own;
+    if (p_hat > 0.0f)
+    {
+        Pcg rz = rng_z;
+        for (int k = 0; k < opt.spatial_count; ++k)
+        {
+            int x, y;
+            spatial_neighbour<M>(px.xi, px.yi, opt.radius, rz, x, y);
+            if (x < 0 || x >= W || y < 0 || y >= H) continue;
+            if (x == px.xi && y == px.yi) continue;
+            const int pid = x + (H - y - 1) * W;
+            const ResHead nh = in.load_head(pid);
+            if (nh.skip()) continue;
+            const Surf ns = g.load(pid);
+            (void)rz.next_f();  // the merge's random number
+            z = z_of(z, confidence<M>(nh.M(), surf, ns, eye), bvh, ns, r.s, false);
+        }
+    }
+    r.ucw = ucw_unbiased(r.w_sum, z, p_hat);
+}
+
 // ---- spatial_resampling (10_restir_di.cu:256-388) with opt.spatial == true (the disabled form is a copy the
 // fused frame skips).
 // A neighbour whose sample is occluded (visibility reuse, :352-355: p_hat_y *= visibility) merges with weight
@@ -295,7 +346,8 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
 // rejection heuristics and one random number is drawn.  That needs plane 0 of the neighbour only.  (Precondition,
 // true for every finite scene: the target function of the neighbour's sample is finite — it is not only if the
 // light sample coincides bit for bit with this pixel's surface point — and ucw is finite, which is checked.)
-template <class M>
+// RW = CRT_REUSE_UNBIASED: spatial_fast_unbiased above
+template <class M, int RW = CRT_REUSE_REFERENCE>
 CRT_HD void px_spatial_fast(const Pix& px, int W, int H, int frame, int pass, const Bvh& bvh, f3 eye, const Opt& opt_in,
                             const SoaStore& in, const SoaStore& out, const GBuf& g, const HaloPeers& peers = HaloPeers())
 {
@@ -312,37 +364,41 @@ CRT_HD void px_spatial_fast(const Pix& px, int W, int H, int frame, int pass, co
     Pcg rng(hash_pcg4(px.xi, px.yi, frame, 2 + pass), 0);
     const Surf surf = g.load(px.idx);
     Res r = in.load(px.idx);
-    for (int k = 0; k < opt.spatial_count; ++k)
+    if (RW == CRT_REUSE_UNBIASED) spatial_fast_unbiased<M>(px, W, H, bvh, eye, opt, in, g, surf, rng, r);
+    else
     {
-        int x, y;
-        spatial_neighbour<M>(px.xi, px.yi, opt.radius, rng, x, y);
-        if (x < 0 || x >= W || y < 0 || y >= H) continue;
-        if (x == px.xi && y == px.yi) continue;
-        const int pid = x + (H - y - 1) * W;
-        const ResHead nh = in.load_head(pid);
-        if (nh.skip()) continue;
-        // common to every neighbour (the warp stays converged here): M after the rejection heuristics, one random
-        Sample ns;
-        ns.op = nh.op;
-        ns.on = nh.on;
-        const int nM = rejected_m<M>(r.s, ns, nh.M(), eye);
-        const float u = rng.next_f();
-        // only a neighbour that can be selected needs its sample: planes 1-2 and the target function
-        float weight = 0.0f;
-        Res nb;
-        const bool weightless = opt.reuse && !nh.visible() && (f2u(nh.ucw) & 0x7f800000u) != 0x7f800000u;
-        if (!weightless)
+        for (int k = 0; k < opt.spatial_count; ++k)
         {
-            nb = in.finish_load(pid, nh);
-            float p_hat_y = target_function(bvh, surf.p, surf.n, nb.s.hp, nb.s.hn, nb.s.rad, false);
-            if (opt.reuse) p_hat_y *= (nb.s.vis & 1u) ? 1.0f : 0.0f;
-            weight = p_hat_y * nb.ucw * (float)nM;
+            int x, y;
+            spatial_neighbour<M>(px.xi, px.yi, opt.radius, rng, x, y);
+            if (x < 0 || x >= W || y < 0 || y >= H) continue;
+            if (x == px.xi && y == px.yi) continue;
+            const int pid = x + (H - y - 1) * W;
+            const ResHead nh = in.load_head(pid);
+            if (nh.skip()) continue;
+            // common to every neighbour (the warp stays converged here): M after the rejection heuristics, one random
+            Sample ns;
+            ns.op = nh.op;
+            ns.on = nh.on;
+            const int nM = rejected_m<M>(r.s, ns, nh.M(), eye);
+            const float u = rng.next_f();
+            // only a neighbour that can be selected needs its sample: planes 1-2 and the target function
+            float weight = 0.0f;
+            Res nb;
+            const bool weightless = opt.reuse && !nh.visible() && (f2u(nh.ucw) & 0x7f800000u) != 0x7f800000u;
+            if (!weightless)
+            {
+                nb = in.finish_load(pid, nh);
+                float p_hat_y = target_function(bvh, surf.p, surf.n, nb.s.hp, nb.s.hn, nb.s.rad, false);
+                if (opt.reuse) p_hat_y *= (nb.s.vis & 1u) ? 1.0f : 0.0f;
+                weight = p_hat_y * nb.ucw * (float)nM;
+            }
+            r.w_sum += weight;  // Reservoir::merge (reservoir.hpp:31-37)
+            r.M += nM;
+            if (!weightless && u < weight / r.w_sum) r.s = nb.s;
         }
-        r.w_sum += weight;  // Reservoir::merge (reservoir.hpp:31-37)
-        r.M += nM;
-        if (!weightless && u < weight / r.w_sum) r.s = nb.s;
+        r.ucw = ucw_of(r, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, false));
     }
-    r.ucw = ucw_of(r, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, false));
     out.store(px.idx, r);
     peers.mirror(px, out.n, r);
 }

@@ -185,7 +185,8 @@ CRT_HD DeferredRay px_generate_candidate(const Pix& px, int frame, const Bvh& bv
 // ---- 10_restir_di.cu:137-237
 // prev_cam != nullptr (extension: crt_temporal_resampling_reprojected): the previous reservoir is read at the pixel this
 // surface point had in the previous frame's camera; no history there = Reservoir{} (restir_core.cuh: reproject_pixel)
-template <class M, class RSP, class RS>
+// RW: CRT_REUSE_REFERENCE (the reference's merge) or CRT_REUSE_UNBIASED (temporal_merge_unbiased; no reprojection)
+template <class M, int RW = CRT_REUSE_REFERENCE, class RSP, class RS>
 CRT_HD void px_temporal(const Pix& px, int frame, const Bvh& bvh, const float* tris60, const crt_visibility* vis,
                         f3 eye, const Opt& opt, const RSP& prev, const RS& cur, const crt_raygen* prev_cam = nullptr,
                         int W = 0, int H = 0)
@@ -205,12 +206,16 @@ CRT_HD void px_temporal(const Pix& px, int frame, const Bvh& bvh, const float* t
         history = reproject_pixel(to_raygen(*prev_cam), W, H, surf.p, xp, yp) ? prev.load(xp + (H - yp - 1) * W) : empty_res();
     }
     else history = prev.load(px.idx);
-    temporal_merge<M>(bvh, surf, eye, opt, history, r, rng);
+    if (RW == CRT_REUSE_UNBIASED) temporal_merge_unbiased<M>(bvh, surf, eye, opt, history, r, rng);
+    else temporal_merge<M>(bvh, surf, eye, opt, history, r, rng);
     cur.store(px.idx, r);
 }
 
 // ---- 10_restir_di.cu:256-388
-template <class M, class RSI, class RSO>
+// RW = CRT_REUSE_UNBIASED: spatial_merge_unbiased with each accepted neighbour's surface (from its Visibility record),
+// then a second pass over the same neighbours — the pixel's random stream replayed from before the loop: the same
+// offsets, skips and one random number per visited neighbour — sums Z for the selected sample
+template <class M, int RW = CRT_REUSE_REFERENCE, class RSI, class RSO>
 CRT_HD void px_spatial(const Pix& px, int W, int H, int frame, int pass, const Bvh& bvh, const float* tris60,
                        const crt_visibility* vis, f3 eye, const Opt& opt, const RSI& in, const RSO& out)
 {
@@ -226,6 +231,8 @@ CRT_HD void px_spatial(const Pix& px, int W, int H, int frame, int pass, const B
         out.store(px.idx, r);
         return;
     }
+    const Pcg rng_z = rng;
+    const int c_own = r.M;
     for (int k = 0; k < opt.spatial_count; ++k)
     {
         int x, y;
@@ -235,10 +242,38 @@ CRT_HD void px_spatial(const Pix& px, int W, int H, int frame, int pass, const B
         const int pid = x + (H - y - 1) * W;
         const Vis nv = load_vis(vis, pid);
         if (nv.index == -1) continue;
-        if (has_emission(tri_at(tris60, nv.index).emissive())) continue;
-        spatial_merge<M>(bvh, surf, eye, opt, in.load(pid), r, rng);
+        const TriRef ntri = tri_at(tris60, nv.index);
+        if (has_emission(ntri.emissive())) continue;
+        if (RW == CRT_REUSE_UNBIASED)
+            spatial_merge_unbiased<M>(bvh, surf, surface_from_visibility(ntri, nv.u, nv.v, eye), eye, opt, in.load(pid), r, rng);
+        else spatial_merge<M>(bvh, surf, eye, opt, in.load(pid), r, rng);
     }
-    r.ucw = ucw_of(r, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, opt.shadowed));
+    const float p_hat = target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, opt.shadowed);
+    if (RW != CRT_REUSE_UNBIASED) r.ucw = ucw_of(r, p_hat);
+    else
+    {
+        int z = c_own;  // the pixel's own domain: ucw_unbiased reads p_hat_q(y) > 0 itself
+        if (p_hat > 0.0f)
+        {
+            Pcg rz = rng_z;
+            for (int k = 0; k < opt.spatial_count; ++k)
+            {
+                int x, y;
+                spatial_neighbour<M>(px.xi, px.yi, opt.radius, rz, x, y);
+                if (x < 0 || x >= W || y < 0 || y >= H) continue;
+                if (x == px.xi && y == px.yi) continue;
+                const int pid = x + (H - y - 1) * W;
+                const Vis nv = load_vis(vis, pid);
+                if (nv.index == -1) continue;
+                const TriRef ntri = tri_at(tris60, nv.index);
+                if (has_emission(ntri.emissive())) continue;
+                const Surf ns = surface_from_visibility(ntri, nv.u, nv.v, eye);
+                (void)rz.next_f();  // the merge's random number
+                z = z_of(z, confidence<M>(in.load(pid).M, surf, ns, eye), bvh, ns, r.s, opt.shadowed);
+            }
+        }
+        r.ucw = ucw_unbiased(r.w_sum, z, p_hat);
+    }
     out.store(px.idx, r);
 }
 

@@ -50,6 +50,8 @@ class Device
     void setRowRange(int y0, int y1) const { CRT_CHECKED(crt_set_row_range(m_ctx, y0, y1)); }
     // CRT_LIGHTS_UNIFORM (the reference) or CRT_LIGHTS_POWER; log2_slots = 0: the default slot count
     void setLightSampling(int mode, int log2_slots = 0) const { CRT_CHECKED(crt_set_light_sampling(m_ctx, mode, log2_slots)); }
+    // CRT_REUSE_REFERENCE (the reference) or CRT_REUSE_UNBIASED (1/Z weights in every temporal and spatial merge)
+    void setReuseWeights(int mode) const { CRT_CHECKED(crt_set_reuse_weights(m_ctx, mode)); }
 
    private:
     crt_ctx* m_ctx = nullptr;

@@ -5,6 +5,7 @@
 //   restir_di_headless --scene assets/blocks_restir.tri[.xz] [--tile NX NZ DX DZ] [--size W H] [--frames N]
 //                      [--eye x y z] [--lookat x y z] [--no-temporal] [--no-spatial] [--no-accumulate]
 //                      [--out image.ppm] [--dump-accum file.f32] [--fused] [--lights uniform|power]
+//                      [--reuse reference|unbiased]
 //
 // --fused issues one crt_restir_di_frame call per frame instead of the launch list (same image, see cedecrt.h).
 //
@@ -42,6 +43,7 @@ int main(int argc, char** argv)
     std::string scene, out_ppm, dump_accum;
     bool fused = false;
     int light_mode = CRT_LIGHTS_UNIFORM;  // --lights power: select lights in proportion to their power (cedecrt.h)
+    int reuse_mode = CRT_REUSE_REFERENCE;  // --reuse unbiased: 1/Z weights in the temporal and spatial merges (cedecrt.h)
     int width = 1920, height = 1080, frames = 4, tile_nx = 1, tile_nz = 1;
     float tile_dx = 130.0f, tile_dz = 82.0f;
     float eye[3] = {-0.579885f, 22.194597f, -6.567105f}, center[3] = {5.224952f, 20.847435f, 1.431192f};  // :188-189
@@ -88,6 +90,17 @@ int main(int argc, char** argv)
             }
             light_mode = m == "power" ? CRT_LIGHTS_POWER : CRT_LIGHTS_UNIFORM;
         }
+        else if (a == "--reuse")
+        {
+            need(1);
+            const std::string m = argv[++i];
+            if (m != "reference" && m != "unbiased")
+            {
+                fprintf(stderr, "--reuse takes reference or unbiased\n");
+                return 2;
+            }
+            reuse_mode = m == "unbiased" ? CRT_REUSE_UNBIASED : CRT_REUSE_REFERENCE;
+        }
         else if (a == "--out") { need(1); out_ppm = argv[++i]; }
         else if (a == "--dump-accum") { need(1); dump_accum = argv[++i]; }
         else
@@ -106,6 +119,7 @@ int main(int argc, char** argv)
         crt::Device device(0);
         printf("Device: %s\n", device.name());
         device.setLightSampling(light_mode);
+        device.setReuseWeights(reuse_mode);
         Shader shader(device);
 
         std::vector<crt_triangle> triangles =

@@ -30,6 +30,7 @@ assert TRIANGLE.itemsize == 60 and VISIBILITY.itemsize == 16 and RESERVOIR.items
 
 MATH_LIBDEVICE, MATH_EXACT, MATH_FAST, MATH_REFERENCE = 0, 1, 2, 3  # include/cedecrt.h: CRT_MATH_*
 LIGHTS_UNIFORM, LIGHTS_POWER = 0, 1  # include/cedecrt.h: CRT_LIGHTS_*
+REUSE_REFERENCE, REUSE_UNBIASED = 0, 1  # include/cedecrt.h: CRT_REUSE_*
 
 
 class Float3(C.Structure):
@@ -124,6 +125,7 @@ def _load():
         "crt_set_light_sampling": [P, I, I],
         "crt_light_sampling_table": [P, G, B, C.POINTER(C.c_void_p), C.POINTER(C.c_uint32)],
         "crt_lights_changed": [P, G],
+        "crt_set_reuse_weights": [P, I],
         "crt_set_stream": [P, C.c_void_p],
         "crt_set_frame_overlap": [P, I],
         "crt_frame_join": [P],
@@ -346,6 +348,12 @@ class Runtime:
     def lights_changed(self, geom):
         """the host changed emission of triangles in place: rebuild the light records at their next use"""
         self._check(self.lib.crt_lights_changed(self.ctx, geom.handle))
+
+    def set_reuse_weights(self, mode):
+        """REUSE_REFERENCE (the reference's biased merge, default) or REUSE_UNBIASED: 1/Z weights in every temporal and
+        spatial merge (include/cedecrt.h: crt_set_reuse_weights)"""
+        self._check(self.lib.crt_set_reuse_weights(self.ctx, mode))
+        self.reuse_mode = mode
 
     def set_row_range(self, y_begin=0, y_end=-1):
         """multi-GPU row slabs: kernels compute rows yi in [y_begin, y_end) only; indices stay global"""

@@ -351,6 +351,9 @@ class SlabRenderer:
     def set_light_sampling(self, mode, log2_slots=0):
         self.rt.set_light_sampling(mode, log2_slots)
 
+    def set_reuse_weights(self, mode):
+        self.rt.set_reuse_weights(mode)
+
     def last_copy_events(self, slot):
         return [self._copy_events[slot]]
 
@@ -693,6 +696,10 @@ class SlabGroup:
     def set_light_sampling(self, mode, log2_slots=0):
         for s in self.slabs:
             s.rt.set_light_sampling(mode, log2_slots)
+
+    def set_reuse_weights(self, mode):
+        for s in self.slabs:
+            s.rt.set_reuse_weights(mode)
 
     def download_pixels(self):
         for s in self.slabs:

@@ -124,6 +124,34 @@ int crt_set_light_sampling(crt_ctx* ctx, int mode, int log2_slots);
 int crt_light_sampling_table(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, const void** d_records, uint32_t* n_slots);
 /* the host has changed emission (Ke) of triangles in place: the light records are rebuilt at their next use */
 int crt_lights_changed(crt_ctx* ctx, crt_geometry geom);
+/* Reuse weights (extension; the reference's reuse is biased).  Applies to every kernel that merges reservoirs:
+ * crt_temporal_resampling and crt_spatial_resampling (directly and through crt_launch), the fused frame's candidate +
+ * temporal kernel and crt_restir_spatial_pass, and the per-kernel path crt_restir_di_frame falls back to.
+ *   CRT_REUSE_REFERENCE  the reference's merge: a neighbour's M counts whether or not it could have produced the selected
+ *                        sample, ucw = w_sum / (M p_hat), the rejection heuristics compare the running reservoir's sample
+ *                        origin, and with use_visibility_reuse the stored visibility bit zeroes a weight.  Default.
+ *   CRT_REUSE_UNBIASED   1/Z weights.  A merge combines domains: the pixel's own input reservoir and each accepted
+ *                        neighbour (spatial), or the current reservoir and the history (temporal).  A domain's surface
+ *                        is its pixel's primary-hit surface (position and shading normal), not the sample's origin.
+ *                        Which neighbours are visited is exactly the reference's (the same draws, skips and random
+ *                        stream).  Domain j has confidence c_j = trunc(M_j * rejection_heuristics(S_q, S_j)) — the
+ *                        reference's formula on the two pixel surfaces; the temporal M cap 20 * ris_sample_count applies
+ *                        first — and its sample y_j merges with weight p_hat_q(y_j) * ucw_j * c_j; the visibility bit
+ *                        weighs nothing (use_visibility_reuse still traces and stores it, and resolve still reads it to
+ *                        skip a shadow ray).  Selection is unchanged and M accumulates sum c_j.  After the last domain,
+ *                        for the selected sample y:
+ *                          Z = sum over domains j (the pixel's own, c = its input M, included) of c_j [p_hat_j(y) > 0]
+ *                          ucw = p_hat_q(y) > 0 && Z > 0 ? w_sum / (Z p_hat_q(y)) : 0
+ *                        with p_hat_j the reference's target function at domain j's surface (including a shadow ray
+ *                        under use_shadowed_target_function, traced only when the unshadowed value is positive).
+ *                        Candidate generation is a single domain and unchanged.  Without reprojection the history's
+ *                        surface is the pixel's own, so temporal Z = M whenever p_hat_q(y) > 0.  Unbiased for static
+ *                        geometry: the first merge after crt_refit_geometry is not exactly so.
+ * CRT_REUSE_UNBIASED is refused (CRT_EINVAL) with a previous camera (crt_temporal_resampling_reprojected, and a camera
+ * set with crt_restir_set_previous_camera) and in the fused frame on a row range narrower than the image or with slab
+ * links (the G-buffer of halo rows is not kept); the per-kernel path takes row ranges.  An unknown mode is CRT_EINVAL. */
+enum { CRT_REUSE_REFERENCE = 0, CRT_REUSE_UNBIASED = 1 };
+int crt_set_reuse_weights(crt_ctx* ctx, int mode);
 /* Multi-GPU row slabs: the kernels of this context compute only image rows yi in [y_begin, y_end) (y_end < 0:
  * to the image height).  Pixel coordinates, RNG keys and buffer indices stay global, so N slabs give exactly
  * the single-GPU frame; buffers are full-size and the host exchanges the halo rows the spatial pass reads. */
