@@ -332,6 +332,10 @@ extern "C" int crt_launch(crt_ctx* ctx, const char* name, void** params, unsigne
         return crt_temporal_resampling_reprojected(ctx, ARG(int, 0), ARG(int, 1), ARG(int, 2), ARG(crt_geometry, 3), ARG(B, 4),
                                                    ARG(B, 5), ARG(crt_float3, 6), ARG(crt_options, 7), ARG(crt_raygen, 8),
                                                    ARG(B, 9), ARG(B, 10));
+    if (!strcmp(name, "temporal_resampling_reprojected_surfaces"))
+        return crt_temporal_resampling_reprojected_surfaces(ctx, ARG(int, 0), ARG(int, 1), ARG(int, 2), ARG(crt_geometry, 3),
+                                                            ARG(B, 4), ARG(B, 5), ARG(crt_float3, 6), ARG(crt_options, 7),
+                                                            ARG(crt_raygen, 8), ARG(B, 9), ARG(B, 10), ARG(B, 11));
     if (!strcmp(name, "save_temporal_reservoir"))
         return crt_save_temporal_reservoir(ctx, ARG(int, 0), ARG(int, 1), ARG(B, 2), ARG(B, 3));
     if (!strcmp(name, "spatial_resampling"))

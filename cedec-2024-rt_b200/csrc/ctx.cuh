@@ -64,6 +64,9 @@ struct crt_ctx
     // of its history (the merge of the fused frame is in place, a look-up at another pixel must not see this frame's records)
     bool prev_cam_set = false;
     crt_raygen prev_cam = {};
+    // the previous frame's Visibility buffer (crt_restir_set_previous_frame; data == nullptr: not given): the history
+    // pixel's surface for CRT_REUSE_UNBIASED
+    crt_buffer prev_vis = {};
     void* history_prev = nullptr;
     size_t history_prev_pixels = 0;
     int resolve_reuse = 1;  // 0: resolve traces every shadow ray like the reference (CRT_RESOLVE_REUSE=0)

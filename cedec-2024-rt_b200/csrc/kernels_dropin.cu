@@ -58,16 +58,19 @@ __global__ void __launch_bounds__(256)
         px_temporal<Math<MODE>, RW>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
                                     AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur});
 }
-// the same with reprojection into the previous frame's camera (extension; reads `prev` anywhere in the image)
-template <int MODE, bool SH>
+// the same with reprojection into the previous frame's camera (extension; reads `prev` anywhere in the image).  RW =
+// CRT_REUSE_UNBIASED reads the previous frame's Visibility `prev_vis` at the history pixel; the reference's merge ignores it
+// (the last parameter, so that the reference instantiations keep their code)
+template <int MODE, bool SH, int RW>
 __global__ void __launch_bounds__(256)
     k_temporal_reprojected(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
-                           crt_options options, crt_raygen prev_cam, const crt_reservoir* prev, crt_reservoir* cur)
+                           crt_options options, crt_raygen prev_cam, const crt_reservoir* prev, crt_reservoir* cur,
+                           const crt_visibility* prev_vis)
 {
     const TilePix t = this_pixel(W, H, rows);
     if (t.in)
-        px_temporal<Math<MODE>>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
-                                AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur}, &prev_cam, W, H);
+        px_temporal<Math<MODE>, RW>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
+                                    AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur}, &prev_cam, W, H, prev_vis);
 }
 // 10_restir_di.cu:239-254 (the first buffer is the source).  Every pixel is copied, so the bottom-up
 // index permutation does not matter: plain word copy.
@@ -430,15 +433,45 @@ extern "C" int crt_temporal_resampling_reprojected(crt_ctx* ctx, int W, int H, i
     CRT_CHECK_BUF(reservoirs, (size_t)W * H, "reservoir");
     CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "reprojection reads other pixels of the previous buffer: it cannot run in place");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
-    CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED, "unbiased reuse weights do not take a previous camera: the history "
-                                                       "pixel's surface in the previous frame is not kept");
+    CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED, "unbiased reuse weights do not take a previous camera here: this call does not receive "
+                                                       "the previous frame's surfaces (crt_temporal_resampling_reprojected_surfaces does)");
     const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_temporal_reprojected<1, true> : k_temporal_reprojected<1, false>)
-                : (sh ? k_temporal_reprojected<0, true> : k_temporal_reprojected<0, false>);
+    auto k = ex ? (sh ? k_temporal_reprojected<1, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<1, false, CRT_REUSE_REFERENCE>)
+                : (sh ? k_temporal_reprojected<0, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<0, false, CRT_REUSE_REFERENCE>);
     k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
                                                (const crt_visibility*)visibility_buffer.data, to_f3(eye), options, previous_raygen,
-                                               (const crt_reservoir*)previous_reservoirs.data, (crt_reservoir*)reservoirs.data);
+                                               (const crt_reservoir*)previous_reservoirs.data, (crt_reservoir*)reservoirs.data,
+                                               nullptr);
     return check_launch(ctx, "temporal_resampling_reprojected");
+}
+
+extern "C" int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom,
+                                                            crt_buffer triangles, crt_buffer visibility_buffer, crt_float3 eye,
+                                                            crt_options options, crt_raygen previous_raygen,
+                                                            crt_buffer previous_visibility_buffer,
+                                                            crt_buffer previous_reservoirs, crt_buffer reservoirs)
+{
+    CRT_REQUIRE(ctx && geom, "null context or geometry");
+    CRT_CHECK_IMAGE(W, H);
+    CRT_CHECK_BUF(visibility_buffer, (size_t)W * H, "visibility");
+    CRT_CHECK_BUF(previous_visibility_buffer, (size_t)W * H, "previous visibility");
+    CRT_CHECK_BUF(previous_reservoirs, (size_t)W * H, "previous reservoir");
+    CRT_CHECK_BUF(reservoirs, (size_t)W * H, "reservoir");
+    CRT_REQUIRE(previous_visibility_buffer.data != visibility_buffer.data,
+                "the previous frame's Visibility must be a buffer of its own: this frame's raycast has overwritten it");
+    CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "reprojection reads other pixels of the previous buffer: it cannot run in place");
+    CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
+    const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
+    auto k = ex ? (sh ? k_temporal_reprojected<1, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<1, false, CRT_REUSE_REFERENCE>)
+                : (sh ? k_temporal_reprojected<0, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<0, false, CRT_REUSE_REFERENCE>);
+    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
+        k = ex ? (sh ? k_temporal_reprojected<1, true, CRT_REUSE_UNBIASED> : k_temporal_reprojected<1, false, CRT_REUSE_UNBIASED>)
+               : (sh ? k_temporal_reprojected<0, true, CRT_REUSE_UNBIASED> : k_temporal_reprojected<0, false, CRT_REUSE_UNBIASED>);
+    k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
+                                               (const crt_visibility*)visibility_buffer.data, to_f3(eye), options, previous_raygen,
+                                               (const crt_reservoir*)previous_reservoirs.data, (crt_reservoir*)reservoirs.data,
+                                               (const crt_visibility*)previous_visibility_buffer.data);
+    return check_launch(ctx, "temporal_resampling_reprojected_surfaces");
 }
 
 extern "C" int crt_save_temporal_reservoir(crt_ctx* ctx, int W, int H, crt_buffer src, crt_buffer dst)

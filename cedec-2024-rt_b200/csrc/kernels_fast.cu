@@ -63,8 +63,8 @@ __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
     queue_push(q, d.want, to_shadow_ray(d, t.px.idx), d.decided);
 }
 // the same with temporal reprojection (px_candidate_temporal<..., REPROJ = true>); a kernel of its own so that the
-// in-place kernel above keeps its registers and its code
-template <class L, int MODE>
+// in-place kernel above keeps its registers and its code.  RW = CRT_REUSE_UNBIASED reads rp.prev_vis at the history pixel.
+template <class L, int MODE, int RW>
 __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
     k_candidate_temporal_reprojected(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
                                      L lights, crt_options options, SoaStore temporal, GBuf g, ShadowQueue q, HaloPeers peers, Reprojection rp)
@@ -73,7 +73,7 @@ __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
     DeferredRay d{false, {0, 0, 0}, {0, 0, 0}};
     CandPixel cp{Vis{0.0f, 0.0f, -1}, true};
     if (t.in) cp = classify_pixel(t.px, tris60, vis);
-    if (t.in) d = px_candidate_temporal<Math<MODE>, L, true>(t.px, cp, frame, bvh, tris60, eye, lights, make_opt(options), temporal, g, peers, 0u, rp);
+    if (t.in) d = px_candidate_temporal<Math<MODE>, L, true, RW>(t.px, cp, frame, bvh, tris60, eye, lights, make_opt(options), temporal, g, peers, 0u, rp);
     queue_push(q, d.want, to_shadow_ray(d, t.px.idx), d.decided);
 }
 #ifndef CRT_SP_MINBLOCKS
@@ -110,23 +110,25 @@ void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, in
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
                                ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse)
 {
+    const bool unb = reuse == CRT_REUSE_UNBIASED;
     if (rp)
     {
         if (table)
         {
             const LightsTable L{table, n_lights};
-            auto k = exact ? k_candidate_temporal_reprojected<LightsTable, 1> : k_candidate_temporal_reprojected<LightsTable, 0>;
+            auto k = exact ? k_candidate_temporal_reprojected<LightsTable, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal_reprojected<LightsTable, 0, CRT_REUSE_REFERENCE>;
+            if (unb) k = exact ? k_candidate_temporal_reprojected<LightsTable, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal_reprojected<LightsTable, 0, CRT_REUSE_UNBIASED>;
             k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
         }
         else
         {
             const LightsIndexed L{tris60, light_ids, n_lights};
-            auto k = exact ? k_candidate_temporal_reprojected<LightsIndexed, 1> : k_candidate_temporal_reprojected<LightsIndexed, 0>;
+            auto k = exact ? k_candidate_temporal_reprojected<LightsIndexed, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal_reprojected<LightsIndexed, 0, CRT_REUSE_REFERENCE>;
+            if (unb) k = exact ? k_candidate_temporal_reprojected<LightsIndexed, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal_reprojected<LightsIndexed, 0, CRT_REUSE_UNBIASED>;
             k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
         }
         return;
     }
-    const bool unb = reuse == CRT_REUSE_UNBIASED;
     if (table)
     {
         const LightsTable L{table, n_lights};
@@ -330,13 +332,26 @@ extern "C" int crt_restir_output_buffer(crt_options options, const crt_restir_bu
 
 extern "C" int crt_restir_is_fused(crt_options options) { return fused(options) ? 1 : 0; }
 
+const char* const kNoSurfacesMsg = "unbiased reuse weights do not take a previous camera without the previous frame's surfaces: "
+                                   "set it with crt_restir_set_previous_frame";
+
 extern "C" int crt_restir_set_previous_camera(crt_ctx* ctx, const crt_raygen* previous_raygen)
 {
     CRT_REQUIRE(ctx, "null context");
-    CRT_REQUIRE(!previous_raygen || ctx->reuse_mode != CRT_REUSE_UNBIASED,
-                "unbiased reuse weights do not take a previous camera: the history pixel's surface in the previous frame is not kept");
+    CRT_REQUIRE(!previous_raygen || ctx->reuse_mode != CRT_REUSE_UNBIASED, kNoSurfacesMsg);
     ctx->prev_cam_set = previous_raygen != nullptr;
     if (previous_raygen) ctx->prev_cam = *previous_raygen;
+    ctx->prev_vis = crt_buffer{};
+    return CRT_OK;
+}
+
+extern "C" int crt_restir_set_previous_frame(crt_ctx* ctx, const crt_raygen* previous_raygen, crt_buffer previous_visibility)
+{
+    CRT_REQUIRE(ctx, "null context");
+    CRT_REQUIRE(!previous_raygen || previous_visibility.data != nullptr, "null previous visibility buffer");
+    ctx->prev_cam_set = previous_raygen != nullptr;
+    if (previous_raygen) ctx->prev_cam = *previous_raygen;
+    ctx->prev_vis = previous_raygen ? previous_visibility : crt_buffer{};
     return CRT_OK;
 }
 
@@ -355,13 +370,19 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     CRT_REQUIRE(ctx && geom, "null context or geometry");
     int rc = check_buffers(W, H, b);
     if (rc != CRT_OK) return rc;
+    const bool with_surfaces = ctx->prev_cam_set && ctx->prev_vis.data != nullptr;  // crt_restir_set_previous_frame
+    if (with_surfaces)
+    {
+        CRT_CHECK_BUF(ctx->prev_vis, (size_t)W * H, "previous visibility");
+        CRT_REQUIRE(ctx->prev_vis.data != b->visibility.data,
+                    "the previous frame's Visibility must be a buffer of its own: this frame's raycast overwrites buffers->visibility");
+    }
     rc = raycast_or_prefetched(ctx, W, H, geom, triangles, raygen, b->visibility);
     if (rc != CRT_OK) return rc;
     ctx->frame_fused = fused(options);
     if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
     {
-        CRT_REQUIRE(!ctx->prev_cam_set, "unbiased reuse weights do not take a previous camera: the history pixel's surface in "
-                                        "the previous frame is not kept");
+        CRT_REQUIRE(!ctx->prev_cam_set || with_surfaces, kNoSurfacesMsg);
         CRT_REQUIRE(unbiased_rows_ok(ctx, H, options), kUnbiasedRowsMsg);
     }
     if (ctx->links_set)
@@ -385,9 +406,12 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     {
         rc = crt_generate_candidate(ctx, W, H, frame, geom, triangles, b->visibility, eye, lights, options, b->reservoir0);
         if (rc == CRT_OK)
-            rc = ctx->prev_cam_set ? crt_temporal_resampling_reprojected(ctx, W, H, frame, geom, triangles, b->visibility, eye, options,
-                                                                         ctx->prev_cam, b->temporal, b->reservoir0)
-                                   : crt_temporal_resampling(ctx, W, H, frame, geom, triangles, b->visibility, eye, options, b->temporal, b->reservoir0);
+            rc = with_surfaces       ? crt_temporal_resampling_reprojected_surfaces(ctx, W, H, frame, geom, triangles, b->visibility, eye,
+                                                                                    options, ctx->prev_cam, ctx->prev_vis, b->temporal,
+                                                                                    b->reservoir0)
+                 : ctx->prev_cam_set ? crt_temporal_resampling_reprojected(ctx, W, H, frame, geom, triangles, b->visibility, eye, options,
+                                                                           ctx->prev_cam, b->temporal, b->reservoir0)
+                                     : crt_temporal_resampling(ctx, W, H, frame, geom, triangles, b->visibility, eye, options, b->temporal, b->reservoir0);
         if (rc == CRT_OK) rc = crt_save_temporal_reservoir(ctx, W, H, b->reservoir0, b->temporal);
         return rc;
     }
@@ -446,6 +470,8 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
         rp.prev_cam = ctx->prev_cam;
         rp.W = W;
         rp.H = H;
+        rp.prev_vis = (const crt_visibility*)ctx->prev_vis.data;
+        rp.prev_eye = to_f3(ctx->prev_cam.m_origin);
     }
     CRT_MODE_NS(ctx, launch_candidate_temporal)(
         ctx->stream, exact, grid, W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), table,

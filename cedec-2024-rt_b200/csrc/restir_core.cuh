@@ -702,6 +702,32 @@ CRT_HD bool temporal_merge_unbiased(const Bvh& bvh, const Surf& surf, f3 eye, co
     r.ucw = ucw_unbiased(r.w_sum, c_own + prev.M, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, opt.shadowed));
     return accepted;
 }
+// temporal_merge_unbiased with reprojection (DESIGN.md section 15, "Reprojection"): the history's pixel h is the reprojected
+// one and its surface S_h = `hsurf` the previous frame's primary hit there (from the previous Visibility record and the
+// previous eye).  has_h = false (no history pixel, sky at h, or M_h = 0) gives c_h = 0.  c_h = trunc(min(M_h, cap) *
+// heuristics(S_q, S_h)) with this frame's eye, and Z = c_own [p_hat_q(y) > 0] + c_h [p_hat_h(y) > 0].  With S_h = S_q this
+// computes temporal_merge_unbiased's bits.
+template <class M>
+CRT_HD bool temporal_merge_unbiased_reprojected(const Bvh& bvh, const Surf& surf, bool has_h, const Surf& hsurf, f3 eye,
+                                                const Opt& opt, Res prev, Res& r, Pcg& rng)
+{
+    const int cap = 20 * opt.ris_count;  // M-cap, :186-188
+    prev.M = prev.M < cap ? prev.M : cap;
+    const float p_hat_y = target_function(bvh, surf.p, surf.n, prev.s.hp, prev.s.hn, prev.s.rad, opt.shadowed);
+    const int c_own = r.M;
+    prev.M = has_h ? confidence<M>(prev.M, surf, hsurf, eye) : 0;
+    const float weight = p_hat_y * prev.ucw * (float)prev.M;
+    const float u = rng.next_f();
+    r.w_sum += weight;
+    r.M += prev.M;
+    const bool accepted = u < weight / r.w_sum;
+    if (accepted) r.s = prev.s;
+    const float p_hat = target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, opt.shadowed);
+    int z = c_own;  // ucw_unbiased reads p_hat_q(y) > 0 itself
+    if (p_hat > 0.0f && prev.M > 0) z = z_of(z, prev.M, bvh, hsurf, r.s, opt.shadowed);
+    r.ucw = ucw_unbiased(r.w_sum, z, p_hat);
+    return accepted;
+}
 // spatial_merge with unbiased weights: `nsurf` is the neighbour pixel's surface, `nb` its input reservoir
 template <class M>
 CRT_HD void spatial_merge_unbiased(const Bvh& bvh, const Surf& surf, const Surf& nsurf, f3 eye, const Opt& opt, const Res& nb,

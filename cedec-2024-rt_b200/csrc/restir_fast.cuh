@@ -231,13 +231,19 @@ CRT_HD unsigned complete_pairs(unsigned lanes) { return lanes & (((lanes & 0x555
 // REPROJ (extension, DESIGN.md section 11): the history is read from `history` — a snapshot of last frame's `temporal` —
 // at the pixel this surface point had in the previous frame's camera (reproject_pixel, restir_core.cuh), Reservoir{} when
 // it had none; `temporal` is only written.  Otherwise the history is `temporal` at this pixel, merged in place.
+// prev_vis / prev_eye: the previous frame's Visibility buffer and eye (crt_restir_set_previous_frame), read by
+// CRT_REUSE_UNBIASED only — the history pixel's surface (DESIGN.md section 15)
 struct Reprojection
 {
     SoaStore history{nullptr, 0};
     crt_raygen prev_cam{};
     int W = 0, H = 0;
+    const crt_visibility* prev_vis = nullptr;
+    f3 prev_eye{0.0f, 0.0f, 0.0f};
 };
-// RW: CRT_REUSE_REFERENCE, or CRT_REUSE_UNBIASED (temporal_merge_unbiased; not combined with REPROJ)
+// RW: CRT_REUSE_REFERENCE, or CRT_REUSE_UNBIASED: temporal_merge_unbiased, and with REPROJ
+// temporal_merge_unbiased_reprojected on the history pixel's previous surface — one 16-byte Visibility load and the
+// triangle's 36 vertex bytes at the history pixel, only when the history has M > 0
 template <class M, class L, bool REPROJ = false, int RW = CRT_REUSE_REFERENCE>
 CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int frame, const Bvh& bvh, const float* tris60,
                                          f3 eye, const L& lights, const Opt& opt_in, const SoaStore& temporal,
@@ -269,14 +275,20 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
     {
         Pcg rng_t(hash_pcg4(px.xi, px.yi, frame, 1), 0);
         Res history;
+        bool has_h = false;
+        Surf hsurf{};
         if (REPROJ)
         {
             int xp, yp;
-            history = reproject_pixel(to_raygen(rp.prev_cam), rp.W, rp.H, surf.p, xp, yp) ? rp.history.load(xp + (rp.H - yp - 1) * rp.W)
-                                                                                          : empty_res();
+            const bool found = reproject_pixel(to_raygen(rp.prev_cam), rp.W, rp.H, surf.p, xp, yp);
+            history = found ? rp.history.load(xp + (rp.H - yp - 1) * rp.W) : empty_res();
+            if (RW == CRT_REUSE_UNBIASED && found && history.M > 0)
+                has_h = previous_surface(rp.prev_vis, tris60, xp + (rp.H - yp - 1) * rp.W, rp.prev_eye, hsurf);
         }
         else history = temporal.load(px.idx);
-        if (RW == CRT_REUSE_UNBIASED) candidate_survives = !temporal_merge_unbiased<M>(bvh, surf, eye, opt, history, r, rng_t);
+        if (RW == CRT_REUSE_UNBIASED && REPROJ)
+            candidate_survives = !temporal_merge_unbiased_reprojected<M>(bvh, surf, has_h, hsurf, eye, opt, history, r, rng_t);
+        else if (RW == CRT_REUSE_UNBIASED) candidate_survives = !temporal_merge_unbiased<M>(bvh, surf, eye, opt, history, r, rng_t);
         else candidate_survives = !temporal_merge<M>(bvh, surf, eye, opt, history, r, rng_t);
     }
     if (opt.reuse && candidate_survives)

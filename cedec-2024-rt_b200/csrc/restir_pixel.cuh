@@ -83,6 +83,16 @@ CRT_HD void primary_ray(const crt_raygen& raygen, const Pix& px, int W, int H, f
 {
     shoot(to_raygen(raygen), (float)px.xi / (float)W, (float)px.yi / (float)H, ro, rd);
 }
+// The previous frame's primary-hit surface at pixel `idx`: its Visibility record and the eye that frame flipped the
+// normal towards (its RayGenerator's origin: crt_raygen_lookat stores the eye).  False on a sky pixel.  Primary rays are
+// deterministic and the geometry static, so this is the surface that frame's kernels used there.
+CRT_HD bool previous_surface(const crt_visibility* prev_vis, const float* tris60, int idx, f3 prev_eye, Surf& s)
+{
+    const Vis hv = load_vis(prev_vis, idx);
+    if (hv.index == -1) return false;
+    s = surface_from_visibility(tri_at(tris60, hv.index), hv.u, hv.v, prev_eye);
+    return true;
+}
 
 // ---- 10_restir_di.cu:9-34
 CRT_HD void px_raycast(const Pix& px, int W, int H, const Bvh& bvh, const crt_raygen& raygen, crt_visibility* vis)
@@ -185,11 +195,13 @@ CRT_HD DeferredRay px_generate_candidate(const Pix& px, int frame, const Bvh& bv
 // ---- 10_restir_di.cu:137-237
 // prev_cam != nullptr (extension: crt_temporal_resampling_reprojected): the previous reservoir is read at the pixel this
 // surface point had in the previous frame's camera; no history there = Reservoir{} (restir_core.cuh: reproject_pixel)
-// RW: CRT_REUSE_REFERENCE (the reference's merge) or CRT_REUSE_UNBIASED (temporal_merge_unbiased; no reprojection)
+// RW: CRT_REUSE_REFERENCE (the reference's merge) or CRT_REUSE_UNBIASED: temporal_merge_unbiased without a previous
+// camera, temporal_merge_unbiased_reprojected with one — the history's surface is then the previous frame's at the
+// history pixel, from `prev_vis` (the previous frame's Visibility buffer, read there only; unused by the reference's merge)
 template <class M, int RW = CRT_REUSE_REFERENCE, class RSP, class RS>
 CRT_HD void px_temporal(const Pix& px, int frame, const Bvh& bvh, const float* tris60, const crt_visibility* vis,
                         f3 eye, const Opt& opt, const RSP& prev, const RS& cur, const crt_raygen* prev_cam = nullptr,
-                        int W = 0, int H = 0)
+                        int W = 0, int H = 0, const crt_visibility* prev_vis = nullptr)
 {
     const Vis v = load_vis(vis, px.idx);
     if (v.index == -1) return;
@@ -200,13 +212,20 @@ CRT_HD void px_temporal(const Pix& px, int frame, const Bvh& bvh, const float* t
     const Surf surf = surface_from_visibility(tri, v.u, v.v, eye);
     Res r = cur.load(px.idx);
     Res history;
+    bool has_h = false;
+    Surf hsurf{};
     if (prev_cam)
     {
         int xp, yp;
-        history = reproject_pixel(to_raygen(*prev_cam), W, H, surf.p, xp, yp) ? prev.load(xp + (H - yp - 1) * W) : empty_res();
+        const bool found = reproject_pixel(to_raygen(*prev_cam), W, H, surf.p, xp, yp);
+        history = found ? prev.load(xp + (H - yp - 1) * W) : empty_res();
+        if (RW == CRT_REUSE_UNBIASED && found && history.M > 0)
+            has_h = previous_surface(prev_vis, tris60, xp + (H - yp - 1) * W, to_raygen(*prev_cam).origin, hsurf);
     }
     else history = prev.load(px.idx);
-    if (RW == CRT_REUSE_UNBIASED) temporal_merge_unbiased<M>(bvh, surf, eye, opt, history, r, rng);
+    if (RW == CRT_REUSE_UNBIASED && prev_cam)
+        temporal_merge_unbiased_reprojected<M>(bvh, surf, has_h, hsurf, eye, opt, history, r, rng);
+    else if (RW == CRT_REUSE_UNBIASED) temporal_merge_unbiased<M>(bvh, surf, eye, opt, history, r, rng);
     else temporal_merge<M>(bvh, surf, eye, opt, history, r, rng);
     cur.store(px.idx, r);
 }

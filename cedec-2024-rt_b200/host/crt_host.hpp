@@ -52,6 +52,22 @@ class Device
     void setLightSampling(int mode, int log2_slots = 0) const { CRT_CHECKED(crt_set_light_sampling(m_ctx, mode, log2_slots)); }
     // CRT_REUSE_REFERENCE (the reference) or CRT_REUSE_UNBIASED (1/Z weights in every temporal and spatial merge)
     void setReuseWeights(int mode) const { CRT_CHECKED(crt_set_reuse_weights(m_ctx, mode)); }
+    // temporal reprojection in the fused frame with the previous frame's Visibility buffer (what CRT_REUSE_UNBIASED needs
+    // with a moving camera); the host keeps that buffer until the next frame has begun.  nullptr clears both.
+    void setPreviousFrame(const crt_raygen* previous_raygen, crt_buffer previous_visibility) const
+    {
+        CRT_CHECKED(crt_restir_set_previous_frame(m_ctx, previous_raygen, previous_visibility));
+    }
+    // the launch list's reprojected temporal resampling with the previous frame's Visibility buffer
+    void temporalResamplingReprojectedSurfaces(int width, int height, int frame, crt_geometry geom, crt_buffer triangles,
+                                               crt_buffer visibility, crt_float3 eye, crt_options options,
+                                               crt_raygen previous_raygen, crt_buffer previous_visibility,
+                                               crt_buffer previous_reservoirs, crt_buffer reservoirs) const
+    {
+        CRT_CHECKED(crt_temporal_resampling_reprojected_surfaces(m_ctx, width, height, frame, geom, triangles, visibility, eye,
+                                                                 options, previous_raygen, previous_visibility,
+                                                                 previous_reservoirs, reservoirs));
+    }
 
    private:
     crt_ctx* m_ctx = nullptr;

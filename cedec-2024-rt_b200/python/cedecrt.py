@@ -154,6 +154,7 @@ def _load():
         "crt_generate_candidate": [P, I, I, I, G, B, B, Float3, B, Options, B],
         "crt_temporal_resampling": [P, I, I, I, G, B, B, Float3, Options, B, B],
         "crt_temporal_resampling_reprojected": [P, I, I, I, G, B, B, Float3, Options, RayGenerator, B, B],
+        "crt_temporal_resampling_reprojected_surfaces": [P, I, I, I, G, B, B, Float3, Options, RayGenerator, B, B, B],
         "crt_save_temporal_reservoir": [P, I, I, B, B],
         "crt_spatial_resampling": [P, I, I, I, I, G, B, B, Float3, Options, B, B],
         "crt_resolve": [P, B, I, I, G, B, B, Float3, Options, B],
@@ -170,6 +171,7 @@ def _load():
         "crt_restir_output_buffer": [Options, C.POINTER(RestirBuffers), C.POINTER(B)],
         "crt_restir_is_fused": [Options],
         "crt_restir_set_previous_camera": [P, C.POINTER(RayGenerator)],
+        "crt_restir_set_previous_frame": [P, C.POINTER(RayGenerator), B],
         "crt_restir_class_plane": [P, C.POINTER(C.c_void_p)],
         "crt_reservoir_export_aos": [P, I, I, B, B],
         "crt_reservoir_import_aos": [P, I, I, B, B],
@@ -481,6 +483,14 @@ class Runtime:
                                                                  visibility.arg(), Float3(*eye), options, prev_raygen,
                                                                  previous.arg(), reservoirs.arg()))
 
+    def temporal_resampling_reprojected_surfaces(self, W, H, frame, geom, triangles, visibility, eye, options, prev_raygen,
+                                                 prev_visibility, previous, reservoirs):
+        """temporal_resampling_reprojected that also reads the previous frame's Visibility buffer at the history pixel: the
+        history's surface under REUSE_UNBIASED (include/cedecrt.h: crt_temporal_resampling_reprojected_surfaces)"""
+        self._check(self.lib.crt_temporal_resampling_reprojected_surfaces(
+            self.ctx, W, H, frame, geom.handle, triangles.arg(), visibility.arg(), Float3(*eye), options, prev_raygen,
+            prev_visibility.arg(), previous.arg(), reservoirs.arg()))
+
     def save_temporal_reservoir(self, W, H, src, dst):
         self._check(self.lib.crt_save_temporal_reservoir(self.ctx, W, H, src.arg(), dst.arg()))
 
@@ -520,6 +530,12 @@ class Runtime:
     def restir_set_previous_camera(self, raygen):
         """temporal reprojection inside the fused frame: the previous frame's camera, or None for the reference's same-pixel history"""
         self._check(self.lib.crt_restir_set_previous_camera(self.ctx, C.byref(raygen) if raygen is not None else None))
+
+    def restir_set_previous_frame(self, raygen, visibility):
+        """restir_set_previous_camera plus the previous frame's Visibility buffer, kept by the host until the next frame has
+        begun (include/cedecrt.h: crt_restir_set_previous_frame); raygen None clears both"""
+        vis = visibility.arg() if raygen is not None else _Buffer()
+        self._check(self.lib.crt_restir_set_previous_frame(self.ctx, C.byref(raygen) if raygen is not None else None, vis))
 
     def restir_di_frame(self, W, H, frame, geom, triangles, raygen, eye, lights, options, bufs):
         self._check(self.lib.crt_restir_di_frame(self.ctx, W, H, frame, geom.handle, triangles.arg(), raygen,
@@ -610,7 +626,11 @@ class RestirDI:
         fused=True: one crt_restir_di_frame call per frame (SoA reservoirs inside the same buffers).
         reproject=True (extension): temporal resampling looks the previous reservoir up at the pixel the surface point had
         in the previous frame's camera (crt_temporal_resampling_reprojected; in fused mode crt_restir_set_previous_camera);
-        set_camera() moves the camera and clears the accumulation like the reference's loop (10_restir_di.cpp:257-267)."""
+        set_camera() moves the camera and clears the accumulation like the reference's loop (10_restir_di.cpp:257-267).
+        reproject="surfaces": the same look-up with the previous frame's surfaces, which unbiased reuse weights need with a
+        moving camera: two Visibility buffers alternate and last frame's is passed on (the launch list's
+        crt_temporal_resampling_reprojected_surfaces; in fused mode crt_restir_set_previous_frame)."""
+        assert reproject in (False, True, "surfaces"), reproject
         self.rt, self.W, self.H, self.fused = rt, width, height, fused
         self.reproject, self.prev_raygen = reproject, None
         self.prefetch = False  # fused + crt_set_frame_overlap: trace the next frame's primary rays right after issuing a frame
@@ -624,6 +644,8 @@ class RestirDI:
         self.pixels = rt.buffer(np.uint8, 4 * n)
         self.accumulation = rt.buffer(FLOAT4, n)
         self.visibility = rt.buffer(VISIBILITY, n)
+        # reproject="surfaces": last frame's Visibility, kept for one more frame (the two buffers swap at each frame)
+        self.prev_visibility = rt.buffer(VISIBILITY, n) if reproject == "surfaces" else None
         self.reservoir0 = rt.buffer(RESERVOIR, n)
         self.reservoir1 = rt.buffer(RESERVOIR, n)
         # the reference leaves this uninitialised (10_restir_di.cpp:121-122); zero = "no history" (M = 0)
@@ -654,13 +676,18 @@ class RestirDI:
         return tmp.to_host()
 
     def frame(self):
+        surfaces = self.reproject == "surfaces"
+        if surfaces:  # this frame traces into the buffer two frames old; last frame's becomes the previous one
+            self.visibility, self.prev_visibility = self.prev_visibility, self.visibility
         rt, W, H, o, g, t, v, eye = (self.rt, self.W, self.H, self.options, self.geom, self.triangles,
                                      self.visibility, self.eye)
         self.frame_index += 1
         f = self.frame_index
         if self.fused:
             bufs = rt.restir_buffers(self.pixels, self.accumulation, v, self.reservoir0, self.reservoir1, self.temporal)
-            if self.reproject:
+            if surfaces:
+                rt.restir_set_previous_frame(self.prev_raygen, self.prev_visibility)  # None before the first frame
+            elif self.reproject:
                 rt.restir_set_previous_camera(self.prev_raygen)  # None before the first frame: no history to look up
             rt.restir_di_frame(W, H, f, g, t, self.raygen, eye, self.lights, o, bufs)
             if self.reproject:
@@ -671,7 +698,10 @@ class RestirDI:
             return
         rt.raycast(W, H, g, t, self.raygen, v)
         rt.generate_candidate(W, H, f, g, t, v, eye, self.lights, o, self.reservoir0)
-        if self.reproject and self.prev_raygen is not None:
+        if surfaces and self.prev_raygen is not None:
+            rt.temporal_resampling_reprojected_surfaces(W, H, f, g, t, v, eye, o, self.prev_raygen, self.prev_visibility,
+                                                        self.temporal, self.reservoir0)
+        elif self.reproject and self.prev_raygen is not None:
             rt.temporal_resampling_reprojected(W, H, f, g, t, v, eye, o, self.prev_raygen, self.temporal, self.reservoir0)
         else:
             rt.temporal_resampling(W, H, f, g, t, v, eye, o, self.temporal, self.reservoir0)

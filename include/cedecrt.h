@@ -147,9 +147,11 @@ int crt_lights_changed(crt_ctx* ctx, crt_geometry geom);
  *                        Candidate generation is a single domain and unchanged.  Without reprojection the history's
  *                        surface is the pixel's own, so temporal Z = M whenever p_hat_q(y) > 0.  Unbiased for static
  *                        geometry: the first merge after crt_refit_geometry is not exactly so.
- * CRT_REUSE_UNBIASED is refused (CRT_EINVAL) with a previous camera (crt_temporal_resampling_reprojected, and a camera
- * set with crt_restir_set_previous_camera) and in the fused frame on a row range narrower than the image or with slab
- * links (the G-buffer of halo rows is not kept); the per-kernel path takes row ranges.  An unknown mode is CRT_EINVAL. */
+ * CRT_REUSE_UNBIASED is refused (CRT_EINVAL) with a previous camera that comes without the previous frame's surfaces
+ * (crt_temporal_resampling_reprojected, and a camera set with crt_restir_set_previous_camera: use
+ * crt_temporal_resampling_reprojected_surfaces and crt_restir_set_previous_frame) and in the fused frame on a row range
+ * narrower than the image or with slab links (the G-buffer of halo rows is not kept); the per-kernel path takes row
+ * ranges.  An unknown mode is CRT_EINVAL. */
 enum { CRT_REUSE_REFERENCE = 0, CRT_REUSE_UNBIASED = 1 };
 int crt_set_reuse_weights(crt_ctx* ctx, int mode);
 /* Multi-GPU row slabs: the kernels of this context compute only image rows yi in [y_begin, y_end) (y_end < 0:
@@ -282,6 +284,35 @@ int crt_temporal_resampling_reprojected(crt_ctx* ctx, int width, int height, int
  * the 87 halo rows only and the call refuses them.  With the previous camera equal to the current one the frame equals
  * the plain fused frame bit for bit. */
 int crt_restir_set_previous_camera(crt_ctx* ctx, const crt_raygen* previous_raygen);
+/* Reprojection that also receives the previous frame's surfaces (extension; DESIGN.md section 15, "Reprojection"): what
+ * CRT_REUSE_UNBIASED needs with a moving camera.  crt_temporal_resampling_reprojected with one more input,
+ * `previous_visibility_buffer`: last frame's Visibility buffer, which the host keeps for one more frame instead of tracing
+ * over it (two Visibility buffers, alternated).  It is read at the history pixel h only.  Under CRT_REUSE_UNBIASED the
+ * history's surface is S_h = make_surface_info of that record with the previous eye (previous_raygen.m_origin), its
+ * confidence c_h = trunc(min(M_h, 20 * ris_sample_count) * rejection_heuristics(S_q, S_h)) with this frame's eye (0 when
+ * h has no history, is sky, or M_h = 0), the history merges with weight p_hat_q(y_h) * ucw_h * c_h, M accumulates c_h, and
+ *   Z = c_own [p_hat_q(y) > 0] + c_h [p_hat_h(y) > 0],   ucw = p_hat_q(y) > 0 && Z > 0 ? w_sum / (Z p_hat_q(y)) : 0
+ * with p_hat_h the target function at S_h (a shadow ray from S_h under use_shadowed_target_function, traced only when
+ * the unshadowed value is positive).  With an unmoved camera and this frame's Visibility as the previous one it equals
+ * crt_temporal_resampling under CRT_REUSE_UNBIASED bit for bit.  Under CRT_REUSE_REFERENCE the previous Visibility is
+ * not read and the result equals crt_temporal_resampling_reprojected bit for bit.  Unbiased for static geometry.
+ * CRT_EINVAL: a buffer smaller than width * height, `previous_visibility_buffer` equal to `visibility_buffer`, or
+ * `previous_reservoirs` equal to `reservoirs`.  Row ranges: the host provides every row of `previous_reservoirs` and
+ * `previous_visibility_buffer` the look-ups can reach.  crt_launch name: "temporal_resampling_reprojected_surfaces"
+ * (previous_visibility_buffer is the 10th param). */
+int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int width, int height, int frame, crt_geometry geom,
+                                                 crt_buffer triangles, crt_buffer visibility_buffer, crt_float3 eye,
+                                                 crt_options options, crt_raygen previous_raygen,
+                                                 crt_buffer previous_visibility_buffer, crt_buffer previous_reservoirs,
+                                                 crt_buffer reservoirs);
+/* The same inside the fused frame: crt_restir_set_previous_camera plus the previous frame's Visibility buffer, which the
+ * context stores (not copies) until it is cleared: the host keeps it unchanged until the next crt_restir_frame_begin has
+ * run.  NULL previous_raygen clears both; crt_restir_set_previous_camera clears the stored Visibility.  Under
+ * CRT_REUSE_UNBIASED crt_restir_frame_begin accepts a previous camera only when it was set here.  The frame checks
+ * (CRT_EINVAL) that the buffer holds width * height records and is not buffers->visibility, which its raycast
+ * overwrites; options that take the per-kernel path use crt_temporal_resampling_reprojected_surfaces.  The fused frame
+ * with unbiased weights still refuses row ranges and slab links. */
+int crt_restir_set_previous_frame(crt_ctx* ctx, const crt_raygen* previous_raygen, crt_buffer previous_visibility);
 /* 10_restir_di.cu:239-254 — note the reference's parameter names are swapped: the first buffer is the source */
 int crt_save_temporal_reservoir(crt_ctx* ctx, int width, int height, crt_buffer src, crt_buffer dst);
 /* 10_restir_di.cu:256-388 */
