@@ -83,6 +83,7 @@ extern "C" int crt_shutdown(crt_ctx* ctx)
     if (ctx->queue_rays) cudaFree(ctx->queue_rays);
     if (ctx->queue_counters) cudaFree(ctx->queue_counters);
     if (ctx->history_prev) cudaFree(ctx->history_prev);
+    if (ctx->halo_vis) cudaFree(ctx->halo_vis);
     if (ctx->gbuf) cudaFree(ctx->gbuf);
     if (ctx->inline_rays) cudaFree(ctx->inline_rays);
     if (ctx->ao_count) cudaFree(ctx->ao_count);
@@ -121,8 +122,8 @@ extern "C" int crt_set_reuse_weights(crt_ctx* ctx, int mode)
 {
     CRT_REQUIRE(ctx, "null context");
     CRT_REQUIRE(mode == CRT_REUSE_REFERENCE || mode == CRT_REUSE_UNBIASED, "unknown reuse weight mode");
-    // the combinations CRT_REUSE_UNBIASED does not cover (a previous camera, the fused frame on a row range) are refused by
-    // the calls that would run them
+    // the combinations CRT_REUSE_UNBIASED does not cover (a previous camera without surfaces, the fused frame on a row range
+    // without crt_restir_set_halo_surfaces) are refused by the calls that would run them
     ctx->reuse_mode = mode;
     return CRT_OK;
 }

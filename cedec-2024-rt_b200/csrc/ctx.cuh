@@ -69,6 +69,13 @@ struct crt_ctx
     crt_buffer prev_vis = {};
     void* history_prev = nullptr;
     size_t history_prev_pixels = 0;
+    // CRT_REUSE_UNBIASED in the fused frame on a row range (crt_restir_set_halo_surfaces): the G-buffer records of the rows
+    // the spatial passes read beyond the range, from primary rays traced into a Visibility buffer of the context's own
+    int halo_surfaces = 0;
+    void* halo_vis = nullptr;      // two bands of h * W records (kernels_fast.cu: halo_surfaces)
+    size_t halo_vis_pixels = 0;    // records allocated
+    int halo_reach = 0;            // rows on each side of the range the last crt_restir_frame_begin covered (0: none)
+    int halo_dims[2] = {0, 0};     // and the image size it covered them for
     int resolve_reuse = 1;  // 0: resolve traces every shadow ray like the reference (CRT_RESOLVE_REUSE=0)
     // slab_p2p.cu: peer pointers of the neighbouring slabs and the exchange counter
     crt_slab_links links = {};

@@ -336,6 +336,17 @@ int raycast_or_prefetched(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_buf
     ctx->vis_consumed_pending = true;
     return CRT_OK;
 }
+// primary rays of rows [rows.y0, rows.y1) into `vis` on the context's stream, hinted under the licence the frame's
+// raycast_or_prefetched has just renewed (the halo bands of crt_restir_set_halo_surfaces)
+int raycast_rows(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_raygen raygen, Rows rows, crt_visibility* vis, const char* what)
+{
+    if (ctx->raycast_hint && ctx->hint_tris != nullptr && ctx->hint_tris == (const void*)geom->src && geom->n_tris)
+        k_raycast_hinted<<<tile_grid(W, rows), 256, 0, ctx->stream>>>(W, H, rows, geom->view(), raygen, vis, (const float*)geom->src,
+                                                                      (uint32_t)geom->n_tris);
+    else
+        k_raycast<<<tile_grid(W, rows), 256, 0, ctx->stream>>>(W, H, rows, geom->view(), raygen, vis);
+    return check_launch(ctx, what);
+}
 }  // namespace crt
 
 extern "C" int crt_generate_candidate(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,

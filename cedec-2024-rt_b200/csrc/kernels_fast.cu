@@ -103,6 +103,13 @@ __global__ void __launch_bounds__(256)
     // L2's limit; in k_candidate_temporal, 2 ms long, the per-warp form is the faster one: 2.035 against 2.086 ms)
     queue_push_block(q, d.want, r);
 }
+// G-buffer records of halo rows (crt_restir_set_halo_surfaces) from the context's own Visibility of those rows
+__global__ void __launch_bounds__(256)
+    k_halo_surfaces(int W, int H, Rows rows, const float* tris60, const crt_visibility* vis, f3 eye, GBuf g)
+{
+    const TilePix t = this_pixel(W, H, rows);
+    if (t.in) px_halo_surface(t.px, tris60, vis, eye, g);
+}
 
 // host-side launchers, one set per namespace (the API below picks the namespace from the context's math mode)
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
@@ -156,6 +163,11 @@ void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H,
 {
     k_resolve_fast<<<grid, 256, 0, st>>>(accum, W, H, rows, tris60, vis, res, g, q, accumulate, reuse_traced);
 }
+void launch_halo_surfaces(cudaStream_t st, dim3 grid, int W, int H, Rows rows, const float* tris60, const crt_visibility* vis,
+                          f3 eye, GBuf g)
+{
+    k_halo_surfaces<<<grid, 256, 0, st>>>(W, H, rows, tris60, vis, eye, g);
+}
 int preload()
 {
     cudaFuncAttributes a;
@@ -165,7 +177,15 @@ int preload()
     CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_REFERENCE>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0, CRT_REUSE_REFERENCE>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1, CRT_REUSE_REFERENCE>));
+    // CRT_REUSE_UNBIASED runs over slab links with halo surfaces (crt_restir_set_halo_surfaces): its kernels are loaded too
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 0, CRT_REUSE_UNBIASED>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 1, CRT_REUSE_UNBIASED>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_UNBIASED>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_UNBIASED>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0, CRT_REUSE_UNBIASED>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1, CRT_REUSE_UNBIASED>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_resolve_fast));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_halo_surfaces));
     return CRT_OK;
 }
 }  // namespace CRT_KNS
@@ -182,6 +202,8 @@ void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows r
                     crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
                     const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
+void launch_halo_surfaces(cudaStream_t st, dim3 grid, int W, int H, Rows rows, const float* tris60, const crt_visibility* vis,
+                          f3 eye, GBuf g);
 }  // namespace fm
 namespace rf
 {
@@ -194,6 +216,8 @@ void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows r
                     crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
                     const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
+void launch_halo_surfaces(cudaStream_t st, dim3 grid, int W, int H, Rows rows, const float* tris60, const crt_visibility* vis,
+                          f3 eye, GBuf g);
 }  // namespace rf
 // the namespace whose kernels implement the context's math mode
 #define CRT_MODE_NS(ctx, fn) ((ctx)->math_mode == CRT_MATH_FAST ? fm::fn : (ctx)->math_mode == CRT_MATH_REFERENCE ? rf::fn : ex::fn)
@@ -302,15 +326,65 @@ HaloPeers halo_peers(const crt_ctx* ctx, int which, Rows rows, bool with_class, 
     (void)n;
     return p;
 }
-// the fused spatial pass of CRT_REUSE_UNBIASED reads its neighbours' G-buffer records, which exist for this context's own
-// rows only (halo rows are neither computed nor mirrored): it runs on the whole image and without slab links
-bool unbiased_rows_ok(const crt_ctx* ctx, int H, const crt_options& o)
+// the fused spatial pass of CRT_REUSE_UNBIASED reads its neighbours' G-buffer records, which the candidate kernel writes for
+// this context's own rows only: it runs on the whole image and without slab links, unless the context produces the records
+// of its halo rows itself (crt_restir_set_halo_surfaces)
+bool whole_image(const crt_ctx* ctx, int H)
 {
     const Rows rows = rows_of(ctx, H);
-    return !fused(o) || (rows.y0 == 0 && rows.y1 == H && !ctx->links_set);
+    return rows.y0 == 0 && rows.y1 == H && !ctx->links_set;
 }
+bool unbiased_rows_ok(const crt_ctx* ctx, int H, const crt_options& o) { return !fused(o) || whole_image(ctx, H) || ctx->halo_surfaces; }
 const char* const kUnbiasedRowsMsg = "unbiased reuse weights in the fused frame need the whole image on one context (no row "
-                                     "range, no slab links): the G-buffer of halo rows is not kept; the per-kernel path takes row ranges";
+                                     "range, no slab links) or crt_restir_set_halo_surfaces: the G-buffer of halo rows is not "
+                                     "kept otherwise; the per-kernel path takes row ranges";
+const char* const kHaloReachMsg = "the halo surfaces of crt_restir_frame_begin do not reach as far as this spatial pass's "
+                                  "spatial_resampling_radius (or were made for another image size): begin the frame with the "
+                                  "options of its spatial passes";
+// CRT_REUSE_UNBIASED on a row range (crt_restir_set_halo_surfaces): the G-buffer records of rows [y0 - h, y0) and
+// [y1, y1 + h), clipped to the image, h = halo_rows_for(radius) — every row this frame's spatial passes can read beyond
+// the range.  Primary rays into a Visibility buffer of the context's own (the host's buffer rows outside the range belong
+// to other contexts or to an NCCL receive), then the surface of every diffuse pixel (px_halo_surface).  Records the reach
+// for crt_restir_spatial_pass.  Nothing is launched under CRT_REUSE_REFERENCE, without spatial passes, on the whole image.
+int halo_surfaces(crt_ctx* ctx, int W, int H, crt_geometry geom, const float* tris60, crt_raygen raygen, f3 eye,
+                  const crt_options& o, Rows rows, const GBuf& g)
+{
+    ctx->halo_reach = 0;
+    if (!ctx->halo_surfaces || ctx->reuse_mode != CRT_REUSE_UNBIASED || !o.use_spatial_resampling || o.spatial_resampling_passes <= 0)
+        return CRT_OK;
+    const int h = halo_rows_for(o.spatial_resampling_radius);
+    const Rows bands[2] = {{rows.y0 - h > 0 ? rows.y0 - h : 0, rows.y0}, {rows.y1, rows.y1 + h < H ? rows.y1 + h : H}};
+    // the Visibility records of the two bands only: h rows of W records each, band k at record k * h * W
+    const size_t band_cap = (size_t)h * W;
+    for (int k = 0; k < 2; k++)
+    {
+        const Rows& b = bands[k];
+        if (b.y1 <= b.y0 || rows.y1 <= rows.y0) continue;
+        if (ctx->halo_vis_pixels < 2 * band_cap)
+        {
+            if (ctx->halo_vis) CRT_CUDA(cudaFree(ctx->halo_vis));
+            ctx->halo_vis = nullptr;
+            ctx->halo_vis_pixels = 0;
+            CRT_CUDA(cudaMalloc(&ctx->halo_vis, 2 * band_cap * sizeof(crt_visibility)));
+            CRT_CUDA(cudaMemsetAsync(ctx->halo_vis, 0xff, 2 * band_cap * sizeof(crt_visibility), ctx->stream));  // index -1: no hint yet
+            ctx->halo_vis_pixels = 2 * band_cap;
+        }
+        // the kernels index records by the global pixel index: the band's first pixel, (H - b.y1) * W, lands on the slot's
+        // first record (only the band's own pixels are read or written)
+        const size_t first = (size_t)(H - b.y1) * W;
+        crt_visibility* vis = (crt_visibility*)((uintptr_t)ctx->halo_vis + (uintptr_t)(k * band_cap) * sizeof(crt_visibility) -
+                                                (uintptr_t)first * sizeof(crt_visibility));
+        int rc = raycast_rows(ctx, W, H, geom, raygen, b, vis, "halo_raycast");
+        if (rc != CRT_OK) return rc;
+        CRT_MODE_NS(ctx, launch_halo_surfaces)(ctx->stream, tile_grid(W, b), W, H, b, tris60, vis, eye, g);
+        rc = check_launch(ctx, "halo_surfaces");
+        if (rc != CRT_OK) return rc;
+    }
+    ctx->halo_reach = h;
+    ctx->halo_dims[0] = W;
+    ctx->halo_dims[1] = H;
+    return CRT_OK;
+}
 int which_of(const crt_restir_buffers* b, const crt_buffer& x) { return x.data == b->temporal.data ? 0 : x.data == b->reservoir0.data ? 1 : 2; }
 // input and output of spatial pass k in fused mode
 void pass_buffers(const crt_restir_buffers* b, int pass, crt_buffer* in, crt_buffer* out)
@@ -352,6 +426,13 @@ extern "C" int crt_restir_set_previous_frame(crt_ctx* ctx, const crt_raygen* pre
     ctx->prev_cam_set = previous_raygen != nullptr;
     if (previous_raygen) ctx->prev_cam = *previous_raygen;
     ctx->prev_vis = previous_raygen ? previous_visibility : crt_buffer{};
+    return CRT_OK;
+}
+
+extern "C" int crt_restir_set_halo_surfaces(crt_ctx* ctx, int enable)
+{
+    CRT_REQUIRE(ctx, "null context");
+    ctx->halo_surfaces = enable ? 1 : 0;
     return CRT_OK;
 }
 
@@ -442,6 +523,8 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
         ctx->history_buffer = b->temporal.data;
     }
 #endif
+    rc = halo_surfaces(ctx, W, H, geom, tris60, raygen, to_f3(eye), options, rows, g);
+    if (rc != CRT_OK) return rc;
     const dim3 grid = tile_grid(W, rows);
     const bool exact = ctx->math_mode == CRT_MATH_EXACT;
     const HaloPeers peers = halo_peers(ctx, 0, rows, true, n);
@@ -502,6 +585,10 @@ extern "C" int crt_restir_spatial_pass(crt_ctx* ctx, int W, int H, int frame, in
     }
     if (!options.use_spatial_resampling) return CRT_OK;  // the reference's disabled pass is a copy
     CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED || unbiased_rows_ok(ctx, H, options), kUnbiasedRowsMsg);
+    CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED || whole_image(ctx, H) ||
+                    (ctx->halo_dims[0] == W && ctx->halo_dims[1] == H &&
+                     halo_rows_for(options.spatial_resampling_radius) <= ctx->halo_reach),
+                kHaloReachMsg);
     CRT_REQUIRE(ctx->gbuf && ctx->gbuf_pixels >= (size_t)W * H, "crt_restir_frame_begin has not run for this image size");
     const size_t n = (size_t)W * H;
     const Rows rows = rows_of(ctx, H);

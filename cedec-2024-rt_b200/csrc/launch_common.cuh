@@ -171,6 +171,7 @@ int path_trace_wavefront(crt_ctx* ctx, int example, int W, int H, int frame, crt
                          const uint32_t* lights, uint32_t n_lights, const LightRec* slots, uint32_t n_slots, crt_raygen raygen,
                          crt_options options, crt_float4* accum, unsigned long long* counters);
 int raycast_or_prefetched(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_buffer triangles, crt_raygen raygen, crt_buffer visibility);
+int raycast_rows(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_raygen raygen, Rows rows, crt_visibility* vis, const char* what);
 int tone_mapping_on(crt_ctx* ctx, cudaStream_t st, crt_buffer pixels, crt_buffer accumulation, int W, int H);
 int preload_fused_kernels();
 int preload_dropin_kernels();

@@ -302,10 +302,23 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
     return ray;
 }
 
+// The G-buffer record of a pixel outside this context's row range (crt_restir_set_halo_surfaces): what px_candidate_temporal
+// stores there on the context that owns the row — the same Visibility record (the same primary ray, traced into a buffer of
+// this context's own), the same surface_from_visibility with this frame's eye.  Sky and emissive pixels get no record (the
+// spatial pass skips them by the neighbour's kSkipBit before it reads one), and the class plane is not written: with slab
+// links the neighbours store into those rows of it.
+CRT_HD void px_halo_surface(const Pix& px, const float* tris60, const crt_visibility* vis, f3 eye, const GBuf& g)
+{
+    const CandPixel cp = classify_pixel(px, tris60, vis);
+    if (cp.skip) return;
+    g.store(px.idx, surface_from_visibility(tri_at(tris60, cp.v.index), cp.v.u, cp.v.v, eye));
+}
+
 // px_spatial's unbiased form (CRT_REUSE_UNBIASED) on this data flow, from the pixel's input reservoir `r` and its random
 // stream: a neighbour's surface is its G-buffer record (24 bytes) instead of plane 0's sample origin, planes 1-2 are read
 // for every visited neighbour (the visibility bit weighs nothing, so there is no weightless shortcut), and the replayed
-// second pass sums Z.  The G-buffer must hold every neighbour's row: the whole image on one context.
+// second pass sums Z.  The G-buffer must hold every neighbour's row: the whole image on one context, or the halo rows
+// px_halo_surface fills on a row range.
 template <class M>
 CRT_HD void spatial_fast_unbiased(const Pix& px, int W, int H, const Bvh& bvh, f3 eye, const Opt& opt, const SoaStore& in,
                                   const GBuf& g, const Surf& surf, Pcg rng, Res& r)

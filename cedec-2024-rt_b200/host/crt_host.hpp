@@ -58,6 +58,9 @@ class Device
     {
         CRT_CHECKED(crt_restir_set_previous_frame(m_ctx, previous_raygen, previous_visibility));
     }
+    // the fused frame with CRT_REUSE_UNBIASED on a row range or with slab links: frame begin also produces the G-buffer
+    // records of the halo rows its spatial passes read; nothing changes under the reference's weights
+    void setHaloSurfaces(bool enable) const { CRT_CHECKED(crt_restir_set_halo_surfaces(m_ctx, enable ? 1 : 0)); }
     // the launch list's reprojected temporal resampling with the previous frame's Visibility buffer
     void temporalResamplingReprojectedSurfaces(int width, int height, int frame, crt_geometry geom, crt_buffer triangles,
                                                crt_buffer visibility, crt_float3 eye, crt_options options,

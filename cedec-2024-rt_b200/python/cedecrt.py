@@ -172,6 +172,7 @@ def _load():
         "crt_restir_is_fused": [Options],
         "crt_restir_set_previous_camera": [P, C.POINTER(RayGenerator)],
         "crt_restir_set_previous_frame": [P, C.POINTER(RayGenerator), B],
+        "crt_restir_set_halo_surfaces": [P, I],
         "crt_restir_class_plane": [P, C.POINTER(C.c_void_p)],
         "crt_reservoir_export_aos": [P, I, I, B, B],
         "crt_reservoir_import_aos": [P, I, I, B, B],
@@ -536,6 +537,12 @@ class Runtime:
         begun (include/cedecrt.h: crt_restir_set_previous_frame); raygen None clears both"""
         vis = visibility.arg() if raygen is not None else _Buffer()
         self._check(self.lib.crt_restir_set_previous_frame(self.ctx, C.byref(raygen) if raygen is not None else None, vis))
+
+    def restir_set_halo_surfaces(self, enable):
+        """the fused frame with unbiased reuse weights on a row range or with slab links: restir_frame_begin also produces
+        the G-buffer records of the halo rows its spatial passes read (include/cedecrt.h: crt_restir_set_halo_surfaces);
+        nothing changes under the reference's weights"""
+        self._check(self.lib.crt_restir_set_halo_surfaces(self.ctx, 1 if enable else 0))
 
     def restir_di_frame(self, W, H, frame, geom, triangles, raygen, eye, lights, options, bufs):
         self._check(self.lib.crt_restir_di_frame(self.ctx, W, H, frame, geom.handle, triangles.arg(), raygen,

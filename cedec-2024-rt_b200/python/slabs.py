@@ -159,7 +159,15 @@ class SlabRenderer:
         had in the previous frame's camera (set_camera).  That pixel may lie in any slab — the displacement is bounded by the
         camera motion, not by the spatial halo — so before such a frame every rank receives every other rank's rows of the
         history (full_plan: the halo plan with an unbounded reach, over NCCL / gloo); the direct-store path mirrors halo
-        rows only and is not used."""
+        rows only and is not used.
+        reproject="surfaces": the same look-up with the previous frame's surfaces, which unbiased reuse weights need with a
+        moving camera (cedecrt.RestirDI(reproject="surfaces")): two Visibility buffers alternate, and before a frame that
+        looks the history up every rank also receives every other rank's rows of last frame's Visibility
+        (crt_restir_set_previous_frame in fused mode, crt_temporal_resampling_reprojected_surfaces in drop-in mode).
+        Under the reference's weights it renders what reproject=True renders.
+        With more than one slab the fused frame produces the G-buffer records of its halo rows itself
+        (crt_restir_set_halo_surfaces), so that unbiased reuse weights (set_reuse_weights) run on every split of the frame;
+        under the reference's weights that costs nothing."""
         import numpy as np
 
         import cedecrt
@@ -177,9 +185,13 @@ class SlabRenderer:
         self.stream = stream if stream is not None else torch.cuda.current_stream()
         assert self.stream.cuda_stream != 0, "bench needs a non-default torch stream"
         self.rt.set_stream(self.stream.cuda_stream)
+        assert reproject in (False, True, "surfaces"), reproject
         self.reproject, self.prev_raygen = bool(reproject), None
+        self.surfaces = reproject == "surfaces"
         if self.reproject:
             p2p = False
+        if self.fused and world > 1:
+            self.rt.restir_set_halo_surfaces(True)
         self.overlap = bool(overlap and self.fused)
         self._tail = None
         if self.overlap:
@@ -231,6 +243,8 @@ class SlabRenderer:
         self.t_pix, self.pixels = tbuf(4 * n, np.uint8, 4 * n)
         self.t_acc, self.accumulation = tbuf(16 * n, cedecrt.FLOAT4, n, zero=True)
         self.t_vis, self.visibility = tbuf(16 * n, cedecrt.VISIBILITY, n, zero=True)
+        # reproject="surfaces": last frame's Visibility, kept for one more frame (the two buffers swap at each frame)
+        self.t_vis_prev, self.visibility_prev = tbuf(16 * n, cedecrt.VISIBILITY, n, zero=True) if self.surfaces else (None, None)
         self.t_r0, self.reservoir0 = tbuf(76 * n, cedecrt.RESERVOIR, n, zero=True, shared=True)
         self.t_r1, self.reservoir1 = tbuf(76 * n, cedecrt.RESERVOIR, n, zero=True, shared=True)
         self.t_tmp, self.temporal = tbuf(76 * n, cedecrt.RESERVOIR, n, zero=True, shared=True)
@@ -404,7 +418,25 @@ class SlabRenderer:
             self.halo_bytes += exchange(self.dist, self.t_tmp, self.W, self.H, SOA_RESERVOIR if self.fused else AOS_RESERVOIR,
                                         self.full_plan)
 
+    def gather_previous_visibility(self):
+        """every rank's rows of last frame's Visibility to every rank (reproject="surfaces" reads it at the history pixel)"""
+        if self.world > 1:
+            self.halo_bytes += exchange(self.dist, self.t_vis_prev, self.W, self.H, AOS_VISIBILITY, self.full_plan)
+
+    def _swap_visibility(self):
+        """reproject="surfaces": this frame traces into the buffer two frames old; last frame's becomes the previous one"""
+        self.t_vis, self.t_vis_prev = self.t_vis_prev, self.t_vis
+        self.visibility, self.visibility_prev = self.visibility_prev, self.visibility
+        rb = self.rt.restir_buffers
+        self.bufs = rb(self.pixels, self.accumulation, self.visibility, self.reservoir0, self.reservoir1, self.temporal)
+        if self._pix_ring is not None:
+            self._pix_ring = [(tp, p, rb(p, self.accumulation, self.visibility, self.reservoir0, self.reservoir1, self.temporal))
+                              for tp, p, _ in self._pix_ring]
+            self.bufs = self._pix_ring[self._pix_cur][2]
+
     def frame(self):
+        if self.surfaces:
+            self._swap_visibility()
         rt, W, H, o, g, t, v, eye = self.rt, self.W, self.H, self.options, self.geom, self.triangles, self.visibility, self.eye
         if self.fused and self.p2p:
             for stage in range(self.n_stages()):
@@ -416,8 +448,13 @@ class SlabRenderer:
         this_raygen = self.raygen
         if look_up:
             self.gather_history()
+            if self.surfaces:
+                self.gather_previous_visibility()
         if self.fused:
-            if self.reproject:
+            if self.surfaces:
+                rt.restir_set_previous_frame(self.prev_raygen if look_up else None, self.visibility_prev)
+                self.prev_raygen = this_raygen
+            elif self.reproject:
                 rt.restir_set_previous_camera(self.prev_raygen if look_up else None)
                 self.prev_raygen = this_raygen
             rt.restir_frame_begin(W, H, f, g, t, self.raygen, eye, self.lights, o, self.bufs)
@@ -432,7 +469,10 @@ class SlabRenderer:
         rt.raycast(W, H, g, t, self.raygen, v)
         self.exchange(self.t_vis, AOS_VISIBILITY)
         rt.generate_candidate(W, H, f, g, t, v, eye, self.lights, o, self.reservoir0)
-        if look_up:
+        if look_up and self.surfaces:
+            rt.temporal_resampling_reprojected_surfaces(W, H, f, g, t, v, eye, o, self.prev_raygen, self.visibility_prev,
+                                                        self.temporal, self.reservoir0)
+        elif look_up:
             rt.temporal_resampling_reprojected(W, H, f, g, t, v, eye, o, self.prev_raygen, self.temporal, self.reservoir0)
         else:
             rt.temporal_resampling(W, H, f, g, t, v, eye, o, self.temporal, self.reservoir0)
@@ -646,6 +686,10 @@ class SlabGroup:
     def reset_history(self):
         for s in self.slabs:
             s.reset_history()
+
+    def set_camera(self, eye, lookat_pt):
+        for s in self.slabs:
+            s.set_camera(eye, lookat_pt)
 
     def set_edges(self, edges):
         for s in self.slabs:

@@ -150,8 +150,8 @@ int crt_lights_changed(crt_ctx* ctx, crt_geometry geom);
  * CRT_REUSE_UNBIASED is refused (CRT_EINVAL) with a previous camera that comes without the previous frame's surfaces
  * (crt_temporal_resampling_reprojected, and a camera set with crt_restir_set_previous_camera: use
  * crt_temporal_resampling_reprojected_surfaces and crt_restir_set_previous_frame) and in the fused frame on a row range
- * narrower than the image or with slab links (the G-buffer of halo rows is not kept); the per-kernel path takes row
- * ranges.  An unknown mode is CRT_EINVAL. */
+ * narrower than the image or with slab links, unless crt_restir_set_halo_surfaces is on (otherwise the G-buffer of halo
+ * rows is not kept); the per-kernel path takes row ranges.  An unknown mode is CRT_EINVAL. */
 enum { CRT_REUSE_REFERENCE = 0, CRT_REUSE_UNBIASED = 1 };
 int crt_set_reuse_weights(crt_ctx* ctx, int mode);
 /* Multi-GPU row slabs: the kernels of this context compute only image rows yi in [y_begin, y_end) (y_end < 0:
@@ -310,9 +310,22 @@ int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int width, int he
  * run.  NULL previous_raygen clears both; crt_restir_set_previous_camera clears the stored Visibility.  Under
  * CRT_REUSE_UNBIASED crt_restir_frame_begin accepts a previous camera only when it was set here.  The frame checks
  * (CRT_EINVAL) that the buffer holds width * height records and is not buffers->visibility, which its raycast
- * overwrites; options that take the per-kernel path use crt_temporal_resampling_reprojected_surfaces.  The fused frame
- * with unbiased weights still refuses row ranges and slab links. */
+ * overwrites; options that take the per-kernel path use crt_temporal_resampling_reprojected_surfaces.  On a row range the
+ * fused frame with unbiased weights needs crt_restir_set_halo_surfaces, and the host provides every row of `temporal` and
+ * of the previous Visibility the look-ups can reach (python/slabs.py: SlabRenderer(reproject="surfaces")). */
 int crt_restir_set_previous_frame(crt_ctx* ctx, const crt_raygen* previous_raygen, crt_buffer previous_visibility);
+/* Halo surfaces (extension; DESIGN.md section 15, "Halo surfaces"; off by default): what the fused frame with
+ * CRT_REUSE_UNBIASED needs on a row range narrower than the image or with slab links.  Its spatial passes read every
+ * visited neighbour's primary-hit surface from the context's G-buffer, which the candidate kernel writes for the context's
+ * own rows only.  With this on, under CRT_REUSE_UNBIASED and fused options, crt_restir_frame_begin also produces the records
+ * of rows [y0 - h, y0) and [y1, y1 + h), clipped to the image, h = the rows a pass of spatial_resampling_radius can reach
+ * (87 at radius 30): primary rays into a Visibility buffer of the context's own (the host's buffers are written in the
+ * context's own rows only, as always), then the surface of every diffuse pixel with this frame's eye — bit for bit what
+ * the context that owns the row stores.  crt_restir_spatial_pass refuses (CRT_EINVAL) a radius that reaches further than
+ * the frame's begin covered.  The reservoirs of halo rows still come from the host's exchange or the slab links, whose own
+ * constraints stay (radius <= 30, spatial_resampling_passes != 1, slabs at least 87 rows tall).  Under
+ * CRT_REUSE_REFERENCE, on the whole image, or without spatial passes nothing is launched and every result is unchanged. */
+int crt_restir_set_halo_surfaces(crt_ctx* ctx, int enable);
 /* 10_restir_di.cu:239-254 — note the reference's parameter names are swapped: the first buffer is the source */
 int crt_save_temporal_reservoir(crt_ctx* ctx, int width, int height, crt_buffer src, crt_buffer dst);
 /* 10_restir_di.cu:256-388 */
