@@ -83,6 +83,7 @@ extern "C" int crt_shutdown(crt_ctx* ctx)
     if (ctx->queue_rays) cudaFree(ctx->queue_rays);
     if (ctx->queue_counters) cudaFree(ctx->queue_counters);
     if (ctx->history_prev) cudaFree(ctx->history_prev);
+    if (ctx->tiles) cudaFree(ctx->tiles);
     if (ctx->halo_vis) cudaFree(ctx->halo_vis);
     if (ctx->gbuf) cudaFree(ctx->gbuf);
     if (ctx->inline_rays) cudaFree(ctx->inline_rays);
@@ -115,6 +116,17 @@ extern "C" int crt_set_light_sampling(crt_ctx* ctx, int mode, int log2_slots)
     // whether 2^log2_slots fits the light count is checked by the first call that samples lights
     ctx->light_mode = mode;
     ctx->light_log2 = log2_slots;
+    return CRT_OK;
+}
+
+extern "C" int crt_set_light_tiles(crt_ctx* ctx, int log2_tiles, int log2_tile_size)
+{
+    CRT_REQUIRE(ctx, "null context");
+    CRT_REQUIRE(log2_tiles >= 0 && log2_tiles <= 16, "log2_tiles must be in [0, 16]");
+    CRT_REQUIRE(log2_tile_size >= 0 && log2_tile_size <= 16, "log2_tile_size must be in [0, 16]");
+    CRT_REQUIRE(log2_tiles + log2_tile_size <= 22, "light tiles hold at most 2^22 records: log2_tiles + log2_tile_size <= 22");
+    ctx->tiles_log2_t = log2_tiles;
+    ctx->tiles_log2_s = log2_tile_size;
     return CRT_OK;
 }
 

@@ -53,6 +53,13 @@ struct crt_ctx
     int light_table = 1;  // 0: sample lights through lights[] -> triangles[] like the reference (CRT_LIGHT_TABLE=0; uniform mode only)
     int light_mode = CRT_LIGHTS_UNIFORM;  // crt_set_light_sampling
     int light_log2 = 0;                   // requested log2 of the slot count of CRT_LIGHTS_POWER; 0: the default
+    // presampled light tiles of the ReSTIR DI candidates (crt_set_light_tiles; both 0: off) and the buffer of the last
+    // build, valid for (geometry serial, source table generation, frame, log2 T, log2 S) = tiles_key
+    int tiles_log2_t = 0, tiles_log2_s = 0;
+    void* tiles = nullptr;
+    size_t tiles_cap = 0;  // records the allocation holds
+    bool tiles_valid = false;
+    unsigned long long tiles_key[5] = {0, 0, 0, 0, 0};
     int reuse_mode = CRT_REUSE_REFERENCE;  // crt_set_reuse_weights
     // fused frame (kernels_fast.cu): G-buffer + pixel-class plane, 25 bytes per pixel, grown on demand
     void* gbuf = nullptr;
@@ -109,6 +116,7 @@ struct crt_geometry_t
     size_t light_table_n = 0;
     size_t light_table_cap = 0;  // records the allocation holds
     int light_table_log2 = -1;
+    unsigned long long light_table_gen = 0;  // counts the rebuilds of light_table (the key of a context's light tiles)
     void* light_scratch = nullptr;  // the slot table's build scratch (geometry.cu: build_light_slots), grown on demand
     size_t light_scratch_bytes = 0;
     float postpone_ratio = crt::kPostponeRatio;

@@ -522,6 +522,20 @@ int build_light_slots(crt_ctx* ctx, crt_geometry geom, const float* tris60, cons
     k_light_slots<<<(unsigned)(want < cap ? want : cap), kBuildBlock, 0, st>>>(K, n, start, tris60, lights, table);
     return check_launch(ctx, "light_slots");
 }
+
+// ---- presampled light tiles (restir_core.cuh: light_tile_slot): one thread per entry, a pure function of its index
+__global__ void __launch_bounds__(kBuildBlock)
+    k_light_tiles(const LightRec* src, uint32_t K, uint32_t frame, uint32_t log2_s, uint32_t count, LightRec* tiles)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < count) tiles[i] = src[light_tile_slot(frame, i >> log2_s, i & ((1u << log2_s) - 1u), K)];
+}
+int build_light_tiles(crt_ctx* ctx, const LightRec* src, uint32_t K, int frame, int log2_t, int log2_s, LightRec* tiles)
+{
+    const uint32_t count = 1u << (log2_t + log2_s);
+    k_light_tiles<<<div_up(count, kBuildBlock), kBuildBlock, 0, ctx->stream>>>(src, K, (uint32_t)frame, (uint32_t)log2_s, count, tiles);
+    return check_launch(ctx, "light_tiles");
+}
 }  // namespace crt
 
 using namespace crt;

@@ -374,22 +374,28 @@ extern "C" int crt_generate_candidate(crt_ctx* ctx, int W, int H, int frame, crt
     }
     const dim3 grid = tile_grid(W, rows);
     const bool sh = options.use_shadowed_target_function != 0;
+    auto launch = [&](auto L)
+    {
+        using LS = decltype(L);
+        if (wf) { if (sh) k_generate_candidate<LS, true, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LS, true, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
+        else { if (sh) k_generate_candidate<LS, false, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LS, false, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
+    };
     if (use_light_table(ctx))
     {
         const LightRec* table = nullptr;
         uint32_t n_slots = 0;
-        const int rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table, &n_slots);
+        int rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table, &n_slots);
         if (rc != CRT_OK) return rc;
-        const LightsTable L{table, n_slots};
-        if (wf) { if (sh) k_generate_candidate<LightsTable, true, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LightsTable, true, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
-        else { if (sh) k_generate_candidate<LightsTable, false, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LightsTable, false, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
+        if (light_tiles_on(ctx, n_lights))  // crt_set_light_tiles: the candidates draw from the pixel's tile of this frame
+        {
+            const LightRec* tiles = nullptr;
+            rc = light_tiles_for(ctx, geom, table, n_slots, frame, &tiles);
+            if (rc != CRT_OK) return rc;
+            launch(LightsTiles{tiles, (uint32_t)ctx->tiles_log2_t, (uint32_t)ctx->tiles_log2_s});
+        }
+        else launch(LightsTable{table, n_slots});
     }
-    else
-    {
-        const LightsIndexed L{tris60, (const uint32_t*)lights.data, n_lights};
-        if (wf) { if (sh) k_generate_candidate<LightsIndexed, true, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LightsIndexed, true, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
-        else { if (sh) k_generate_candidate<LightsIndexed, false, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LightsIndexed, false, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
-    }
+    else launch(LightsIndexed{tris60, (const uint32_t*)lights.data, n_lights});
     int rc = check_launch(ctx, "generate_candidate");
     if (rc != CRT_OK || !wf) return rc;
     return queue_trace<kEpiReservoirVisibility>(ctx, geom, q, ShadowSink{res, nullptr, 0, nullptr});
@@ -406,6 +412,28 @@ extern "C" int crt_light_sampling_table(crt_ctx* ctx, crt_geometry geom, crt_buf
     const int rc = light_table_for(ctx, geom, (const float*)geom->src, (const uint32_t*)lights.data, bsize(lights), &table, n_slots);
     if (rc != CRT_OK) return rc;
     *d_records = table;
+    return CRT_OK;
+}
+
+extern "C" int crt_light_tiles(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, int frame, const void** d_records,
+                               uint32_t* n_tiles, uint32_t* tile_size)
+{
+    CRT_REQUIRE(ctx && geom && d_records && n_tiles && tile_size, "null argument");
+    CRT_REQUIRE(bsize(lights) > 0 && lights.data != nullptr, "light tiles need a non-empty light buffer");
+    CRT_REQUIRE(bsize(lights) < 0xffffffffull, "too many lights");
+    CRT_REQUIRE(geom->src != nullptr, "geometry has no triangle array");
+    CRT_REQUIRE(light_tiles_on(ctx, 1), "light tiles are off (crt_set_light_tiles)");
+    CRT_JOIN_TAIL(ctx);
+    const LightRec* table = nullptr;
+    uint32_t K = 0;
+    int rc = light_table_for(ctx, geom, (const float*)geom->src, (const uint32_t*)lights.data, bsize(lights), &table, &K);
+    if (rc != CRT_OK) return rc;
+    const LightRec* tiles = nullptr;
+    rc = light_tiles_for(ctx, geom, table, K, frame, &tiles);
+    if (rc != CRT_OK) return rc;
+    *d_records = tiles;
+    *n_tiles = 1u << ctx->tiles_log2_t;
+    *tile_size = 1u << ctx->tiles_log2_s;
     return CRT_OK;
 }
 

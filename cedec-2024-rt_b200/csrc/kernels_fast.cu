@@ -115,9 +115,26 @@ __global__ void __launch_bounds__(256)
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse)
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles)
 {
     const bool unb = reuse == CRT_REUSE_UNBIASED;
+    if (tiles)  // crt_set_light_tiles: the candidates draw from the pixel's tile of this frame
+    {
+        const LightsTiles L = *tiles;
+        if (rp)
+        {
+            auto k = exact ? k_candidate_temporal_reprojected<LightsTiles, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal_reprojected<LightsTiles, 0, CRT_REUSE_REFERENCE>;
+            if (unb) k = exact ? k_candidate_temporal_reprojected<LightsTiles, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal_reprojected<LightsTiles, 0, CRT_REUSE_UNBIASED>;
+            k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
+        }
+        else
+        {
+            auto k = exact ? k_candidate_temporal<LightsTiles, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal<LightsTiles, 0, CRT_REUSE_REFERENCE>;
+            if (unb) k = exact ? k_candidate_temporal<LightsTiles, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal<LightsTiles, 0, CRT_REUSE_UNBIASED>;
+            k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
+        }
+        return;
+    }
     if (rp)
     {
         if (table)
@@ -182,6 +199,11 @@ int preload()
     CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 1, CRT_REUSE_UNBIASED>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_UNBIASED>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_UNBIASED>));
+    // light tiles over slab links too
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 0, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 1, CRT_REUSE_REFERENCE>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 0, CRT_REUSE_UNBIASED>));
+    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 1, CRT_REUSE_UNBIASED>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0, CRT_REUSE_UNBIASED>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1, CRT_REUSE_UNBIASED>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_resolve_fast));
@@ -197,7 +219,7 @@ int preload();
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse);
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles);
 void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
                     crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
@@ -211,7 +233,7 @@ int preload();
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse);
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles);
 void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
                     crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
@@ -535,6 +557,12 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
         rc = light_table_for(ctx, geom, tris60, (const uint32_t*)lights.data, n_lights, &table, &n_slots);
         if (rc != CRT_OK) return rc;
     }
+    LightsTiles tiles{nullptr, (uint32_t)ctx->tiles_log2_t, (uint32_t)ctx->tiles_log2_s};
+    if (light_tiles_on(ctx, n_lights))
+    {
+        rc = light_tiles_for(ctx, geom, table, n_slots, frame, &tiles.tiles);
+        if (rc != CRT_OK) return rc;
+    }
     Reprojection rp;
     const bool reproject = ctx->prev_cam_set && options.use_temporal_resampling;
     if (reproject)
@@ -558,7 +586,8 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     }
     CRT_MODE_NS(ctx, launch_candidate_temporal)(
         ctx->stream, exact, grid, W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), table,
-        (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr, ctx->reuse_mode);
+        (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr, ctx->reuse_mode,
+        tiles.tiles ? &tiles : nullptr);
     rc = check_launch(ctx, "candidate_temporal");
     if (rc != CRT_OK || !options.use_visibility_reuse) return rc;
     ShadowSink sink{nullptr, nullptr, 0, (uint32_t*)T.plane(0, 0)};

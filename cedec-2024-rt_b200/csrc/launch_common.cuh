@@ -154,13 +154,48 @@ static int light_table_for(crt_ctx* ctx, crt_geometry geom, const float* tris60,
         geom->light_table_key = lights;
         geom->light_table_n = n;
         geom->light_table_log2 = k;
+        geom->light_table_gen++;
     }
     *out = (const LightRec*)geom->light_table;
     *n_out = (uint32_t)count;
     return CRT_OK;
 }
-// every kernel that samples lights reads the table in power mode; in uniform mode CRT_LIGHT_TABLE=0 reads lights[] instead
-inline bool use_light_table(const crt_ctx* ctx) { return ctx->light_table || ctx->light_mode == CRT_LIGHTS_POWER; }
+// every kernel that samples lights reads the table in power mode and with light tiles; in uniform mode CRT_LIGHT_TABLE=0
+// reads lights[] instead
+inline bool use_light_table(const crt_ctx* ctx) { return ctx->light_table || ctx->light_mode == CRT_LIGHTS_POWER || ctx->tiles_log2_s || ctx->tiles_log2_t; }
+// presampled light tiles (geometry.cu)
+int build_light_tiles(crt_ctx* ctx, const LightRec* src, uint32_t K, int frame, int log2_t, int log2_s, LightRec* tiles);
+// the context's light tiles of `frame` over the source table (src, K) of `geom` (light_table_for), rebuilt on the context's
+// stream when any of (geometry, source table, frame, T, S) changed.  Every kernel that reads the tiles runs on that stream
+// too (the frame tail and the primary-ray prefetch read none), so a rebuild is ordered after the last frame's reads.
+static int light_tiles_for(crt_ctx* ctx, crt_geometry geom, const LightRec* src, uint32_t K, int frame, const LightRec** out)
+{
+    const int a = ctx->tiles_log2_t, b = ctx->tiles_log2_s;
+    const unsigned long long key[5] = {geom->serial, geom->light_table_gen, (unsigned long long)(unsigned)frame,
+                                       (unsigned long long)a, (unsigned long long)b};
+    bool same = ctx->tiles_valid;
+    for (int i = 0; i < 5; i++) same = same && ctx->tiles_key[i] == key[i];
+    if (!same)
+    {
+        ctx->tiles_valid = false;
+        const size_t count = (size_t)1 << (a + b);
+        if (ctx->tiles_cap < count)
+        {
+            if (ctx->tiles) CRT_CUDA(cudaFree(ctx->tiles));
+            ctx->tiles = nullptr;
+            ctx->tiles_cap = 0;
+            CRT_CUDA(cudaMalloc(&ctx->tiles, count * sizeof(LightRec)));
+            ctx->tiles_cap = count;
+        }
+        const int rc = build_light_tiles(ctx, src, K, frame, a, b, (LightRec*)ctx->tiles);
+        if (rc != CRT_OK) return rc;
+        for (int i = 0; i < 5; i++) ctx->tiles_key[i] = key[i];
+        ctx->tiles_valid = true;
+    }
+    *out = (const LightRec*)ctx->tiles;
+    return CRT_OK;
+}
+inline bool light_tiles_on(const crt_ctx* ctx, uint32_t n_lights) { return (ctx->tiles_log2_t || ctx->tiles_log2_s) && n_lights; }
 }  // namespace crt
 
 namespace crt

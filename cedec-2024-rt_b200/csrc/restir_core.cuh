@@ -311,6 +311,37 @@ CRT_HD float light_pdf_of(const LightSample& ls, uint32_t n)
 {
     return L::kHasPdf ? ls.pdf : 1.0f / (float)n * 1.0f / ls.area;
 }
+
+// ---- presampled light tiles (crt_set_light_tiles; DESIGN.md section 16).  Once per frame T = 2^log2_t tiles of
+// S = 2^log2_s records are drawn from the source table (K records: one per light, or the slot table of CRT_LIGHTS_POWER):
+// entry e of tile t copies record light_tile_slot(frame, t, e, K), pdf included.  A pixel's candidates draw from the one
+// tile of its 8x4 block (light_tile_of: one warp of tile_grid reads one tile), nth = (uint32)(rv0 * (float)S): entries
+// are uniform, and every entry is marginally distributed like a candidate drawn from the source, so each candidate is too.
+// the source slot of entry e of tile t: drawn from a stream of its own as a candidate draws rv0 (LightsTable::fetch)
+CRT_HD uint32_t light_tile_slot(uint32_t frame, uint32_t t, uint32_t e, uint32_t K)
+{
+    Pcg rng(hash_pcg3(frame, t, e), 1);
+    uint32_t s = (uint32_t)(rng.next_f() * (float)K);
+    if (s == K) s = K - 1;
+    return s;
+}
+// the tile of pixel (xi, yi), in global pixel coordinates (every row range agrees); reads no pixel's random stream
+CRT_HD uint32_t light_tile_of(int xi, int yi, int frame, uint32_t log2_t)
+{
+    return hash_pcg3((uint32_t)frame, (uint32_t)xi >> 3, (uint32_t)yi >> 2) & ((1u << log2_t) - 1u);
+}
+struct LightsTiles
+{
+    const LightRec* tiles;  // T * S records, tile t at tiles + t * S
+    uint32_t log2_t, log2_s;
+};
+// the light source a pixel's candidates draw from: the source itself, or with tiles a LightsTable over the pixel's tile
+template <class L>
+CRT_HD const L& pixel_lights(const L& lights, int, int, int) { return lights; }
+CRT_HD LightsTable pixel_lights(const LightsTiles& lights, int xi, int yi, int frame)
+{
+    return LightsTable{lights.tiles + ((size_t)light_tile_of(xi, yi, frame, lights.log2_t) << lights.log2_s), 1u << lights.log2_s};
+}
 CRT_HD float geometry_term(f3 p0, f3 n0, f3 p1, f3 n1)  // core.hpp:287-295
 {
     f3 v = p1 - p0;

@@ -268,7 +268,7 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
     Pcg rng(hash_pcg4(px.xi, px.yi, frame, 0), 0);
     const Surf surf = surface_from_visibility(tri, v.u, v.v, eye);
     g.store(px.idx, surf);
-    Res r = ris_candidates(bvh, lights, surf, opt.ris_count, false, rng, pair_mask);
+    Res r = ris_candidates(bvh, pixel_lights(lights, px.xi, px.yi, frame), surf, opt.ris_count, false, rng, pair_mask);
     r.ucw = ucw_of(r, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, false));
     bool candidate_survives = true;
     if (opt.temporal)

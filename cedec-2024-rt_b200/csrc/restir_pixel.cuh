@@ -181,7 +181,7 @@ CRT_HD DeferredRay px_generate_candidate(const Pix& px, int frame, const Bvh& bv
     }
     Pcg rng(hash_pcg4(px.xi, px.yi, frame, 0), 0);
     const Surf surf = surface_from_visibility(tri, v.u, v.v, eye);
-    Res r = ris_candidates(bvh, lights, surf, opt.ris_count, false, rng);
+    Res r = ris_candidates(bvh, pixel_lights(lights, px.xi, px.yi, frame), surf, opt.ris_count, false, rng);
     r.ucw = ucw_of(r, target_function(bvh, surf.p, surf.n, r.s.hp, r.s.hn, r.s.rad, opt.shadowed));
     if (opt.reuse)
     {

@@ -50,6 +50,8 @@ class Device
     void setRowRange(int y0, int y1) const { CRT_CHECKED(crt_set_row_range(m_ctx, y0, y1)); }
     // CRT_LIGHTS_UNIFORM (the reference) or CRT_LIGHTS_POWER; log2_slots = 0: the default slot count
     void setLightSampling(int mode, int log2_slots = 0) const { CRT_CHECKED(crt_set_light_sampling(m_ctx, mode, log2_slots)); }
+    // presampled light tiles for the ReSTIR DI candidates: 2^log2_tiles tiles of 2^log2_tile_size records; (0, 0): off
+    void setLightTiles(int log2_tiles, int log2_tile_size) const { CRT_CHECKED(crt_set_light_tiles(m_ctx, log2_tiles, log2_tile_size)); }
     // CRT_REUSE_REFERENCE (the reference) or CRT_REUSE_UNBIASED (1/Z weights in every temporal and spatial merge)
     void setReuseWeights(int mode) const { CRT_CHECKED(crt_set_reuse_weights(m_ctx, mode)); }
     // temporal reprojection in the fused frame with the previous frame's Visibility buffer (what CRT_REUSE_UNBIASED needs

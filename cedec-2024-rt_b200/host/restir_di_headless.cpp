@@ -5,7 +5,7 @@
 //   restir_di_headless --scene assets/blocks_restir.tri[.xz] [--tile NX NZ DX DZ] [--size W H] [--frames N]
 //                      [--eye x y z] [--lookat x y z] [--no-temporal] [--no-spatial] [--no-accumulate]
 //                      [--out image.ppm] [--dump-accum file.f32] [--fused] [--lights uniform|power]
-//                      [--reuse reference|unbiased]
+//                      [--reuse reference|unbiased] [--light-tiles LOG2_T LOG2_S]
 //
 // --fused issues one crt_restir_di_frame call per frame instead of the launch list (same image, see cedecrt.h).
 //
@@ -44,6 +44,7 @@ int main(int argc, char** argv)
     bool fused = false;
     int light_mode = CRT_LIGHTS_UNIFORM;  // --lights power: select lights in proportion to their power (cedecrt.h)
     int reuse_mode = CRT_REUSE_REFERENCE;  // --reuse unbiased: 1/Z weights in the temporal and spatial merges (cedecrt.h)
+    int tiles_log2_t = 0, tiles_log2_s = 0;  // --light-tiles 7 10: the candidates draw from presampled light tiles (cedecrt.h)
     int width = 1920, height = 1080, frames = 4, tile_nx = 1, tile_nz = 1;
     float tile_dx = 130.0f, tile_dz = 82.0f;
     float eye[3] = {-0.579885f, 22.194597f, -6.567105f}, center[3] = {5.224952f, 20.847435f, 1.431192f};  // :188-189
@@ -101,6 +102,7 @@ int main(int argc, char** argv)
             }
             reuse_mode = m == "unbiased" ? CRT_REUSE_UNBIASED : CRT_REUSE_REFERENCE;
         }
+        else if (a == "--light-tiles") { need(2); tiles_log2_t = atoi(argv[++i]); tiles_log2_s = atoi(argv[++i]); }
         else if (a == "--out") { need(1); out_ppm = argv[++i]; }
         else if (a == "--dump-accum") { need(1); dump_accum = argv[++i]; }
         else
@@ -120,6 +122,7 @@ int main(int argc, char** argv)
         printf("Device: %s\n", device.name());
         device.setLightSampling(light_mode);
         device.setReuseWeights(reuse_mode);
+        device.setLightTiles(tiles_log2_t, tiles_log2_s);
         Shader shader(device);
 
         std::vector<crt_triangle> triangles =

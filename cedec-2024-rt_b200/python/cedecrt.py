@@ -30,6 +30,8 @@ assert TRIANGLE.itemsize == 60 and VISIBILITY.itemsize == 16 and RESERVOIR.items
 
 MATH_LIBDEVICE, MATH_EXACT, MATH_FAST, MATH_REFERENCE = 0, 1, 2, 3  # include/cedecrt.h: CRT_MATH_*
 LIGHTS_UNIFORM, LIGHTS_POWER = 0, 1  # include/cedecrt.h: CRT_LIGHTS_*
+# (log2 T, log2 S) of RestirDI(light_tiles=True): 512 tiles of 1024 records, 32 MB, measured in DESIGN.md section 16
+LIGHT_TILES_DEFAULT = (9, 10)
 REUSE_REFERENCE, REUSE_UNBIASED = 0, 1  # include/cedecrt.h: CRT_REUSE_*
 
 
@@ -126,6 +128,8 @@ def _load():
         "crt_light_sampling_table": [P, G, B, C.POINTER(C.c_void_p), C.POINTER(C.c_uint32)],
         "crt_lights_changed": [P, G],
         "crt_set_reuse_weights": [P, I],
+        "crt_set_light_tiles": [P, I, I],
+        "crt_light_tiles": [P, G, B, I, C.POINTER(C.c_void_p), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)],
         "crt_set_stream": [P, C.c_void_p],
         "crt_set_frame_overlap": [P, I],
         "crt_frame_join": [P],
@@ -351,6 +355,19 @@ class Runtime:
     def lights_changed(self, geom):
         """the host changed emission of triangles in place: rebuild the light records at their next use"""
         self._check(self.lib.crt_lights_changed(self.ctx, geom.handle))
+
+    def set_light_tiles(self, log2_tiles, log2_tile_size):
+        """presampled light tiles for the ReSTIR DI candidates: 2^log2_tiles tiles of 2^log2_tile_size records drawn once
+        per frame from the light records; (0, 0) turns them off (include/cedecrt.h: crt_set_light_tiles)"""
+        self._check(self.lib.crt_set_light_tiles(self.ctx, log2_tiles, log2_tile_size))
+
+    def light_tiles(self, geom, lights, frame):
+        """the tiles the candidates of `frame` read for `lights`, copied to the host as float32 (T, S, 16)"""
+        ptr, t, s = C.c_void_p(), C.c_uint32(), C.c_uint32()
+        self._check(self.lib.crt_light_tiles(self.ctx, geom.handle, lights.arg(), frame, C.byref(ptr), C.byref(t), C.byref(s)))
+        out = np.zeros((t.value, s.value, 16), np.float32)
+        self._check(self.lib.crt_memcpy_d2h(self.ctx, out.ctypes.data, ptr, out.nbytes))
+        return out
 
     def set_reuse_weights(self, mode):
         """REUSE_REFERENCE (the reference's biased merge, default) or REUSE_UNBIASED: 1/Z weights in every temporal and
@@ -628,7 +645,8 @@ class RestirDI:
     """The application loop of examples/10_restir_di/10_restir_di.cpp:96-122,184-226,229-380, headless:
     buffers live on the device, one `frame()` issues the reference's launch list on the context's stream."""
 
-    def __init__(self, rt, width, height, triangles_host, eye, lookat_pt, options=None, fused=False, reproject=False):
+    def __init__(self, rt, width, height, triangles_host, eye, lookat_pt, options=None, fused=False, reproject=False,
+                 light_tiles=None):
         """fused=False: the reference's launch list, one crt_* call per kernel, AoS reservoir buffers (drop-in mode);
         fused=True: one crt_restir_di_frame call per frame (SoA reservoirs inside the same buffers).
         reproject=True (extension): temporal resampling looks the previous reservoir up at the pixel the surface point had
@@ -636,8 +654,12 @@ class RestirDI:
         set_camera() moves the camera and clears the accumulation like the reference's loop (10_restir_di.cpp:257-267).
         reproject="surfaces": the same look-up with the previous frame's surfaces, which unbiased reuse weights need with a
         moving camera: two Visibility buffers alternate and last frame's is passed on (the launch list's
-        crt_temporal_resampling_reprojected_surfaces; in fused mode crt_restir_set_previous_frame)."""
+        crt_temporal_resampling_reprojected_surfaces; in fused mode crt_restir_set_previous_frame).
+        light_tiles (extension): None leaves the context's setting as it is; True sets LIGHT_TILES_DEFAULT, a pair
+        (log2_tiles, log2_tile_size) sets those, (0, 0) turns tiles off (Runtime.set_light_tiles)."""
         assert reproject in (False, True, "surfaces"), reproject
+        if light_tiles is not None:
+            rt.set_light_tiles(*(LIGHT_TILES_DEFAULT if light_tiles is True else light_tiles))
         self.rt, self.W, self.H, self.fused = rt, width, height, fused
         self.reproject, self.prev_raygen = reproject, None
         self.prefetch = False  # fused + crt_set_frame_overlap: trace the next frame's primary rays right after issuing a frame

@@ -365,6 +365,9 @@ class SlabRenderer:
     def set_light_sampling(self, mode, log2_slots=0):
         self.rt.set_light_sampling(mode, log2_slots)
 
+    def set_light_tiles(self, log2_tiles, log2_tile_size):
+        self.rt.set_light_tiles(log2_tiles, log2_tile_size)
+
     def set_reuse_weights(self, mode):
         self.rt.set_reuse_weights(mode)
 
@@ -740,6 +743,10 @@ class SlabGroup:
     def set_light_sampling(self, mode, log2_slots=0):
         for s in self.slabs:
             s.rt.set_light_sampling(mode, log2_slots)
+
+    def set_light_tiles(self, log2_tiles, log2_tile_size):
+        for s in self.slabs:
+            s.rt.set_light_tiles(log2_tiles, log2_tile_size)
 
     def set_reuse_weights(self, mode):
         for s in self.slabs:

@@ -124,6 +124,26 @@ int crt_set_light_sampling(crt_ctx* ctx, int mode, int log2_slots);
 int crt_light_sampling_table(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, const void** d_records, uint32_t* n_slots);
 /* the host has changed emission (Ke) of triangles in place: the light records are rebuilt at their next use */
 int crt_lights_changed(crt_ctx* ctx, crt_geometry geom);
+/* Presampled light tiles (extension; RTXDI's light presampling).  Off by default (log2_tiles = log2_tile_size = 0).
+ * Applies only to the light pick of 10_restir_di's candidates: crt_generate_candidate (directly and through crt_launch),
+ * the fused frame's candidate + temporal kernel and the per-kernel path crt_restir_di_frame falls back to.  The NEE
+ * sample of crt_path_trace_08 and the candidates of crt_path_trace_09 keep reading the source records.
+ * Once per frame the context draws T = 2^log2_tiles tiles of S = 2^log2_tile_size records from the source records the
+ * candidates read otherwise (one per light, or the K slots of CRT_LIGHTS_POWER): entry e of tile t copies source slot
+ * (uint32)(u * (float)K), u a PCG draw keyed on (frame, t, e) only, pdf included.  The pixel (xi, yi) draws its candidates
+ * from tile hash(frame, xi >> 3, yi >> 2) & (T - 1) with nth = (uint32)(rv0 * (float)S), in global pixel coordinates, so
+ * every row range agrees; it consumes the same random numbers as without tiles.  Each candidate keeps the source's
+ * marginal distribution and divides by the record's own pdf, so RIS stays unbiased; candidates that share a tile are
+ * correlated, which costs variance, not bias.  Reuse, resolve and the shadow rays are unchanged.  The candidates then
+ * read T * S * 64 bytes per frame whatever the light count.  log2_tiles and log2_tile_size are in [0, 16] with
+ * log2_tiles + log2_tile_size <= 22; anything else returns CRT_EINVAL.  The tiles are owned by the context, rebuilt on its
+ * stream when the frame, the source records, T or S change. */
+int crt_set_light_tiles(crt_ctx* ctx, int log2_tiles, int log2_tile_size);
+/* the tiles of `frame` the candidates would read for this light list (built now if needed), for inspection: *n_tiles *
+ * *tile_size LightRec records (crt_light_sampling_table's layout), tile t first at record t * *tile_size; device memory
+ * owned by the context, valid until the next rebuild.  CRT_EINVAL while tiles are off. */
+int crt_light_tiles(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, int frame, const void** d_records, uint32_t* n_tiles,
+                    uint32_t* tile_size);
 /* Reuse weights (extension; the reference's reuse is biased).  Applies to every kernel that merges reservoirs:
  * crt_temporal_resampling and crt_spatial_resampling (directly and through crt_launch), the fused frame's candidate +
  * temporal kernel and crt_restir_spatial_pass, and the per-kernel path crt_restir_di_frame falls back to.
