@@ -194,4 +194,21 @@ inline int join_tail(crt_ctx* ctx)
     } while (0)
 
 inline unsigned div_up(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
+
+// device memory grown on demand: when the capacity `cap` (in the caller's unit) is below `want`, the buffer is replaced by
+// one of `bytes` bytes.  Pointer and capacity are cleared before the allocation, so a failed cudaMalloc leaves an empty,
+// consistent buffer.  *fresh tells whether the memory is new (its contents undefined): each caller fills it on its own stream.
+template <class T>
+int grow(T*& p, size_t& cap, size_t want, size_t bytes, bool* fresh = nullptr)
+{
+    if (fresh) *fresh = false;
+    if (cap >= want) return CRT_OK;
+    if (p) CRT_CUDA(cudaFree(p));
+    p = nullptr;
+    cap = 0;
+    CRT_CUDA(cudaMalloc((void**)&p, bytes));
+    cap = want;
+    if (fresh) *fresh = true;
+    return CRT_OK;
+}
 }  // namespace crt

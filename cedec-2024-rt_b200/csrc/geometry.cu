@@ -493,21 +493,15 @@ int build_light_slots(crt_ctx* ctx, crt_geometry geom, const float* tris60, cons
     const size_t q_bytes = ((size_t)n + 1) * 8, off_prefix = q_bytes, off_power = 2 * q_bytes,
                  off_start = off_power + (((size_t)n * 4 + 255) & ~(size_t)255), off_max = off_start + ((((size_t)n + 1) * 4 + 255) & ~(size_t)255),
                  off_tmp = off_max + 256, bytes = off_tmp + scan_bytes;
-    if (geom->light_scratch_bytes < bytes)
-    {
-        if (geom->light_scratch) CRT_CUDA(cudaFree(geom->light_scratch));
-        geom->light_scratch = nullptr;
-        geom->light_scratch_bytes = 0;
-        CRT_CUDA(cudaMalloc(&geom->light_scratch, bytes));
-        geom->light_scratch_bytes = bytes;
-    }
+    int rc = grow(geom->light_scratch, geom->light_scratch_bytes, bytes, bytes);
+    if (rc != CRT_OK) return rc;
     char* base = (char*)geom->light_scratch;
     unsigned long long *q = (unsigned long long*)base, *prefix = (unsigned long long*)(base + off_prefix);
     float* power = (float*)(base + off_power);
     uint32_t *start = (uint32_t*)(base + off_start), *pmax = (uint32_t*)(base + off_max);
     CRT_CUDA(cudaMemsetAsync(pmax, 0, 4, st));
     k_light_power<<<div_up(n, kBuildBlock), kBuildBlock, 0, st>>>(n, tris60, lights, power, pmax);
-    int rc = check_launch(ctx, "light_power");
+    rc = check_launch(ctx, "light_power");
     if (rc != CRT_OK) return rc;
     k_light_quantise<<<div_up((size_t)n + 1, kBuildBlock), kBuildBlock, 0, st>>>(n, power, pmax, q);
     rc = check_launch(ctx, "light_quantise");

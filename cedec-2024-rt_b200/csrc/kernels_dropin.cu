@@ -255,16 +255,8 @@ extern "C" int crt_raycast(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_bu
     // when it is the very array the tree was built over, the record each pixel already holds seeds its walk.
     if (triangles.data == nullptr || triangles.data != (const void*)geom->src) ctx->hint_tris = nullptr;
     if (ctx->raycast_hint && triangles.data != nullptr && triangles.data == (const void*)geom->src && geom->n_tris)
-    {
         ctx->hint_tris = geom->src;
-        k_raycast_hinted<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), geom->view(), raygen,
-                                                                  (crt_visibility*)visibility_buffer.data,
-                                                                  (const float*)geom->src, (uint32_t)geom->n_tris);
-    }
-    else
-        k_raycast<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), geom->view(), raygen,
-                                                           (crt_visibility*)visibility_buffer.data);
-    return check_launch(ctx, "raycast");
+    return raycast_rows(ctx, W, H, geom, raygen, rows_of(ctx, H), (crt_visibility*)visibility_buffer.data, "raycast");
 }
 
 // ---- primary rays of the next frame, ahead of time (frame overlap; include/cedecrt.h)
@@ -281,16 +273,11 @@ extern "C" int crt_restir_prefetch_raycast(crt_ctx* ctx, int W, int H, crt_geome
         CRT_CUDA(cudaEventCreateWithFlags(&ctx->ev_ray_ready, cudaEventDisableTiming));
         CRT_CUDA(cudaEventCreateWithFlags(&ctx->ev_vis_consumed, cudaEventDisableTiming));
     }
-    if (ctx->vis_next_pixels < n)
-    {
-        CRT_CUDA(cudaStreamSynchronize(ctx->head_stream));
-        if (ctx->vis_next) CRT_CUDA(cudaFree(ctx->vis_next));
-        ctx->vis_next = nullptr;
-        ctx->vis_next_pixels = 0;
-        CRT_CUDA(cudaMalloc(&ctx->vis_next, n * sizeof(crt_visibility)));
-        CRT_CUDA(cudaMemsetAsync(ctx->vis_next, 0xff, n * sizeof(crt_visibility), ctx->head_stream));  // index -1: no hint yet
-        ctx->vis_next_pixels = n;
-    }
+    if (ctx->vis_next_pixels < n) CRT_CUDA(cudaStreamSynchronize(ctx->head_stream));  // the last prefetch may still write the buffer
+    bool fresh = false;
+    int rc = grow(ctx->vis_next, ctx->vis_next_pixels, n, n * sizeof(crt_visibility), &fresh);
+    if (rc != CRT_OK) return rc;
+    if (fresh) CRT_CUDA(cudaMemsetAsync(ctx->vis_next, 0xff, n * sizeof(crt_visibility), ctx->head_stream));  // index -1: no hint yet
     if (ctx->vis_consumed_pending)  // the frame in flight may still be copying the previous prefetch out of the buffer
     {
         CRT_CUDA(cudaStreamWaitEvent(ctx->head_stream, ctx->ev_vis_consumed, 0));
@@ -299,12 +286,7 @@ extern "C" int crt_restir_prefetch_raycast(crt_ctx* ctx, int W, int H, crt_geome
     const Rows rows = rows_of(ctx, H);
     // hinted when a frame of this context has shown the tree's own triangle array to be alive (crt_raycast above); the
     // buffer is the context's own and holds the previous prefetch, or index -1 everywhere after its allocation
-    if (ctx->raycast_hint && ctx->hint_tris != nullptr && ctx->hint_tris == (const void*)geom->src && geom->n_tris)
-        k_raycast_hinted<<<tile_grid(W, rows), 256, 0, ctx->head_stream>>>(W, H, rows, geom->view(), raygen, (crt_visibility*)ctx->vis_next,
-                                                                           (const float*)geom->src, (uint32_t)geom->n_tris);
-    else
-        k_raycast<<<tile_grid(W, rows), 256, 0, ctx->head_stream>>>(W, H, rows, geom->view(), raygen, (crt_visibility*)ctx->vis_next);
-    const int rc = check_launch(ctx, "raycast", ctx->head_stream);
+    rc = raycast_rows(ctx, W, H, geom, raygen, rows, (crt_visibility*)ctx->vis_next, "raycast", ctx->head_stream);
     if (rc != CRT_OK) return rc;
     CRT_CUDA(cudaEventRecord(ctx->ev_ray_ready, ctx->head_stream));
     ctx->ray_next_cam = raygen;
@@ -336,16 +318,19 @@ int raycast_or_prefetched(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_buf
     ctx->vis_consumed_pending = true;
     return CRT_OK;
 }
-// primary rays of rows [rows.y0, rows.y1) into `vis` on the context's stream, hinted under the licence the frame's
-// raycast_or_prefetched has just renewed (the halo bands of crt_restir_set_halo_surfaces)
-int raycast_rows(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_raygen raygen, Rows rows, crt_visibility* vis, const char* what)
+// primary rays of rows [rows.y0, rows.y1) into `vis` on stream `on` (default: the context's), each walk seeded with the
+// pixel's record (k_raycast_hinted) while the context holds the licence for the tree's own triangle array (ctx->hint_tris,
+// set or cleared by crt_raycast and raycast_or_prefetched)
+int raycast_rows(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_raygen raygen, Rows rows, crt_visibility* vis, const char* what,
+                 cudaStream_t on)
 {
+    cudaStream_t st = on ? on : ctx->stream;
     if (ctx->raycast_hint && ctx->hint_tris != nullptr && ctx->hint_tris == (const void*)geom->src && geom->n_tris)
-        k_raycast_hinted<<<tile_grid(W, rows), 256, 0, ctx->stream>>>(W, H, rows, geom->view(), raygen, vis, (const float*)geom->src,
-                                                                      (uint32_t)geom->n_tris);
+        k_raycast_hinted<<<tile_grid(W, rows), 256, 0, st>>>(W, H, rows, geom->view(), raygen, vis, (const float*)geom->src,
+                                                             (uint32_t)geom->n_tris);
     else
-        k_raycast<<<tile_grid(W, rows), 256, 0, ctx->stream>>>(W, H, rows, geom->view(), raygen, vis);
-    return check_launch(ctx, what);
+        k_raycast<<<tile_grid(W, rows), 256, 0, st>>>(W, H, rows, geom->view(), raygen, vis);
+    return check_launch(ctx, what, on);
 }
 }  // namespace crt
 
@@ -373,12 +358,16 @@ extern "C" int crt_generate_candidate(crt_ctx* ctx, int W, int H, int frame, crt
         if (rc != CRT_OK) return rc;
     }
     const dim3 grid = tile_grid(W, rows);
-    const bool sh = options.use_shadowed_target_function != 0;
     auto launch = [&](auto L)
     {
-        using LS = decltype(L);
-        if (wf) { if (sh) k_generate_candidate<LS, true, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LS, true, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
-        else { if (sh) k_generate_candidate<LS, false, true><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); else k_generate_candidate<LS, false, false><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), L, options, res, q); }
+        with_flag(wf, [&](auto WF)
+        {
+            with_flag(options.use_shadowed_target_function != 0, [&](auto SH)
+            {
+                k_generate_candidate<decltype(L), WF, SH><<<grid, 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis,
+                                                                                          to_f3(eye), L, options, res, q);
+            });
+        });
     };
     if (use_light_table(ctx))
     {
@@ -437,6 +426,32 @@ extern "C" int crt_light_tiles(crt_ctx* ctx, crt_geometry geom, crt_buffer light
     return CRT_OK;
 }
 
+// the temporal merge of the three entry points below: in place (prev_cam null) or reprojected into the previous camera,
+// where prev_vis is the previous frame's Visibility (null: not given; CRT_REUSE_UNBIASED reads it at the history pixel)
+static int temporal_resampling(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,
+                               crt_buffer visibility_buffer, crt_float3 eye, crt_options options, const crt_raygen* prev_cam,
+                               const crt_visibility* prev_vis, crt_buffer previous_reservoirs, crt_buffer reservoirs, const char* what)
+{
+    const Rows rows = rows_of(ctx, H);
+    const float* tris60 = (const float*)triangles.data;
+    const crt_visibility* vis = (const crt_visibility*)visibility_buffer.data;
+    const crt_reservoir* prev = (const crt_reservoir*)previous_reservoirs.data;
+    crt_reservoir* cur = (crt_reservoir*)reservoirs.data;
+    with_math_reuse(ctx->math_mode == CRT_MATH_EXACT, ctx->reuse_mode, [&](auto MODE, auto RW)
+    {
+        with_flag(options.use_shadowed_target_function != 0, [&](auto SH)
+        {
+            if (prev_cam)
+                k_temporal_reprojected<MODE, SH, RW><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(
+                    W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), options, *prev_cam, prev, cur, prev_vis);
+            else
+                k_temporal<MODE, SH, RW><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis,
+                                                                                   to_f3(eye), options, prev, cur);
+        });
+    });
+    return check_launch(ctx, what);
+}
+
 extern "C" int crt_temporal_resampling(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,
                                        crt_buffer visibility_buffer, crt_float3 eye, crt_options options,
                                        crt_buffer previous_reservoirs, crt_buffer reservoirs)
@@ -447,17 +462,8 @@ extern "C" int crt_temporal_resampling(crt_ctx* ctx, int W, int H, int frame, cr
     CRT_CHECK_BUF(previous_reservoirs, (size_t)W * H, "previous reservoir");
     CRT_CHECK_BUF(reservoirs, (size_t)W * H, "reservoir");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
-    const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_temporal<1, true, CRT_REUSE_REFERENCE> : k_temporal<1, false, CRT_REUSE_REFERENCE>)
-                : (sh ? k_temporal<0, true, CRT_REUSE_REFERENCE> : k_temporal<0, false, CRT_REUSE_REFERENCE>);
-    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
-        k = ex ? (sh ? k_temporal<1, true, CRT_REUSE_UNBIASED> : k_temporal<1, false, CRT_REUSE_UNBIASED>)
-               : (sh ? k_temporal<0, true, CRT_REUSE_UNBIASED> : k_temporal<0, false, CRT_REUSE_UNBIASED>);
-    k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
-                                               (const crt_visibility*)visibility_buffer.data, to_f3(eye), options,
-                                               (const crt_reservoir*)previous_reservoirs.data,
-                                               (crt_reservoir*)reservoirs.data);
-    return check_launch(ctx, "temporal_resampling");
+    return temporal_resampling(ctx, W, H, frame, geom, triangles, visibility_buffer, eye, options, nullptr, nullptr,
+                               previous_reservoirs, reservoirs, "temporal_resampling");
 }
 
 extern "C" int crt_temporal_resampling_reprojected(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,
@@ -474,14 +480,8 @@ extern "C" int crt_temporal_resampling_reprojected(crt_ctx* ctx, int W, int H, i
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
     CRT_REQUIRE(ctx->reuse_mode != CRT_REUSE_UNBIASED, "unbiased reuse weights do not take a previous camera here: this call does not receive "
                                                        "the previous frame's surfaces (crt_temporal_resampling_reprojected_surfaces does)");
-    const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_temporal_reprojected<1, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<1, false, CRT_REUSE_REFERENCE>)
-                : (sh ? k_temporal_reprojected<0, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<0, false, CRT_REUSE_REFERENCE>);
-    k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
-                                               (const crt_visibility*)visibility_buffer.data, to_f3(eye), options, previous_raygen,
-                                               (const crt_reservoir*)previous_reservoirs.data, (crt_reservoir*)reservoirs.data,
-                                               nullptr);
-    return check_launch(ctx, "temporal_resampling_reprojected");
+    return temporal_resampling(ctx, W, H, frame, geom, triangles, visibility_buffer, eye, options, &previous_raygen, nullptr,
+                               previous_reservoirs, reservoirs, "temporal_resampling_reprojected");
 }
 
 extern "C" int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom,
@@ -500,17 +500,9 @@ extern "C" int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int W,
                 "the previous frame's Visibility must be a buffer of its own: this frame's raycast has overwritten it");
     CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "reprojection reads other pixels of the previous buffer: it cannot run in place");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
-    const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_temporal_reprojected<1, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<1, false, CRT_REUSE_REFERENCE>)
-                : (sh ? k_temporal_reprojected<0, true, CRT_REUSE_REFERENCE> : k_temporal_reprojected<0, false, CRT_REUSE_REFERENCE>);
-    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
-        k = ex ? (sh ? k_temporal_reprojected<1, true, CRT_REUSE_UNBIASED> : k_temporal_reprojected<1, false, CRT_REUSE_UNBIASED>)
-               : (sh ? k_temporal_reprojected<0, true, CRT_REUSE_UNBIASED> : k_temporal_reprojected<0, false, CRT_REUSE_UNBIASED>);
-    k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
-                                               (const crt_visibility*)visibility_buffer.data, to_f3(eye), options, previous_raygen,
-                                               (const crt_reservoir*)previous_reservoirs.data, (crt_reservoir*)reservoirs.data,
-                                               (const crt_visibility*)previous_visibility_buffer.data);
-    return check_launch(ctx, "temporal_resampling_reprojected_surfaces");
+    return temporal_resampling(ctx, W, H, frame, geom, triangles, visibility_buffer, eye, options, &previous_raygen,
+                               (const crt_visibility*)previous_visibility_buffer.data, previous_reservoirs, reservoirs,
+                               "temporal_resampling_reprojected_surfaces");
 }
 
 extern "C" int crt_save_temporal_reservoir(crt_ctx* ctx, int W, int H, crt_buffer src, crt_buffer dst)
@@ -540,16 +532,16 @@ extern "C" int crt_spatial_resampling(crt_ctx* ctx, int W, int H, int frame, int
     CRT_CHECK_BUF(reservoirs, (size_t)W * H, "output reservoir");
     CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "spatial_resampling cannot run in place");
     CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
-    const bool ex = ctx->math_mode == CRT_MATH_EXACT, sh = options.use_shadowed_target_function != 0;
-    auto k = ex ? (sh ? k_spatial<1, true, CRT_REUSE_REFERENCE> : k_spatial<1, false, CRT_REUSE_REFERENCE>)
-                : (sh ? k_spatial<0, true, CRT_REUSE_REFERENCE> : k_spatial<0, false, CRT_REUSE_REFERENCE>);
-    if (ctx->reuse_mode == CRT_REUSE_UNBIASED)
-        k = ex ? (sh ? k_spatial<1, true, CRT_REUSE_UNBIASED> : k_spatial<1, false, CRT_REUSE_UNBIASED>)
-               : (sh ? k_spatial<0, true, CRT_REUSE_UNBIASED> : k_spatial<0, false, CRT_REUSE_UNBIASED>);
-    k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, pass, geom->view(), (const float*)triangles.data,
-                                               (const crt_visibility*)visibility_buffer.data, to_f3(eye), options,
-                                               (const crt_reservoir*)previous_reservoirs.data,
-                                               (crt_reservoir*)reservoirs.data);
+    const Rows rows = rows_of(ctx, H);
+    with_math_reuse(ctx->math_mode == CRT_MATH_EXACT, ctx->reuse_mode, [&](auto MODE, auto RW)
+    {
+        with_flag(options.use_shadowed_target_function != 0, [&](auto SH)
+        {
+            k_spatial<MODE, SH, RW><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(
+                W, H, rows, frame, pass, geom->view(), (const float*)triangles.data, (const crt_visibility*)visibility_buffer.data,
+                to_f3(eye), options, (const crt_reservoir*)previous_reservoirs.data, (crt_reservoir*)reservoirs.data);
+        });
+    });
     return check_launch(ctx, "spatial_resampling");
 }
 
@@ -679,17 +671,18 @@ static int path_trace(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, 
     if (ctx->wavefront && wave_ok)
         return path_trace_wavefront(ctx, EX, W, H, frame, geom, (const float*)triangles.data, (const uint32_t*)lights.data,
                                     (uint32_t)bsize(lights), slots, n_slots, raygen, options, (crt_float4*)accumulation.data, counters);
-    if (slots)
+    const Rows rows = rows_of(ctx, H);
+    const float* tris60 = (const float*)triangles.data;
+    crt_float4* accum = (crt_float4*)accumulation.data;
+    with_flag(ctx->math_mode == CRT_MATH_EXACT, [&](auto MODE)
     {
-        auto k = ctx->math_mode == CRT_MATH_EXACT ? k_path_trace<EX, 1, LightsTable> : k_path_trace<EX, 0, LightsTable>;
-        k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
-                                                   slots, n_slots, raygen, options, (crt_float4*)accumulation.data, counters);
-        return check_launch(ctx, "path_trace");
-    }
-    auto k = ctx->math_mode == CRT_MATH_EXACT ? k_path_trace<EX, 1, LightsIndexed> : k_path_trace<EX, 0, LightsIndexed>;
-    k<<<tile_grid(W, rows_of(ctx, H)), 256, 0, ctx->stream>>>(W, H, rows_of(ctx, H), frame, geom->view(), (const float*)triangles.data,
-                                               (const uint32_t*)lights.data, (uint32_t)bsize(lights), raygen, options,
-                                               (crt_float4*)accumulation.data, counters);
+        if (slots)
+            k_path_trace<EX, MODE, LightsTable><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(
+                W, H, rows, frame, geom->view(), tris60, slots, n_slots, raygen, options, accum, counters);
+        else
+            k_path_trace<EX, MODE, LightsIndexed><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(
+                W, H, rows, frame, geom->view(), tris60, (const uint32_t*)lights.data, (uint32_t)bsize(lights), raygen, options, accum, counters);
+    });
     return check_launch(ctx, "path_trace");
 }
 extern "C" int crt_path_trace_07(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,
@@ -728,14 +721,8 @@ extern "C" int crt_ao_06(crt_ctx* ctx, crt_buffer pixels, crt_raygen raygen, int
         const size_t per_row = (size_t)W * (size_t)n_rays * 32u;
         int band = (int)(((size_t)4 << 30) / (per_row ? per_row : 1));
         band = band < kTileH ? kTileH : band / kTileH * kTileH;
-        if (ctx->ao_count_pixels < (size_t)W * H)
-        {
-            if (ctx->ao_count) CRT_CUDA(cudaFree(ctx->ao_count));
-            ctx->ao_count = nullptr;
-            ctx->ao_count_pixels = 0;
-            CRT_CUDA(cudaMalloc((void**)&ctx->ao_count, (size_t)W * H * sizeof(uint32_t)));
-            ctx->ao_count_pixels = (size_t)W * H;
-        }
+        rc = grow(ctx->ao_count, ctx->ao_count_pixels, (size_t)W * H, (size_t)W * H * sizeof(uint32_t));
+        if (rc != CRT_OK) return rc;
         for (int y0 = all.y0; y0 < all.y1; y0 += band)
         {
             const Rows rows{y0, y0 + band < all.y1 ? y0 + band : all.y1};

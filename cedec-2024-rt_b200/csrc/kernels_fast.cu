@@ -42,6 +42,21 @@
 
 namespace crt
 {
+// the host-side launchers of the fused frame's per-pixel kernels; each of ex, rf and fm defines one set, kLaunchers
+struct FusedLaunchers
+{
+    int (*preload)();
+    void (*candidate_temporal)(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
+                               const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
+                               const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles);
+    void (*spatial)(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
+                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
+    void (*resolve)(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
+                    const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
+    void (*halo_surfaces)(cudaStream_t st, dim3 grid, int W, int H, Rows rows, const float* tris60, const crt_visibility* vis,
+                          f3 eye, GBuf g);
+};
 namespace CRT_KNS
 {
 #ifndef CRT_CT_MINBLOCKS
@@ -111,69 +126,29 @@ __global__ void __launch_bounds__(256)
     if (t.in) px_halo_surface(t.px, tris60, vis, eye, g);
 }
 
-// host-side launchers, one set per namespace (the API below picks the namespace from the context's math mode)
+// host-side launchers, one set per namespace (the API below picks the set of the context's math mode: FusedLaunchers)
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
                                ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles)
 {
-    const bool unb = reuse == CRT_REUSE_UNBIASED;
-    if (tiles)  // crt_set_light_tiles: the candidates draw from the pixel's tile of this frame
+    auto launch = [&](auto L)
     {
-        const LightsTiles L = *tiles;
-        if (rp)
+        with_math_reuse(exact, reuse, [&](auto MODE, auto RW)
         {
-            auto k = exact ? k_candidate_temporal_reprojected<LightsTiles, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal_reprojected<LightsTiles, 0, CRT_REUSE_REFERENCE>;
-            if (unb) k = exact ? k_candidate_temporal_reprojected<LightsTiles, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal_reprojected<LightsTiles, 0, CRT_REUSE_UNBIASED>;
-            k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
-        }
-        else
-        {
-            auto k = exact ? k_candidate_temporal<LightsTiles, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal<LightsTiles, 0, CRT_REUSE_REFERENCE>;
-            if (unb) k = exact ? k_candidate_temporal<LightsTiles, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal<LightsTiles, 0, CRT_REUSE_UNBIASED>;
-            k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
-        }
-        return;
-    }
-    if (rp)
-    {
-        if (table)
-        {
-            const LightsTable L{table, n_lights};
-            auto k = exact ? k_candidate_temporal_reprojected<LightsTable, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal_reprojected<LightsTable, 0, CRT_REUSE_REFERENCE>;
-            if (unb) k = exact ? k_candidate_temporal_reprojected<LightsTable, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal_reprojected<LightsTable, 0, CRT_REUSE_UNBIASED>;
-            k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
-        }
-        else
-        {
-            const LightsIndexed L{tris60, light_ids, n_lights};
-            auto k = exact ? k_candidate_temporal_reprojected<LightsIndexed, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal_reprojected<LightsIndexed, 0, CRT_REUSE_REFERENCE>;
-            if (unb) k = exact ? k_candidate_temporal_reprojected<LightsIndexed, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal_reprojected<LightsIndexed, 0, CRT_REUSE_UNBIASED>;
-            k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
-        }
-        return;
-    }
-    if (table)
-    {
-        const LightsTable L{table, n_lights};
-        auto k = exact ? k_candidate_temporal<LightsTable, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal<LightsTable, 0, CRT_REUSE_REFERENCE>;
-        if (unb) k = exact ? k_candidate_temporal<LightsTable, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal<LightsTable, 0, CRT_REUSE_UNBIASED>;
-        k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
-    }
-    else
-    {
-        const LightsIndexed L{tris60, light_ids, n_lights};
-        auto k = exact ? k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_REFERENCE> : k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_REFERENCE>;
-        if (unb) k = exact ? k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_UNBIASED> : k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_UNBIASED>;
-        k<<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
-    }
+            if (rp) k_candidate_temporal_reprojected<decltype(L), MODE, RW><<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
+            else k_candidate_temporal<decltype(L), MODE, RW><<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
+        });
+    };
+    if (tiles) launch(*tiles);  // crt_set_light_tiles: the candidates draw from the pixel's tile of this frame
+    else if (table) launch(LightsTable{table, n_lights});
+    else launch(LightsIndexed{tris60, light_ids, n_lights});
 }
 void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
                     crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse)
 {
-    auto k = exact ? k_spatial_fast<1, CRT_REUSE_REFERENCE> : k_spatial_fast<0, CRT_REUSE_REFERENCE>;
-    if (reuse == CRT_REUSE_UNBIASED) k = exact ? k_spatial_fast<1, CRT_REUSE_UNBIASED> : k_spatial_fast<0, CRT_REUSE_UNBIASED>;
-    k<<<grid, 256, 0, st>>>(W, H, rows, frame, pass, bvh, eye, options, in, out, g, peers);
+    with_math_reuse(exact, reuse, [&](auto MODE, auto RW)
+                    { k_spatial_fast<MODE, RW><<<grid, 256, 0, st>>>(W, H, rows, frame, pass, bvh, eye, options, in, out, g, peers); });
 }
 void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
                     const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced)
@@ -188,61 +163,43 @@ void launch_halo_surfaces(cudaStream_t st, dim3 grid, int W, int H, Rows rows, c
 int preload()
 {
     cudaFuncAttributes a;
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 0, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 1, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1, CRT_REUSE_REFERENCE>));
-    // CRT_REUSE_UNBIASED runs over slab links with halo surfaces (crt_restir_set_halo_surfaces): its kernels are loaded too
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 0, CRT_REUSE_UNBIASED>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, 1, CRT_REUSE_UNBIASED>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 0, CRT_REUSE_UNBIASED>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, 1, CRT_REUSE_UNBIASED>));
-    // light tiles over slab links too
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 0, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 1, CRT_REUSE_REFERENCE>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 0, CRT_REUSE_UNBIASED>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, 1, CRT_REUSE_UNBIASED>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<0, CRT_REUSE_UNBIASED>));
-    CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<1, CRT_REUSE_UNBIASED>));
+    // both reuse weights and every light source: CRT_REUSE_UNBIASED (with halo surfaces, crt_restir_set_halo_surfaces) and
+    // light tiles run over slab links too.  The reprojected candidate kernels are not loaded: reprojection does not run over
+    // slab links.
+    for (int exact = 0; exact < 2; exact++)
+        for (int reuse : {CRT_REUSE_REFERENCE, CRT_REUSE_UNBIASED})
+        {
+            const int rc = with_math_reuse(exact, reuse, [&](auto MODE, auto RW) -> int
+            {
+                CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTable, MODE, RW>));
+                CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsIndexed, MODE, RW>));
+                CRT_CUDA(cudaFuncGetAttributes(&a, k_candidate_temporal<LightsTiles, MODE, RW>));
+                CRT_CUDA(cudaFuncGetAttributes(&a, k_spatial_fast<MODE, RW>));
+                return CRT_OK;
+            });
+            if (rc != CRT_OK) return rc;
+        }
     CRT_CUDA(cudaFuncGetAttributes(&a, k_resolve_fast));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_halo_surfaces));
     return CRT_OK;
 }
+extern const FusedLaunchers kLaunchers = {preload, launch_candidate_temporal, launch_spatial, launch_resolve, launch_halo_surfaces};
 }  // namespace CRT_KNS
 
 #if !defined(CRT_AUX_TU)
 namespace fm
 {
-int preload();
-void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
-                               const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
-                               const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles);
-void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
-                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
-void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
-                    const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
-void launch_halo_surfaces(cudaStream_t st, dim3 grid, int W, int H, Rows rows, const float* tris60, const crt_visibility* vis,
-                          f3 eye, GBuf g);
-}  // namespace fm
+extern const FusedLaunchers kLaunchers;
+}
 namespace rf
 {
-int preload();
-void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
-                               const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
-                               const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles);
-void launch_spatial(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
-                    crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
-void launch_resolve(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
-                    const crt_visibility* vis, SoaStore res, GBuf g, ShadowQueue q, int accumulate, int reuse_traced);
-void launch_halo_surfaces(cudaStream_t st, dim3 grid, int W, int H, Rows rows, const float* tris60, const crt_visibility* vis,
-                          f3 eye, GBuf g);
-}  // namespace rf
-// the namespace whose kernels implement the context's math mode
-#define CRT_MODE_NS(ctx, fn) ((ctx)->math_mode == CRT_MATH_FAST ? fm::fn : (ctx)->math_mode == CRT_MATH_REFERENCE ? rf::fn : ex::fn)
+extern const FusedLaunchers kLaunchers;
+}
+// the launchers whose kernels implement the context's math mode
+static const FusedLaunchers& launchers(const crt_ctx* ctx)
+{
+    return ctx->math_mode == CRT_MATH_FAST ? fm::kLaunchers : ctx->math_mode == CRT_MATH_REFERENCE ? rf::kLaunchers : ex::kLaunchers;
+}
 // the traced marks of a history buffer stop being true when the geometry they were traced against is replaced
 // Only this context's own rows (pixels [first, first + n) of the bottom-up buffer): with slab links set, the halo rows
 // of the buffer are stored into by the neighbours' kernels — and rewritten by them in full every frame, marks included —
@@ -264,9 +221,9 @@ int preload_fused_kernels()
     CRT_CUDA(cudaFuncGetAttributes(&a, k_trace_shadow_queue<kEpiSoaVisibility>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_trace_shadow_queue<kEpiResolve>));
     CRT_CUDA(cudaFuncGetAttributes(&a, k_build_light_table));
-    int rc = ex::preload();
-    if (rc == CRT_OK) rc = rf::preload();
-    return rc != CRT_OK ? rc : fm::preload();
+    int rc = ex::kLaunchers.preload();
+    if (rc == CRT_OK) rc = rf::kLaunchers.preload();
+    return rc != CRT_OK ? rc : fm::kLaunchers.preload();
 }
 // layout conversion for inspection / parity dumps / switching modes with history
 __global__ void __launch_bounds__(256) k_soa_to_aos(size_t n, SoaStore s, crt_reservoir* aos)
@@ -283,25 +240,21 @@ __global__ void __launch_bounds__(256) k_aos_to_soa(size_t n, const crt_reservoi
 #if !defined(CRT_AUX_TU)
 using namespace crt;
 
-namespace
+int crt::ensure_gbuf(crt_ctx* ctx, size_t n, GBuf* g)
 {
-int ensure_gbuf(crt_ctx* ctx, size_t n, GBuf* g)
-{
-    if (ctx->gbuf_pixels < n)
-    {
-        if (ctx->gbuf) CRT_CUDA(cudaFree(ctx->gbuf));
-        ctx->gbuf = nullptr;
-        ctx->gbuf_pixels = 0;
-        CRT_CUDA(cudaMalloc(&ctx->gbuf, n * 25 + 256));
-        CRT_CUDA(cudaMemsetAsync(ctx->gbuf, 0, n * 25 + 256, ctx->stream));
-        ctx->gbuf_pixels = n;
-    }
+    bool fresh = false;
+    const int rc = grow(ctx->gbuf, ctx->gbuf_pixels, n, n * 25 + 256, &fresh);
+    if (rc != CRT_OK) return rc;
+    if (fresh) CRT_CUDA(cudaMemsetAsync(ctx->gbuf, 0, n * 25 + 256, ctx->stream));
     const size_t cap = ctx->gbuf_pixels;
     g->g0 = (char*)ctx->gbuf;
     g->g1 = g->g0 + cap * 16;
     g->cls = (uint8_t*)(g->g1 + cap * 8);
     return CRT_OK;
 }
+
+namespace
+{
 // The fused bodies cover every option set except rays inside the target function; M must fit the 29 bits the
 // record gives it: (M-cap + candidates) x (neighbours + 1)^passes (10_restir_di.cu:186-188, reservoir.hpp:31-37).
 bool fused(const crt_options& o)
@@ -382,23 +335,18 @@ int halo_surfaces(crt_ctx* ctx, int W, int H, crt_geometry geom, const float* tr
     {
         const Rows& b = bands[k];
         if (b.y1 <= b.y0 || rows.y1 <= rows.y0) continue;
-        if (ctx->halo_vis_pixels < 2 * band_cap)
-        {
-            if (ctx->halo_vis) CRT_CUDA(cudaFree(ctx->halo_vis));
-            ctx->halo_vis = nullptr;
-            ctx->halo_vis_pixels = 0;
-            CRT_CUDA(cudaMalloc(&ctx->halo_vis, 2 * band_cap * sizeof(crt_visibility)));
-            CRT_CUDA(cudaMemsetAsync(ctx->halo_vis, 0xff, 2 * band_cap * sizeof(crt_visibility), ctx->stream));  // index -1: no hint yet
-            ctx->halo_vis_pixels = 2 * band_cap;
-        }
+        bool fresh = false;
+        int rc = grow(ctx->halo_vis, ctx->halo_vis_pixels, 2 * band_cap, 2 * band_cap * sizeof(crt_visibility), &fresh);
+        if (rc != CRT_OK) return rc;
+        if (fresh) CRT_CUDA(cudaMemsetAsync(ctx->halo_vis, 0xff, 2 * band_cap * sizeof(crt_visibility), ctx->stream));  // index -1: no hint yet
         // the kernels index records by the global pixel index: the band's first pixel, (H - b.y1) * W, lands on the slot's
         // first record (only the band's own pixels are read or written)
         const size_t first = (size_t)(H - b.y1) * W;
         crt_visibility* vis = (crt_visibility*)((uintptr_t)ctx->halo_vis + (uintptr_t)(k * band_cap) * sizeof(crt_visibility) -
                                                 (uintptr_t)first * sizeof(crt_visibility));
-        int rc = raycast_rows(ctx, W, H, geom, raygen, b, vis, "halo_raycast");
+        rc = raycast_rows(ctx, W, H, geom, raygen, b, vis, "halo_raycast");
         if (rc != CRT_OK) return rc;
-        CRT_MODE_NS(ctx, launch_halo_surfaces)(ctx->stream, tile_grid(W, b), W, H, b, tris60, vis, eye, g);
+        launchers(ctx).halo_surfaces(ctx->stream, tile_grid(W, b), W, H, b, tris60, vis, eye, g);
         rc = check_launch(ctx, "halo_surfaces");
         if (rc != CRT_OK) return rc;
     }
@@ -568,14 +516,8 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     if (reproject)
     {
         // snapshot of last frame's history: this frame's records overwrite `temporal` while other pixels still look theirs up
-        if (ctx->history_prev_pixels < n)
-        {
-            if (ctx->history_prev) CRT_CUDA(cudaFree(ctx->history_prev));
-            ctx->history_prev = nullptr;
-            ctx->history_prev_pixels = 0;
-            CRT_CUDA(cudaMalloc(&ctx->history_prev, n * 72));
-            ctx->history_prev_pixels = n;
-        }
+        rc = grow(ctx->history_prev, ctx->history_prev_pixels, n, n * 72);
+        if (rc != CRT_OK) return rc;
         CRT_CUDA(cudaMemcpyAsync(ctx->history_prev, b->temporal.data, n * 72, cudaMemcpyDeviceToDevice, ctx->stream));
         rp.history = SoaStore{(char*)ctx->history_prev, n};
         rp.prev_cam = ctx->prev_cam;
@@ -584,7 +526,7 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
         rp.prev_vis = (const crt_visibility*)ctx->prev_vis.data;
         rp.prev_eye = to_f3(ctx->prev_cam.m_origin);
     }
-    CRT_MODE_NS(ctx, launch_candidate_temporal)(
+    launchers(ctx).candidate_temporal(
         ctx->stream, exact, grid, W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), table,
         (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr, ctx->reuse_mode,
         tiles.tiles ? &tiles : nullptr);
@@ -628,7 +570,7 @@ extern "C" int crt_restir_spatial_pass(crt_ctx* ctx, int W, int H, int frame, in
     pass_buffers(b, pass, &in, &out);
     // the last pass's output is only read by this rank's resolve: nothing to mirror
     const HaloPeers peers = pass + 1 < options.spatial_resampling_passes ? halo_peers(ctx, which_of(b, out), rows, false, n) : HaloPeers();
-    CRT_MODE_NS(ctx, launch_spatial)(
+    launchers(ctx).spatial(
         ctx->stream, ctx->math_mode == CRT_MATH_EXACT, tile_grid(W, rows), W, H, rows, frame, pass, geom->view(), to_f3(eye),
         options, soa(in, n), soa(out, n), g, peers, ctx->reuse_mode);
     return check_launch(ctx, "spatial_fast");
@@ -661,7 +603,7 @@ extern "C" int crt_restir_frame_end(crt_ctx* ctx, int W, int H, crt_geometry geo
     rc = queue_prepare(ctx, (size_t)(rows.y1 - rows.y0) * W, &q, overlap ? 1 : 0);
     if (rc != CRT_OK) return rc;
     crt_float4* accum = (crt_float4*)b->accumulation.data;
-    CRT_MODE_NS(ctx, launch_resolve)(
+    launchers(ctx).resolve(
         ctx->stream, tile_grid(W, rows), accum, W, H, rows, (const float*)triangles.data,
         (const crt_visibility*)b->visibility.data, soa(fin, n), g, q, options.accumulate,
         ctx->resolve_reuse && options.use_visibility_reuse);

@@ -452,14 +452,8 @@ __global__ void __launch_bounds__(256) k_pt_write(int W, int H, Rows rows, PathS
 
 static int path_state(crt_ctx* ctx, size_t n, PathState* st)
 {
-    if (ctx->path_state_pixels < n)
-    {
-        if (ctx->path_state) CRT_CUDA(cudaFree(ctx->path_state));
-        ctx->path_state = nullptr;
-        ctx->path_state_pixels = 0;
-        CRT_CUDA(cudaMalloc(&ctx->path_state, n * kPathStateBytes + 256));
-        ctx->path_state_pixels = n;
-    }
+    const int rc = grow(ctx->path_state, ctx->path_state_pixels, n, n * kPathStateBytes + 256);
+    if (rc != CRT_OK) return rc;
     const size_t cap = ctx->path_state_pixels;
     char* p = (char*)ctx->path_state;
     st->ro_t = (float4*)p; p += cap * 16;
@@ -570,14 +564,17 @@ int path_trace_wavefront(crt_ctx* ctx, int example, int W, int H, int frame, crt
                          const uint32_t* lights, uint32_t n_lights, const LightRec* slots, uint32_t n_slots, crt_raygen raygen,
                          crt_options options, crt_float4* accum, unsigned long long* counters)
 {
-    const bool ex = ctx->math_mode == CRT_MATH_EXACT;
-#define CRT_PT_LS(EX, LS, P, N) (ex ? path_trace_wavefront_impl<EX, 1, LS>(ctx, W, H, frame, geom, tris60, P, N, raygen, options, accum, counters) \
-                                    : path_trace_wavefront_impl<EX, 0, LS>(ctx, W, H, frame, geom, tris60, P, N, raygen, options, accum, counters))
-#define CRT_PT(EX) (slots ? CRT_PT_LS(EX, LightsTable, slots, n_slots) : CRT_PT_LS(EX, LightsIndexed, lights, n_lights))
-    if (example == 7) return CRT_PT_LS(7, LightsIndexed, lights, n_lights);
-    if (example == 8) return CRT_PT(8);
-    return CRT_PT(9);
-#undef CRT_PT
-#undef CRT_PT_LS
+    auto run = [&](auto EX)
+    {
+        return with_flag(ctx->math_mode == CRT_MATH_EXACT, [&](auto MODE)
+        {
+            if constexpr (EX != 7)  // 07_pt samples no light
+                if (slots) return path_trace_wavefront_impl<EX, MODE, LightsTable>(ctx, W, H, frame, geom, tris60, slots, n_slots, raygen, options, accum, counters);
+            return path_trace_wavefront_impl<EX, MODE, LightsIndexed>(ctx, W, H, frame, geom, tris60, lights, n_lights, raygen, options, accum, counters);
+        });
+    };
+    if (example == 7) return run(std::integral_constant<int, 7>{});
+    if (example == 8) return run(std::integral_constant<int, 8>{});
+    return run(std::integral_constant<int, 9>{});
 }
 }  // namespace crt

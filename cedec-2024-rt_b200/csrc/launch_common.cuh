@@ -2,11 +2,31 @@
 // kernel translation units (kernels_dropin.cu: the reference's per-kernel entry points on AoS buffers;
 // kernels_fast.cu: the fused frame on SoA buffers).
 #pragma once
+#include <type_traits>
+
 #include "ctx.cuh"
 #include "shadow_queue.cuh"
 
 namespace crt
 {
+// A launch takes its kernel's template arguments from runtime state through these: f is called with each choice as a
+// std::integral_constant and names the kernel once, e.g. k<MODE, RW>, instead of once per combination in a ladder whose
+// single mistyped branch would launch the wrong variant.
+template <class F>
+inline auto with_flag(bool on, F&& f)
+{
+    return on ? f(std::true_type{}) : f(std::false_type{});
+}
+// f(MODE, RW): the MODE of Math<MODE> (1 for CRT_MATH_EXACT, else 0) and the reuse weights RW (CRT_REUSE_REFERENCE or
+// CRT_REUSE_UNBIASED)
+template <class F>
+inline auto with_math_reuse(bool exact, int reuse, F&& f)
+{
+    return with_flag(exact, [&](auto MODE)
+                     { return reuse == CRT_REUSE_UNBIASED ? f(MODE, std::integral_constant<int, CRT_REUSE_UNBIASED>{})
+                                                          : f(MODE, std::integral_constant<int, CRT_REUSE_REFERENCE>{}); });
+}
+
 constexpr int kTileW = 32, kTileH = 8;
 
 // pixel of this thread
@@ -78,14 +98,8 @@ static int queue_prepare(crt_ctx* ctx, size_t n_pixels, ShadowQueue* q, int whic
     }
     void*& rays = which ? ctx->queue2_rays : ctx->queue_rays;
     size_t& capacity = which ? ctx->queue2_capacity : ctx->queue_capacity;
-    if (capacity < n_pixels)
-    {
-        if (rays) CRT_CUDA(cudaFree(rays));
-        rays = nullptr;
-        capacity = 0;
-        CRT_CUDA(cudaMalloc(&rays, n_pixels * sizeof(ShadowRay)));
-        capacity = n_pixels;
-    }
+    const int rc = grow(rays, capacity, n_pixels, n_pixels * sizeof(ShadowRay));
+    if (rc != CRT_OK) return rc;
     if (which && !ctx->queue2_counters) CRT_CUDA(cudaMalloc((void**)&ctx->queue2_counters, 2 * sizeof(unsigned)));
     unsigned* counters = which ? ctx->queue2_counters : ctx->queue_counters;
     CRT_CUDA(cudaMemsetAsync(counters, 0, 2 * sizeof(unsigned), ctx->stream));
@@ -132,23 +146,18 @@ static int light_table_for(crt_ctx* ctx, crt_geometry geom, const float* tris60,
     if (geom->light_table_key != lights || geom->light_table_n != n || geom->light_table_log2 != k)
     {
         geom->light_table_key = nullptr;
-        if (geom->light_table_cap < (count ? count : 1))  // a rebuild of the same size (refit, new emission) reuses the memory
-        {
-            if (geom->light_table) CRT_CUDA(cudaFree(geom->light_table));
-            geom->light_table = nullptr;
-            geom->light_table_cap = 0;
-            CRT_CUDA(cudaMalloc(&geom->light_table, (count ? count : 1) * sizeof(LightRec)));
-            geom->light_table_cap = count ? count : 1;
-        }
+        // a rebuild of the same size (refit, new emission) reuses the memory
+        int rc = grow(geom->light_table, geom->light_table_cap, count ? count : 1, (count ? count : 1) * sizeof(LightRec));
+        if (rc != CRT_OK) return rc;
         if (power)
         {
-            const int rc = build_light_slots(ctx, geom, tris60, lights, (uint32_t)n, k, (LightRec*)geom->light_table);
+            rc = build_light_slots(ctx, geom, tris60, lights, (uint32_t)n, k, (LightRec*)geom->light_table);
             if (rc != CRT_OK) return rc;
         }
         else if (n)
         {
             k_build_light_table<<<div_up(n, 256), 256, 0, ctx->stream>>>((uint32_t)n, tris60, lights, (LightRec*)geom->light_table);
-            const int rc = check_launch(ctx, "build_light_table");
+            rc = check_launch(ctx, "build_light_table");
             if (rc != CRT_OK) return rc;
         }
         geom->light_table_key = lights;
@@ -179,15 +188,9 @@ static int light_tiles_for(crt_ctx* ctx, crt_geometry geom, const LightRec* src,
     {
         ctx->tiles_valid = false;
         const size_t count = (size_t)1 << (a + b);
-        if (ctx->tiles_cap < count)
-        {
-            if (ctx->tiles) CRT_CUDA(cudaFree(ctx->tiles));
-            ctx->tiles = nullptr;
-            ctx->tiles_cap = 0;
-            CRT_CUDA(cudaMalloc(&ctx->tiles, count * sizeof(LightRec)));
-            ctx->tiles_cap = count;
-        }
-        const int rc = build_light_tiles(ctx, src, K, frame, a, b, (LightRec*)ctx->tiles);
+        int rc = grow(ctx->tiles, ctx->tiles_cap, count, count * sizeof(LightRec));
+        if (rc != CRT_OK) return rc;
+        rc = build_light_tiles(ctx, src, K, frame, a, b, (LightRec*)ctx->tiles);
         if (rc != CRT_OK) return rc;
         for (int i = 0; i < 5; i++) ctx->tiles_key[i] = key[i];
         ctx->tiles_valid = true;
@@ -206,8 +209,11 @@ int path_trace_wavefront(crt_ctx* ctx, int example, int W, int H, int frame, crt
                          const uint32_t* lights, uint32_t n_lights, const LightRec* slots, uint32_t n_slots, crt_raygen raygen,
                          crt_options options, crt_float4* accum, unsigned long long* counters);
 int raycast_or_prefetched(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_buffer triangles, crt_raygen raygen, crt_buffer visibility);
-int raycast_rows(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_raygen raygen, Rows rows, crt_visibility* vis, const char* what);
+int raycast_rows(crt_ctx* ctx, int W, int H, crt_geometry geom, crt_raygen raygen, Rows rows, crt_visibility* vis, const char* what,
+                 cudaStream_t on = nullptr);
 int tone_mapping_on(crt_ctx* ctx, cudaStream_t st, crt_buffer pixels, crt_buffer accumulation, int W, int H);
+// the fused frame's G-buffer for n pixels, zeroed when (re)allocated (kernels_fast.cu)
+int ensure_gbuf(crt_ctx* ctx, size_t n, GBuf* g);
 int preload_fused_kernels();
 int preload_dropin_kernels();
 }  // namespace crt

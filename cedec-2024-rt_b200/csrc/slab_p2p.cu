@@ -96,16 +96,9 @@ extern "C" int crt_restir_reserve(crt_ctx* ctx, int W, int H, void** class_plane
 {
     CRT_REQUIRE(ctx, "null context");
     CRT_CHECK_IMAGE(W, H);
-    const size_t n = (size_t)W * H;
-    if (ctx->gbuf_pixels < n)
-    {
-        if (ctx->gbuf) CRT_CUDA(cudaFree(ctx->gbuf));
-        ctx->gbuf = nullptr;
-        ctx->gbuf_pixels = 0;
-        CRT_CUDA(cudaMalloc(&ctx->gbuf, n * 25 + 256));
-        CRT_CUDA(cudaMemsetAsync(ctx->gbuf, 0, n * 25 + 256, ctx->stream));
-        ctx->gbuf_pixels = n;
-    }
+    GBuf g;
+    const int rc = ensure_gbuf(ctx, (size_t)W * H, &g);
+    if (rc != CRT_OK) return rc;
     if (class_plane_base) *class_plane_base = ctx->gbuf;  // the allocation to export; the plane starts at 24 * capacity
     return CRT_OK;
 }
