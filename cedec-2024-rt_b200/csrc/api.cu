@@ -227,6 +227,15 @@ extern "C" int crt_memcpy_h2d(crt_ctx* ctx, void* dst, const void* src, size_t b
     CRT_CUDA(cudaStreamSynchronize(ctx->stream));
     return CRT_OK;
 }
+// device to device on the context's stream, ordered like every other copy (after the frame tail in flight); asynchronous
+extern "C" int crt_memcpy_d2d(crt_ctx* ctx, void* dst, const void* src, size_t bytes)
+{
+    CRT_REQUIRE(ctx && ((dst && src) || !bytes), "null argument");
+    CRT_JOIN_TAIL(ctx);
+    if (!bytes) return CRT_OK;
+    CRT_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+    return CRT_OK;
+}
 extern "C" int crt_memcpy_d2h(crt_ctx* ctx, void* dst, const void* src, size_t bytes)
 {
     CRT_REQUIRE(ctx && ((dst && src) || !bytes), "null argument");
@@ -349,6 +358,10 @@ extern "C" int crt_launch(crt_ctx* ctx, const char* name, void** params, unsigne
         return crt_temporal_resampling_reprojected_surfaces(ctx, ARG(int, 0), ARG(int, 1), ARG(int, 2), ARG(crt_geometry, 3),
                                                             ARG(B, 4), ARG(B, 5), ARG(crt_float3, 6), ARG(crt_options, 7),
                                                             ARG(crt_raygen, 8), ARG(B, 9), ARG(B, 10), ARG(B, 11));
+    if (!strcmp(name, "temporal_resampling_reprojected_motion"))
+        return crt_temporal_resampling_reprojected_motion(ctx, ARG(int, 0), ARG(int, 1), ARG(int, 2), ARG(crt_geometry, 3),
+                                                          ARG(B, 4), ARG(B, 5), ARG(crt_float3, 6), ARG(crt_options, 7),
+                                                          ARG(crt_raygen, 8), ARG(B, 9), ARG(B, 10), ARG(B, 11), ARG(B, 12));
     if (!strcmp(name, "save_temporal_reservoir"))
         return crt_save_temporal_reservoir(ctx, ARG(int, 0), ARG(int, 1), ARG(B, 2), ARG(B, 3));
     if (!strcmp(name, "spatial_resampling"))

@@ -74,6 +74,9 @@ struct crt_ctx
     // the previous frame's Visibility buffer (crt_restir_set_previous_frame; data == nullptr: not given): the history
     // pixel's surface for CRT_REUSE_UNBIASED
     crt_buffer prev_vis = {};
+    // the previous frame's triangle array (crt_restir_set_previous_triangles; data == nullptr: the geometry did not move),
+    // read with a previous camera only
+    crt_buffer prev_tris = {};
     void* history_prev = nullptr;
     size_t history_prev_pixels = 0;
     // CRT_REUSE_UNBIASED in the fused frame on a row range (crt_restir_set_halo_surfaces): the G-buffer records of the rows

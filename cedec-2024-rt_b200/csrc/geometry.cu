@@ -562,6 +562,10 @@ extern "C" int crt_refit_geometry(crt_ctx* ctx, crt_geometry g)
     CRT_REQUIRE(ctx && g, "null context or geometry");
     CRT_REQUIRE(g->device == ctx->device, "geometry belongs to another device");
     CRT_CUDA(cudaSetDevice(ctx->device));
+    // With frame overlap the previous frame's resolve rays (tail stream) and a primary-ray prefetch (head stream) may still
+    // walk g->nodes / g->tris: the refit kernels rewrite them only after both.  A prefetch is dropped anyway (new serial).
+    CRT_JOIN_TAIL(ctx);
+    if (ctx->head_stream) CRT_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_ray_ready, 0));  // the last prefetch, used or not
     return refit(ctx, g);
 }
 

@@ -60,17 +60,19 @@ __global__ void __launch_bounds__(256)
 }
 // the same with reprojection into the previous frame's camera (extension; reads `prev` anywhere in the image).  RW =
 // CRT_REUSE_UNBIASED reads the previous frame's Visibility `prev_vis` at the history pixel; the reference's merge ignores it
-// (the last parameter, so that the reference instantiations keep their code)
-template <int MODE, bool SH, int RW>
+// (the last parameter, so that the reference instantiations keep their code).  MOTION: moving geometry, `prev_tris60` is
+// the previous frame's triangle array (crt_temporal_resampling_reprojected_motion); the other instantiations ignore it
+template <int MODE, bool SH, int RW, bool MOTION = false>
 __global__ void __launch_bounds__(256)
     k_temporal_reprojected(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
                            crt_options options, crt_raygen prev_cam, const crt_reservoir* prev, crt_reservoir* cur,
-                           const crt_visibility* prev_vis)
+                           const crt_visibility* prev_vis, const float* prev_tris60)
 {
     const TilePix t = this_pixel(W, H, rows);
     if (t.in)
-        px_temporal<Math<MODE>, RW>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
-                                    AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur}, &prev_cam, W, H, prev_vis);
+        px_temporal<Math<MODE>, RW, MOTION>(t.px, frame, bvh, tris60, vis, eye, kernel_opt<SH>(options),
+                                            AosStore{const_cast<crt_reservoir*>(prev)}, AosStore{cur}, &prev_cam, W, H,
+                                            prev_vis, prev_tris60);
 }
 // 10_restir_di.cu:239-254 (the first buffer is the source).  Every pixel is copied, so the bottom-up
 // index permutation does not matter: plain word copy.
@@ -426,11 +428,13 @@ extern "C" int crt_light_tiles(crt_ctx* ctx, crt_geometry geom, crt_buffer light
     return CRT_OK;
 }
 
-// the temporal merge of the three entry points below: in place (prev_cam null) or reprojected into the previous camera,
+// the temporal merge of the four entry points below: in place (prev_cam null) or reprojected into the previous camera,
 // where prev_vis is the previous frame's Visibility (null: not given; CRT_REUSE_UNBIASED reads it at the history pixel)
+// and prev_tris60 the previous frame's triangle array (null: the geometry did not move)
 static int temporal_resampling(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom, crt_buffer triangles,
                                crt_buffer visibility_buffer, crt_float3 eye, crt_options options, const crt_raygen* prev_cam,
-                               const crt_visibility* prev_vis, crt_buffer previous_reservoirs, crt_buffer reservoirs, const char* what)
+                               const crt_visibility* prev_vis, crt_buffer previous_reservoirs, crt_buffer reservoirs, const char* what,
+                               const float* prev_tris60 = nullptr)
 {
     const Rows rows = rows_of(ctx, H);
     const float* tris60 = (const float*)triangles.data;
@@ -442,8 +446,12 @@ static int temporal_resampling(crt_ctx* ctx, int W, int H, int frame, crt_geomet
         with_flag(options.use_shadowed_target_function != 0, [&](auto SH)
         {
             if (prev_cam)
-                k_temporal_reprojected<MODE, SH, RW><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(
-                    W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), options, *prev_cam, prev, cur, prev_vis);
+                with_flag(prev_tris60 != nullptr, [&](auto MOTION)
+                {
+                    k_temporal_reprojected<MODE, SH, RW, MOTION><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(
+                        W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), options, *prev_cam, prev, cur, prev_vis,
+                        prev_tris60);
+                });
             else
                 k_temporal<MODE, SH, RW><<<tile_grid(W, rows), 256, 0, ctx->stream>>>(W, H, rows, frame, geom->view(), tris60, vis,
                                                                                    to_f3(eye), options, prev, cur);
@@ -503,6 +511,36 @@ extern "C" int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int W,
     return temporal_resampling(ctx, W, H, frame, geom, triangles, visibility_buffer, eye, options, &previous_raygen,
                                (const crt_visibility*)previous_visibility_buffer.data, previous_reservoirs, reservoirs,
                                "temporal_resampling_reprojected_surfaces");
+}
+
+extern "C" int crt_temporal_resampling_reprojected_motion(crt_ctx* ctx, int W, int H, int frame, crt_geometry geom,
+                                                          crt_buffer triangles, crt_buffer visibility_buffer, crt_float3 eye,
+                                                          crt_options options, crt_raygen previous_raygen,
+                                                          crt_buffer previous_triangles, crt_buffer previous_visibility_buffer,
+                                                          crt_buffer previous_reservoirs, crt_buffer reservoirs)
+{
+    CRT_REQUIRE(ctx && geom, "null context or geometry");
+    CRT_CHECK_IMAGE(W, H);
+    CRT_CHECK_BUF(visibility_buffer, (size_t)W * H, "visibility");
+    const bool unbiased = ctx->reuse_mode == CRT_REUSE_UNBIASED;
+    CRT_REQUIRE(!unbiased || previous_visibility_buffer.data != nullptr,
+                "unbiased reuse weights need the previous frame's Visibility buffer to follow moving geometry");
+    if (previous_visibility_buffer.data != nullptr)
+    {
+        CRT_CHECK_BUF(previous_visibility_buffer, (size_t)W * H, "previous visibility");
+        CRT_REQUIRE(previous_visibility_buffer.data != visibility_buffer.data,
+                    "the previous frame's Visibility must be a buffer of its own: this frame's raycast has overwritten it");
+    }
+    CRT_CHECK_BUF(previous_reservoirs, (size_t)W * H, "previous reservoir");
+    CRT_CHECK_BUF(reservoirs, (size_t)W * H, "reservoir");
+    CRT_REQUIRE(previous_reservoirs.data != reservoirs.data, "reprojection reads other pixels of the previous buffer: it cannot run in place");
+    CRT_REQUIRE(triangles.data != nullptr, "null triangle buffer");
+    CRT_REQUIRE(previous_triangles.data != nullptr || bsize(previous_triangles) == 0, "null previous triangle buffer");
+    CRT_REQUIRE(bsize(previous_triangles) == bsize(triangles),
+                "the previous triangle array must hold as many triangles as the current one, in the same order");
+    return temporal_resampling(ctx, W, H, frame, geom, triangles, visibility_buffer, eye, options, &previous_raygen,
+                               unbiased ? (const crt_visibility*)previous_visibility_buffer.data : nullptr, previous_reservoirs,
+                               reservoirs, "temporal_resampling_reprojected_motion", (const float*)previous_triangles.data);
 }
 
 extern "C" int crt_save_temporal_reservoir(crt_ctx* ctx, int W, int H, crt_buffer src, crt_buffer dst)

@@ -49,7 +49,8 @@ struct FusedLaunchers
     void (*candidate_temporal)(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles);
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles,
+                               const float* prev_tris60);
     void (*spatial)(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, int pass, Bvh bvh, f3 eye,
                     crt_options options, SoaStore in, SoaStore out, GBuf g, HaloPeers peers, int reuse);
     void (*resolve)(cudaStream_t st, dim3 grid, crt_float4* accum, int W, int H, Rows rows, const float* tris60,
@@ -79,16 +80,21 @@ __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
 }
 // the same with temporal reprojection (px_candidate_temporal<..., REPROJ = true>); a kernel of its own so that the
 // in-place kernel above keeps its registers and its code.  RW = CRT_REUSE_UNBIASED reads rp.prev_vis at the history pixel.
-template <class L, int MODE, int RW>
+// MOTION: moving geometry, `prev_tris60` is the previous frame's triangle array (crt_restir_set_previous_triangles); the
+// other instantiations ignore it (the last parameter, so that they keep their code)
+template <class L, int MODE, int RW, bool MOTION = false>
 __global__ void __launch_bounds__(256, CRT_CT_MINBLOCKS)
     k_candidate_temporal_reprojected(int W, int H, Rows rows, int frame, Bvh bvh, const float* tris60, const crt_visibility* vis, f3 eye,
-                                     L lights, crt_options options, SoaStore temporal, GBuf g, ShadowQueue q, HaloPeers peers, Reprojection rp)
+                                     L lights, crt_options options, SoaStore temporal, GBuf g, ShadowQueue q, HaloPeers peers, Reprojection rp,
+                                     const float* prev_tris60)
 {
     const TilePix t = this_pixel(W, H, rows);
     DeferredRay d{false, {0, 0, 0}, {0, 0, 0}};
     CandPixel cp{Vis{0.0f, 0.0f, -1}, true};
     if (t.in) cp = classify_pixel(t.px, tris60, vis);
-    if (t.in) d = px_candidate_temporal<Math<MODE>, L, true, RW>(t.px, cp, frame, bvh, tris60, eye, lights, make_opt(options), temporal, g, peers, 0u, rp);
+    if (t.in)
+        d = px_candidate_temporal<Math<MODE>, L, true, RW, MOTION>(t.px, cp, frame, bvh, tris60, eye, lights, make_opt(options),
+                                                                   temporal, g, peers, 0u, rp, prev_tris60);
     queue_push(q, d.want, to_shadow_ray(d, t.px.idx), d.decided);
 }
 #ifndef CRT_SP_MINBLOCKS
@@ -130,13 +136,19 @@ __global__ void __launch_bounds__(256)
 void launch_candidate_temporal(cudaStream_t st, bool exact, dim3 grid, int W, int H, Rows rows, int frame, Bvh bvh,
                                const float* tris60, const crt_visibility* vis, f3 eye, const LightRec* table,
                                const uint32_t* light_ids, uint32_t n_lights, crt_options options, SoaStore T, GBuf g,
-                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles)
+                               ShadowQueue q, HaloPeers peers, const Reprojection* rp, int reuse, const LightsTiles* tiles,
+                               const float* prev_tris60)
 {
     auto launch = [&](auto L)
     {
         with_math_reuse(exact, reuse, [&](auto MODE, auto RW)
         {
-            if (rp) k_candidate_temporal_reprojected<decltype(L), MODE, RW><<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp);
+            if (rp)
+                with_flag(prev_tris60 != nullptr, [&](auto MOTION)
+                {
+                    k_candidate_temporal_reprojected<decltype(L), MODE, RW, MOTION><<<grid, 256, 0, st>>>(
+                        W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers, *rp, prev_tris60);
+                });
             else k_candidate_temporal<decltype(L), MODE, RW><<<grid, 256, 0, st>>>(W, H, rows, frame, bvh, tris60, vis, eye, L, options, T, g, q, peers);
         });
     };
@@ -386,6 +398,7 @@ extern "C" int crt_restir_set_previous_camera(crt_ctx* ctx, const crt_raygen* pr
     ctx->prev_cam_set = previous_raygen != nullptr;
     if (previous_raygen) ctx->prev_cam = *previous_raygen;
     ctx->prev_vis = crt_buffer{};
+    if (!previous_raygen) ctx->prev_tris = crt_buffer{};
     return CRT_OK;
 }
 
@@ -396,6 +409,15 @@ extern "C" int crt_restir_set_previous_frame(crt_ctx* ctx, const crt_raygen* pre
     ctx->prev_cam_set = previous_raygen != nullptr;
     if (previous_raygen) ctx->prev_cam = *previous_raygen;
     ctx->prev_vis = previous_raygen ? previous_visibility : crt_buffer{};
+    if (!previous_raygen) ctx->prev_tris = crt_buffer{};
+    return CRT_OK;
+}
+
+extern "C" int crt_restir_set_previous_triangles(crt_ctx* ctx, crt_buffer previous_triangles)
+{
+    CRT_REQUIRE(ctx, "null context");
+    CRT_REQUIRE(previous_triangles.data != nullptr || bsize(previous_triangles) == 0, "null previous triangle buffer");
+    ctx->prev_tris = previous_triangles.data ? previous_triangles : crt_buffer{};
     return CRT_OK;
 }
 
@@ -428,6 +450,9 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
         CRT_REQUIRE(ctx->prev_vis.data != b->visibility.data,
                     "the previous frame's Visibility must be a buffer of its own: this frame's raycast overwrites buffers->visibility");
     }
+    const bool motion = ctx->prev_cam_set && ctx->prev_tris.data != nullptr;  // crt_restir_set_previous_triangles
+    CRT_REQUIRE(!motion || bsize(ctx->prev_tris) == bsize(triangles),
+                "the previous triangle array must hold as many triangles as the current one, in the same order");
     rc = raycast_or_prefetched(ctx, W, H, geom, triangles, raygen, b->visibility);
     if (rc != CRT_OK) return rc;
     ctx->frame_fused = fused(options);
@@ -457,7 +482,10 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     {
         rc = crt_generate_candidate(ctx, W, H, frame, geom, triangles, b->visibility, eye, lights, options, b->reservoir0);
         if (rc == CRT_OK)
-            rc = with_surfaces       ? crt_temporal_resampling_reprojected_surfaces(ctx, W, H, frame, geom, triangles, b->visibility, eye,
+            rc = motion              ? crt_temporal_resampling_reprojected_motion(ctx, W, H, frame, geom, triangles, b->visibility, eye,
+                                                                                  options, ctx->prev_cam, ctx->prev_tris, ctx->prev_vis,
+                                                                                  b->temporal, b->reservoir0)
+                 : with_surfaces     ? crt_temporal_resampling_reprojected_surfaces(ctx, W, H, frame, geom, triangles, b->visibility, eye,
                                                                                     options, ctx->prev_cam, ctx->prev_vis, b->temporal,
                                                                                     b->reservoir0)
                  : ctx->prev_cam_set ? crt_temporal_resampling_reprojected(ctx, W, H, frame, geom, triangles, b->visibility, eye, options,
@@ -529,7 +557,7 @@ extern "C" int crt_restir_frame_begin(crt_ctx* ctx, int W, int H, int frame, crt
     launchers(ctx).candidate_temporal(
         ctx->stream, exact, grid, W, H, rows, frame, geom->view(), tris60, vis, to_f3(eye), table,
         (const uint32_t*)lights.data, n_slots, options, T, g, q, peers, reproject ? &rp : nullptr, ctx->reuse_mode,
-        tiles.tiles ? &tiles : nullptr);
+        tiles.tiles ? &tiles : nullptr, reproject && motion ? (const float*)ctx->prev_tris.data : nullptr);
     rc = check_launch(ctx, "candidate_temporal");
     if (rc != CRT_OK || !options.use_visibility_reuse) return rc;
     ShadowSink sink{nullptr, nullptr, 0, (uint32_t*)T.plane(0, 0)};

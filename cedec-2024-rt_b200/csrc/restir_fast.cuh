@@ -244,11 +244,13 @@ struct Reprojection
 // RW: CRT_REUSE_REFERENCE, or CRT_REUSE_UNBIASED: temporal_merge_unbiased, and with REPROJ
 // temporal_merge_unbiased_reprojected on the history pixel's previous surface — one 16-byte Visibility load and the
 // triangle's 36 vertex bytes at the history pixel, only when the history has M > 0
-template <class M, class L, bool REPROJ = false, int RW = CRT_REUSE_REFERENCE>
+// MOTION (with REPROJ; crt_restir_set_previous_triangles): `prev_tris60` is the previous frame's triangle array; the
+// look-up and the history's surface follow moved triangles as px_temporal<..., MOTION> does (DESIGN.md section 17)
+template <class M, class L, bool REPROJ = false, int RW = CRT_REUSE_REFERENCE, bool MOTION = false>
 CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int frame, const Bvh& bvh, const float* tris60,
                                          f3 eye, const L& lights, const Opt& opt_in, const SoaStore& temporal,
                                          const GBuf& g, const HaloPeers& peers = HaloPeers(), unsigned pair_mask = 0u,
-                                         const Reprojection& rp = Reprojection())
+                                         const Reprojection& rp = Reprojection(), const float* prev_tris60 = nullptr)
 {
     Opt opt = opt_in;
     opt.shadowed = false;  // compile-time constant here: no traversal code inside the target function
@@ -280,10 +282,12 @@ CRT_HD DeferredRay px_candidate_temporal(const Pix& px, const CandPixel& cp, int
         if (REPROJ)
         {
             int xp, yp;
-            const bool found = reproject_pixel(to_raygen(rp.prev_cam), rp.W, rp.H, surf.p, xp, yp);
+            const f3 p_prev = MOTION ? previous_point(tris60, prev_tris60, v, surf) : surf.p;
+            const bool found = reproject_pixel(to_raygen(rp.prev_cam), rp.W, rp.H, p_prev, xp, yp);
             history = found ? rp.history.load(xp + (rp.H - yp - 1) * rp.W) : empty_res();
             if (RW == CRT_REUSE_UNBIASED && found && history.M > 0)
-                has_h = previous_surface(rp.prev_vis, tris60, xp + (rp.H - yp - 1) * rp.W, rp.prev_eye, hsurf);
+                has_h = previous_surface<MOTION>(rp.prev_vis, tris60, xp + (rp.H - yp - 1) * rp.W, rp.prev_eye, hsurf,
+                                                 prev_tris60);
         }
         else history = temporal.load(px.idx);
         if (RW == CRT_REUSE_UNBIASED && REPROJ)

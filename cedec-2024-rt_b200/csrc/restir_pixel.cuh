@@ -83,14 +83,37 @@ CRT_HD void primary_ray(const crt_raygen& raygen, const Pix& px, int W, int H, f
 {
     shoot(to_raygen(raygen), (float)px.xi / (float)W, (float)px.yi / (float)H, ro, rd);
 }
+// Moving geometry (crt_temporal_resampling_reprojected_motion, crt_restir_set_previous_triangles; DESIGN.md section 17):
+// whether triangle `index` has other vertex bits (its 36 vertex bytes) in the previous frame's array than in this one's
+CRT_HD bool tri_moved(const float* tris60, const float* prev_tris60, int index)
+{
+    const float* a = tris60 + (size_t)index * 15;
+    const float* b = prev_tris60 + (size_t)index * 15;
+    bool moved = false;
+    for (int k = 0; k < 9; ++k) moved |= f2u(CRT_LDG(a + k)) != f2u(CRT_LDG(b + k));
+    return moved;
+}
+// The point this surface point was at in the previous frame: the same barycentrics on the triangle's previous vertices,
+// or `surf.p` itself when the triangle did not move (not a recomputation, which a contracted build may round otherwise)
+CRT_HD f3 previous_point(const float* tris60, const float* prev_tris60, const Vis& v, const Surf& surf)
+{
+    if (!tri_moved(tris60, prev_tris60, v.index)) return surf.p;
+    const TriRef pt = tri_at(prev_tris60, v.index);
+    return bary_point(pt.v(0), pt.v(1), pt.v(2), v.u, v.v);
+}
 // The previous frame's primary-hit surface at pixel `idx`: its Visibility record and the eye that frame flipped the
 // normal towards (its RayGenerator's origin: crt_raygen_lookat stores the eye).  False on a sky pixel.  Primary rays are
-// deterministic and the geometry static, so this is the surface that frame's kernels used there.
-CRT_HD bool previous_surface(const crt_visibility* prev_vis, const float* tris60, int idx, f3 prev_eye, Surf& s)
+// deterministic, so this is the surface that frame's kernels used there when the geometry is static.  MOTION: the triangle
+// is read from `prev_tris60`, the previous frame's array, when it moved (tri_moved) — only the pointer is chosen, so an
+// unmoved triangle gives the static surface bit for bit.
+template <bool MOTION = false>
+CRT_HD bool previous_surface(const crt_visibility* prev_vis, const float* tris60, int idx, f3 prev_eye, Surf& s,
+                             const float* prev_tris60 = nullptr)
 {
     const Vis hv = load_vis(prev_vis, idx);
     if (hv.index == -1) return false;
-    s = surface_from_visibility(tri_at(tris60, hv.index), hv.u, hv.v, prev_eye);
+    const float* t = MOTION && tri_moved(tris60, prev_tris60, hv.index) ? prev_tris60 : tris60;
+    s = surface_from_visibility(tri_at(t, hv.index), hv.u, hv.v, prev_eye);
     return true;
 }
 
@@ -198,10 +221,13 @@ CRT_HD DeferredRay px_generate_candidate(const Pix& px, int frame, const Bvh& bv
 // RW: CRT_REUSE_REFERENCE (the reference's merge) or CRT_REUSE_UNBIASED: temporal_merge_unbiased without a previous
 // camera, temporal_merge_unbiased_reprojected with one — the history's surface is then the previous frame's at the
 // history pixel, from `prev_vis` (the previous frame's Visibility buffer, read there only; unused by the reference's merge)
-template <class M, int RW = CRT_REUSE_REFERENCE, class RSP, class RS>
+// MOTION (with a previous camera; crt_temporal_resampling_reprojected_motion): the look-up projects the point's previous
+// position (previous_point on `prev_tris60`, the previous frame's triangle array) and the history's surface is built on
+// the triangle the previous frame saw (previous_surface<true>)
+template <class M, int RW = CRT_REUSE_REFERENCE, bool MOTION = false, class RSP, class RS>
 CRT_HD void px_temporal(const Pix& px, int frame, const Bvh& bvh, const float* tris60, const crt_visibility* vis,
                         f3 eye, const Opt& opt, const RSP& prev, const RS& cur, const crt_raygen* prev_cam = nullptr,
-                        int W = 0, int H = 0, const crt_visibility* prev_vis = nullptr)
+                        int W = 0, int H = 0, const crt_visibility* prev_vis = nullptr, const float* prev_tris60 = nullptr)
 {
     const Vis v = load_vis(vis, px.idx);
     if (v.index == -1) return;
@@ -217,10 +243,12 @@ CRT_HD void px_temporal(const Pix& px, int frame, const Bvh& bvh, const float* t
     if (prev_cam)
     {
         int xp, yp;
-        const bool found = reproject_pixel(to_raygen(*prev_cam), W, H, surf.p, xp, yp);
+        const f3 p_prev = MOTION ? previous_point(tris60, prev_tris60, v, surf) : surf.p;
+        const bool found = reproject_pixel(to_raygen(*prev_cam), W, H, p_prev, xp, yp);
         history = found ? prev.load(xp + (H - yp - 1) * W) : empty_res();
         if (RW == CRT_REUSE_UNBIASED && found && history.M > 0)
-            has_h = previous_surface(prev_vis, tris60, xp + (H - yp - 1) * W, to_raygen(*prev_cam).origin, hsurf);
+            has_h = previous_surface<MOTION>(prev_vis, tris60, xp + (H - yp - 1) * W, to_raygen(*prev_cam).origin, hsurf,
+                                             prev_tris60);
     }
     else history = prev.load(px.idx);
     if (RW == CRT_REUSE_UNBIASED && prev_cam)

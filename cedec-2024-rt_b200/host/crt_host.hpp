@@ -63,6 +63,12 @@ class Device
     // the fused frame with CRT_REUSE_UNBIASED on a row range or with slab links: frame begin also produces the G-buffer
     // records of the halo rows its spatial passes read; nothing changes under the reference's weights
     void setHaloSurfaces(bool enable) const { CRT_CHECKED(crt_restir_set_halo_surfaces(m_ctx, enable ? 1 : 0)); }
+    // moving geometry in the fused frame's reprojection: the previous frame's triangle array (same count and order), kept
+    // by the host until the next frame has begun; an empty buffer clears it
+    void setPreviousTriangles(crt_buffer previous_triangles) const
+    {
+        CRT_CHECKED(crt_restir_set_previous_triangles(m_ctx, previous_triangles));
+    }
     // the launch list's reprojected temporal resampling with the previous frame's Visibility buffer
     void temporalResamplingReprojectedSurfaces(int width, int height, int frame, crt_geometry geom, crt_buffer triangles,
                                                crt_buffer visibility, crt_float3 eye, crt_options options,

@@ -140,6 +140,7 @@ def _load():
         "crt_memset": [P, C.c_void_p, I, C.c_size_t],
         "crt_memcpy_h2d": [P, C.c_void_p, C.c_void_p, C.c_size_t],
         "crt_memcpy_d2h": [P, C.c_void_p, C.c_void_p, C.c_size_t],
+        "crt_memcpy_d2d": [P, C.c_void_p, C.c_void_p, C.c_size_t],
         "crt_memcpy_d2h_async": [P, C.c_void_p, C.c_void_p, C.c_size_t],
         "crt_sync": [P],
         "crt_timer_start": [P],
@@ -159,6 +160,7 @@ def _load():
         "crt_temporal_resampling": [P, I, I, I, G, B, B, Float3, Options, B, B],
         "crt_temporal_resampling_reprojected": [P, I, I, I, G, B, B, Float3, Options, RayGenerator, B, B],
         "crt_temporal_resampling_reprojected_surfaces": [P, I, I, I, G, B, B, Float3, Options, RayGenerator, B, B, B],
+        "crt_temporal_resampling_reprojected_motion": [P, I, I, I, G, B, B, Float3, Options, RayGenerator, B, B, B, B],
         "crt_save_temporal_reservoir": [P, I, I, B, B],
         "crt_spatial_resampling": [P, I, I, I, I, G, B, B, Float3, Options, B, B],
         "crt_resolve": [P, B, I, I, G, B, B, Float3, Options, B],
@@ -176,6 +178,7 @@ def _load():
         "crt_restir_is_fused": [Options],
         "crt_restir_set_previous_camera": [P, C.POINTER(RayGenerator)],
         "crt_restir_set_previous_frame": [P, C.POINTER(RayGenerator), B],
+        "crt_restir_set_previous_triangles": [P, B],
         "crt_restir_set_halo_surfaces": [P, I],
         "crt_restir_class_plane": [P, C.POINTER(C.c_void_p)],
         "crt_reservoir_export_aos": [P, I, I, B, B],
@@ -267,6 +270,13 @@ class TypedBuffer:
         assert arr.nbytes == self.nbytes, (arr.nbytes, self.nbytes)
         if self.n:
             self.rt._check(self.rt.lib.crt_memcpy_h2d(self.rt.ctx, self.ptr, arr.ctypes.data, self.nbytes))
+        return self
+
+    def copy_from(self, other):
+        """device-to-device copy of another buffer of the same size, on the context's stream"""
+        assert other.nbytes == self.nbytes, (other.nbytes, self.nbytes)
+        if self.n:
+            self.rt._check(self.rt.lib.crt_memcpy_d2d(self.rt.ctx, self.ptr, other.ptr, self.nbytes))
         return self
 
     def zero(self):
@@ -509,6 +519,16 @@ class Runtime:
             self.ctx, W, H, frame, geom.handle, triangles.arg(), visibility.arg(), Float3(*eye), options, prev_raygen,
             prev_visibility.arg(), previous.arg(), reservoirs.arg()))
 
+    def temporal_resampling_reprojected_motion(self, W, H, frame, geom, triangles, visibility, eye, options, prev_raygen,
+                                               prev_triangles, prev_visibility, previous, reservoirs):
+        """temporal_resampling_reprojected_surfaces that follows moving geometry: prev_triangles is the previous frame's
+        triangle array (include/cedecrt.h: crt_temporal_resampling_reprojected_motion); prev_visibility may be None under
+        the reference's weights"""
+        pv = prev_visibility.arg() if prev_visibility is not None else _Buffer()
+        self._check(self.lib.crt_temporal_resampling_reprojected_motion(
+            self.ctx, W, H, frame, geom.handle, triangles.arg(), visibility.arg(), Float3(*eye), options, prev_raygen,
+            prev_triangles.arg(), pv, previous.arg(), reservoirs.arg()))
+
     def save_temporal_reservoir(self, W, H, src, dst):
         self._check(self.lib.crt_save_temporal_reservoir(self.ctx, W, H, src.arg(), dst.arg()))
 
@@ -554,6 +574,11 @@ class Runtime:
         begun (include/cedecrt.h: crt_restir_set_previous_frame); raygen None clears both"""
         vis = visibility.arg() if raygen is not None else _Buffer()
         self._check(self.lib.crt_restir_set_previous_frame(self.ctx, C.byref(raygen) if raygen is not None else None, vis))
+
+    def restir_set_previous_triangles(self, triangles):
+        """the previous frame's triangle array for the fused frame's reprojection, kept by the host until the next frame has
+        begun (include/cedecrt.h: crt_restir_set_previous_triangles); None clears it"""
+        self._check(self.lib.crt_restir_set_previous_triangles(self.ctx, triangles.arg() if triangles is not None else _Buffer()))
 
     def restir_set_halo_surfaces(self, enable):
         """the fused frame with unbiased reuse weights on a row range or with slab links: restir_frame_begin also produces
@@ -656,7 +681,8 @@ class RestirDI:
         moving camera: two Visibility buffers alternate and last frame's is passed on (the launch list's
         crt_temporal_resampling_reprojected_surfaces; in fused mode crt_restir_set_previous_frame).
         light_tiles (extension): None leaves the context's setting as it is; True sets LIGHT_TILES_DEFAULT, a pair
-        (log2_tiles, log2_tile_size) sets those, (0, 0) turns tiles off (Runtime.set_light_tiles)."""
+        (log2_tiles, log2_tile_size) sets those, (0, 0) turns tiles off (Runtime.set_light_tiles).
+        set_triangles() moves the geometry; with reprojection the next frame follows it (DESIGN.md section 17)."""
         assert reproject in (False, True, "surfaces"), reproject
         if light_tiles is not None:
             rt.set_light_tiles(*(LIGHT_TILES_DEFAULT if light_tiles is True else light_tiles))
@@ -668,6 +694,8 @@ class RestirDI:
         self.eye = tuple(float(np.float32(v)) for v in eye)
         self.raygen = lookat(eye, lookat_pt, width, height)
         self.triangles = rt.to_device(triangles_host)
+        # set_triangles: last frame's triangle array (allocated on the first move), passed on while `moved` is set
+        self.prev_triangles, self.moved = None, False
         self.lights = rt.to_device(light_indices(triangles_host))
         self.geom = rt.build_geometry(self.triangles)
         self.pixels = rt.buffer(np.uint8, 4 * n)
@@ -687,6 +715,23 @@ class RestirDI:
         self.eye = tuple(float(np.float32(v)) for v in eye)
         self.raygen = lookat(eye, lookat_pt, self.W, self.H)
         self.rt.clear(self.accumulation, self.W, self.H)
+
+    def set_triangles(self, triangles_host):
+        """Moves the geometry: new vertices for the same triangles, in the same order, the same ones emitting.  The tree is
+        refitted (Geometry.refit).  With reprojection the next frame follows the motion: its look-ups and, under unbiased
+        weights, the history's surfaces read the outgoing array, which is kept in `prev_triangles`
+        (crt_temporal_resampling_reprojected_motion; in fused mode crt_restir_set_previous_triangles).  Several calls
+        between two frames keep the array of the last frame."""
+        triangles_host = np.ascontiguousarray(triangles_host)
+        if len(triangles_host) != self.triangles.n or triangles_host.dtype != self.triangles.dtype:
+            raise ValueError("set_triangles takes the same number of triangles (%d), in the same layout" % self.triangles.n)
+        if self.reproject and not self.moved:
+            if self.prev_triangles is None:
+                self.prev_triangles = self.rt.buffer(self.triangles.dtype, self.triangles.n)
+            self.prev_triangles.copy_from(self.triangles)  # ordered before the upload on the context's stream
+            self.moved = True
+        self.triangles.upload(triangles_host)
+        self.geom.refit()
 
     def output_reservoirs(self):
         """final reservoirs of the last frame in the reference's AoS layout (host numpy array)"""
@@ -712,22 +757,31 @@ class RestirDI:
                                      self.visibility, self.eye)
         self.frame_index += 1
         f = self.frame_index
+        # set_triangles since the last frame: the look-up follows the motion (no history to follow before the first frame)
+        motion = self.moved and self.prev_raygen is not None
+        self.moved = False
         if self.fused:
             bufs = rt.restir_buffers(self.pixels, self.accumulation, v, self.reservoir0, self.reservoir1, self.temporal)
             if surfaces:
                 rt.restir_set_previous_frame(self.prev_raygen, self.prev_visibility)  # None before the first frame
             elif self.reproject:
                 rt.restir_set_previous_camera(self.prev_raygen)  # None before the first frame: no history to look up
+            if motion:
+                rt.restir_set_previous_triangles(self.prev_triangles)
             rt.restir_di_frame(W, H, f, g, t, self.raygen, eye, self.lights, o, bufs)
             if self.reproject:
                 self.prev_raygen = RayGenerator.from_buffer_copy(bytes(self.raygen))
                 rt.restir_set_previous_camera(None)  # the context serves other hosts too: leave it as the reference behaves
+                # (which clears the previous triangles too)
             if self.prefetch:
                 rt.restir_prefetch_raycast(W, H, g, self.raygen)
             return
         rt.raycast(W, H, g, t, self.raygen, v)
         rt.generate_candidate(W, H, f, g, t, v, eye, self.lights, o, self.reservoir0)
-        if surfaces and self.prev_raygen is not None:
+        if motion:
+            rt.temporal_resampling_reprojected_motion(W, H, f, g, t, v, eye, o, self.prev_raygen, self.prev_triangles,
+                                                      self.prev_visibility, self.temporal, self.reservoir0)
+        elif surfaces and self.prev_raygen is not None:
             rt.temporal_resampling_reprojected_surfaces(W, H, f, g, t, v, eye, o, self.prev_raygen, self.prev_visibility,
                                                         self.temporal, self.reservoir0)
         elif self.reproject and self.prev_raygen is not None:

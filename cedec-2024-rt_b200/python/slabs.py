@@ -165,6 +165,8 @@ class SlabRenderer:
         looks the history up every rank also receives every other rank's rows of last frame's Visibility
         (crt_restir_set_previous_frame in fused mode, crt_temporal_resampling_reprojected_surfaces in drop-in mode).
         Under the reference's weights it renders what reproject=True renders.
+        set_triangles() moves the geometry; with reprojection the next frame follows it (cedecrt.RestirDI.set_triangles:
+        every rank holds the whole triangle array, so the previous one is local).
         With more than one slab the fused frame produces the G-buffer records of its halo rows itself
         (crt_restir_set_halo_surfaces), so that unbiased reuse weights (set_reuse_weights) run on every split of the frame;
         under the reference's weights that costs nothing."""
@@ -188,6 +190,8 @@ class SlabRenderer:
         assert reproject in (False, True, "surfaces"), reproject
         self.reproject, self.prev_raygen = bool(reproject), None
         self.surfaces = reproject == "surfaces"
+        # set_triangles: last frame's triangle array (allocated on the first move), passed on while `moved` is set
+        self.t_tris_prev, self.prev_triangles, self.moved = None, None, False
         if self.reproject:
             p2p = False
         if self.fused and world > 1:
@@ -415,6 +419,29 @@ class SlabRenderer:
         self.raygen = self.c.lookat(eye, lookat_pt, self.W, self.H)
         self.rt.clear(self.accumulation, self.W, self.H)  # 10_restir_di.cpp:257-267
 
+    def set_triangles(self, tris):
+        """new vertices for the same triangles, in the same order (the same ones emitting): the scene array is rewritten and
+        the tree refitted.  With reproject the outgoing array is kept on the device and the next frame's look-ups and, under
+        unbiased weights, the history's surfaces follow the motion (crt_restir_set_previous_triangles in fused mode,
+        crt_temporal_resampling_reprojected_motion in drop-in mode).  Slabs sharing this one's scene (share=) see the new
+        vertices too; their frames must not be in flight (SlabGroup.set_triangles)."""
+        import numpy as np
+
+        tris = np.ascontiguousarray(tris)
+        if len(tris) != self.n_tris or tris.dtype.itemsize != self.c.TRIANGLE.itemsize:
+            raise ValueError("set_triangles takes the same number of triangles (%d), in the same layout" % self.n_tris)
+        src = self.torch.from_numpy(tris.view(np.uint8).reshape(-1))
+        self.rt.frame_join()  # the frame tail in flight may still read the vertices
+        with self.torch.cuda.stream(self.stream):
+            if self.reproject and not self.moved:
+                if self.t_tris_prev is None:
+                    self.t_tris_prev = self.torch.empty_like(self.t_tris)
+                    self.prev_triangles = self.rt.wrap(self.t_tris_prev.data_ptr(), self.c.TRIANGLE, self.n_tris)
+                self.t_tris_prev.copy_(self.t_tris)
+                self.moved = True
+            self.t_tris.copy_(src)
+        self.geom.refit()  # on the context's stream, which is self.stream: after the copies
+
     def gather_history(self):
         """every rank's rows of the temporal reservoirs to every rank (reprojection reads the history anywhere)"""
         if self.world > 1:
@@ -448,6 +475,8 @@ class SlabRenderer:
         self.frame_index += 1
         f = self.frame_index
         look_up = self.reproject and self.prev_raygen is not None and o.use_temporal_resampling
+        motion = look_up and self.moved  # set_triangles since the last frame
+        self.moved = False
         this_raygen = self.raygen
         if look_up:
             self.gather_history()
@@ -460,6 +489,8 @@ class SlabRenderer:
             elif self.reproject:
                 rt.restir_set_previous_camera(self.prev_raygen if look_up else None)
                 self.prev_raygen = this_raygen
+            if self.reproject:
+                rt.restir_set_previous_triangles(self.prev_triangles if motion else None)
             rt.restir_frame_begin(W, H, f, g, t, self.raygen, eye, self.lights, o, self.bufs)
             if self.overlap:
                 rt.restir_prefetch_raycast(W, H, g, self.raygen)  # the next frame's camera (static here)
@@ -472,7 +503,11 @@ class SlabRenderer:
         rt.raycast(W, H, g, t, self.raygen, v)
         self.exchange(self.t_vis, AOS_VISIBILITY)
         rt.generate_candidate(W, H, f, g, t, v, eye, self.lights, o, self.reservoir0)
-        if look_up and self.surfaces:
+        if motion:
+            rt.temporal_resampling_reprojected_motion(W, H, f, g, t, v, eye, o, self.prev_raygen, self.prev_triangles,
+                                                      self.visibility_prev if self.surfaces else None, self.temporal,
+                                                      self.reservoir0)
+        elif look_up and self.surfaces:
             rt.temporal_resampling_reprojected_surfaces(W, H, f, g, t, v, eye, o, self.prev_raygen, self.visibility_prev,
                                                         self.temporal, self.reservoir0)
         elif look_up:
@@ -693,6 +728,14 @@ class SlabGroup:
     def set_camera(self, eye, lookat_pt):
         for s in self.slabs:
             s.set_camera(eye, lookat_pt)
+
+    def set_triangles(self, tris):
+        """new vertices for the same triangles: the slabs of this GPU share one scene array and one tree, so every slab's
+        frame is finished first and the first slab rewrites the array and refits.  The slabs run over direct-store links,
+        which refuse reprojection, so there is no previous array to pass on (as RestirDI(reproject=False))."""
+        self._barrier()
+        self.slabs[0].set_triangles(tris)
+        self._barrier()
 
     def set_edges(self, edges):
         for s in self.slabs:

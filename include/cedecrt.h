@@ -165,8 +165,13 @@ int crt_light_tiles(crt_ctx* ctx, crt_geometry geom, crt_buffer lights, int fram
  *                        with p_hat_j the reference's target function at domain j's surface (including a shadow ray
  *                        under use_shadowed_target_function, traced only when the unshadowed value is positive).
  *                        Candidate generation is a single domain and unchanged.  Without reprojection the history's
- *                        surface is the pixel's own, so temporal Z = M whenever p_hat_q(y) > 0.  Unbiased for static
- *                        geometry: the first merge after crt_refit_geometry is not exactly so.
+ *                        surface is the pixel's own, so temporal Z = M whenever p_hat_q(y) > 0.  After
+ *                        crt_refit_geometry, without the previous frame's triangles (crt_temporal_resampling_reprojected_motion,
+ *                        crt_restir_set_previous_triangles; DESIGN.md section 17) the history is merged from where the
+ *                        moved surface point now lies, and S_h is rebuilt on this frame's triangles: that changes which
+ *                        history is merged and its c_h, not the estimator's unbiasedness, because the target function's
+ *                        support does not depend on S_h's orientation.  Under use_shadowed_target_function, where p_hat
+ *                        includes visibility, neither form is claimed unbiased across a refit.
  * CRT_REUSE_UNBIASED is refused (CRT_EINVAL) with a previous camera that comes without the previous frame's surfaces
  * (crt_temporal_resampling_reprojected, and a camera set with crt_restir_set_previous_camera: use
  * crt_temporal_resampling_reprojected_surfaces and crt_restir_set_previous_frame) and in the fused frame on a row range
@@ -221,6 +226,8 @@ int crt_free(crt_ctx* ctx, void* p);
 int crt_memset(crt_ctx* ctx, void* p, int byte, size_t bytes);
 int crt_memcpy_h2d(crt_ctx* ctx, void* dst, const void* src, size_t bytes);       /* oroMemcpyHtoD */
 int crt_memcpy_d2h(crt_ctx* ctx, void* dst, const void* src, size_t bytes);       /* oroMemcpyDtoH */
+/* device to device on the context's stream, asynchronous (extension: a host keeping last frame's triangle array) */
+int crt_memcpy_d2d(crt_ctx* ctx, void* dst, const void* src, size_t bytes);
 int crt_memcpy_d2h_async(crt_ctx* ctx, void* dst, const void* src, size_t bytes); /* oroMemcpyDtoHAsync, :386 */
 int crt_sync(crt_ctx* ctx);                                                       /* oroStreamSynchronize, :389 */
 /* OroStopwatch (libs/orochi/Orochi/OrochiUtils.h:179-209): events on the context's stream */
@@ -247,7 +254,9 @@ int crt_destroy_geometry(crt_ctx* ctx, crt_geometry g);
 /* The host has moved vertices in the triangle array the tree was built over (same count, same order): bring the tree
  * up to date without rebuilding it — HIPRT's hiprtBuildOperationUpdate (libs/hiprt/hiprt/hiprt_types.h:131-135), which
  * the reference never calls (it builds once, loader.hpp:106-110).  Topology is kept, boxes are recomputed bottom-up;
- * hits stay exact (the tree only culls).  Synchronous. */
+ * hits stay exact (the tree only culls).  Synchronous.  With frame overlap it first orders itself after the frame tail
+ * and the primary-ray prefetch in flight, which walk the tree; a host that writes the vertices on a stream of its own calls
+ * crt_frame_join first, since the tail may still read them. */
 int crt_refit_geometry(crt_ctx* ctx, crt_geometry g);
 /* statistics: {n_tris, n_wide_nodes, max_depth, build_ms, node_bytes, tri_bytes, box padding, last refit_ms} */
 int crt_geometry_stats(crt_geometry g, double out[8]);
@@ -334,6 +343,34 @@ int crt_temporal_resampling_reprojected_surfaces(crt_ctx* ctx, int width, int he
  * fused frame with unbiased weights needs crt_restir_set_halo_surfaces, and the host provides every row of `temporal` and
  * of the previous Visibility the look-ups can reach (python/slabs.py: SlabRenderer(reproject="surfaces")). */
 int crt_restir_set_previous_frame(crt_ctx* ctx, const crt_raygen* previous_raygen, crt_buffer previous_visibility);
+/* Reprojection that follows moving geometry (extension; DESIGN.md section 17): crt_temporal_resampling_reprojected_surfaces
+ * with one more input, `previous_triangles`: the triangle array of the previous frame, the same count and order as
+ * `triangles` (a host that writes vertices and calls crt_refit_geometry keeps the outgoing array for one frame).  For a
+ * pixel with Visibility (prim, u, v) the look-up projects the point's previous position into the previous camera: the
+ * surface point itself when the 36 vertex bytes of `prim` are equal in both arrays, otherwise the same barycentrics on
+ * the previous vertices.  Under CRT_REUSE_UNBIASED the history's surface S_h is built from the previous Visibility at h
+ * on the previous array's triangle when that triangle's vertex bytes differ, on `triangles` otherwise; the merge is
+ * crt_temporal_resampling_reprojected_surfaces'.  With `previous_triangles` byte-equal to `triangles` the result equals
+ * crt_temporal_resampling_reprojected_surfaces (CRT_REUSE_UNBIASED) or crt_temporal_resampling_reprojected
+ * (CRT_REUSE_REFERENCE) bit for bit.  Under CRT_REUSE_REFERENCE `previous_visibility_buffer` is not read and may be empty.
+ * The merged history is then the one built at the same material point; unbiasedness is as for
+ * crt_temporal_resampling_reprojected_surfaces with static emitters and the unshadowed target function (DESIGN.md
+ * section 17, "Scope" and "What the test can see").
+ * CRT_EINVAL: the refusals of crt_temporal_resampling_reprojected_surfaces, `previous_triangles` of another size than
+ * `triangles` or null with a nonzero size, and CRT_REUSE_UNBIASED without a previous Visibility buffer.  crt_launch name:
+ * "temporal_resampling_reprojected_motion" (previous_triangles is the 10th param, previous_visibility_buffer the 11th). */
+int crt_temporal_resampling_reprojected_motion(crt_ctx* ctx, int width, int height, int frame, crt_geometry geom,
+                                               crt_buffer triangles, crt_buffer visibility_buffer, crt_float3 eye,
+                                               crt_options options, crt_raygen previous_raygen, crt_buffer previous_triangles,
+                                               crt_buffer previous_visibility_buffer, crt_buffer previous_reservoirs,
+                                               crt_buffer reservoirs);
+/* The same inside the fused frame: the previous frame's triangle array, which the context stores (not copies) until it is
+ * cleared; the host keeps it unchanged until the next crt_restir_frame_begin has run.  NULL data clears it, and so does a
+ * NULL previous_raygen passed to crt_restir_set_previous_camera or crt_restir_set_previous_frame.  It applies while a
+ * previous camera is set: crt_restir_frame_begin then checks (CRT_EINVAL) that it holds as many triangles as `triangles`,
+ * and options that take the per-kernel path use crt_temporal_resampling_reprojected_motion.  CRT_EINVAL: null data with a
+ * nonzero size. */
+int crt_restir_set_previous_triangles(crt_ctx* ctx, crt_buffer previous_triangles);
 /* Halo surfaces (extension; DESIGN.md section 15, "Halo surfaces"; off by default): what the fused frame with
  * CRT_REUSE_UNBIASED needs on a row range narrower than the image or with slab links.  Its spatial passes read every
  * visited neighbour's primary-hit surface from the context's G-buffer, which the candidate kernel writes for the context's
